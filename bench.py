@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — measures the VSOM hot path on B200 (contract: see DESIGN.md §Measurement).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload = BASELINE.json configs[1]: VSOM 64x64 grid, median-estimator transformation, synthetic 128-dim data,
 1M samples per step (one step = one pass of the online training hot path over one 1M-sample chunk at the
@@ -231,6 +231,24 @@ def cpu_baseline_leg(train_gpu, score_state, score_rows_host, score_gpu, order_n
     return out
 
 
+DUMP_ROWS = 1 << 21  # per-sample outputs of up to this many rows are dumped whole, larger chunks as a fixed sample (dump < 64 MB)
+
+
+def dump_outputs(out_dir, ctx, bmu_dev, dist_dev, n):
+    """--dump-outputs: what the last timed step hands its caller, as <name>.npy: the per-sample BMU ids and distances it wrote
+    into the caller's buffers, and the map it leaves behind (mean, S, sigma, weight, hits).  Integers are written as float64,
+    which holds them exactly.  Above DUMP_ROWS samples, bmu / dist are taken at a fixed seeded set of rows, stored as row.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    out = {"bmu": bmu_dev.cpu().numpy()[rows].astype(np.float64), "dist": dist_dev.cpu().numpy()[rows]}
+    if n > DUMP_ROWS:
+        out["row"] = rows.astype(np.float64)
+    st = ctx.download_state()
+    out.update(mean=st["mean"], S=st["S"], sigma=st["sigma"], weight=st["weight"], hits=st["hits"].astype(np.float64))
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def _claim_stdout():
     """Libraries under us (NCCL's version banner) write to the C-level stdout; the contract is ONE JSON line there.  Point fd 1 at
     stderr for the run and keep the real stdout for the result line."""
@@ -257,7 +275,11 @@ def main():
     ap.add_argument("--no-large-map", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
     ap.add_argument("--large-rows", type=int, default=1024)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (rank 0); the inputs depend only on the arguments")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     SCORE_ROWS = args.score_rows
 
     rank = int(os.environ.get("RANK", "0"))
@@ -313,6 +335,8 @@ def main():
     barrier()
     clocks = sampler.stop() if sampler else None
     launches = ctx.launch_count - launches0
+    if args.dump_outputs and rank == 0:  # before the legs below reuse out_bmu / out_dist and train this map further
+        dump_outputs(args.dump_outputs, ctx, out_bmu, out_dist, n)
     k1_name = "online_step_fast_kernel" if ctx.last_train_fast else "online_step_kernel"
     total_ms = ev[0].elapsed_time(ev[-1])
     kernel_ms = [ev[i].elapsed_time(ev[i + 1]) for i in range(args.steps)]

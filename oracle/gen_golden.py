@@ -1,9 +1,16 @@
 """TEST INFRASTRUCTURE — generates tests/golden/ref_*.npz by driving the reference's OWN code
-(oracle/_ref/libvsom_ref.so = /root/reference/src/*.cpp compiled unmodified, see oracle/Makefile).
+(oracle/_ref/libvsom_ref.so = the reference's src/*.cpp compiled unmodified, see oracle/Makefile).
 
-Needs /root/reference (this container); the fixtures it writes are committed and travel to the GPU box.
-Usage: python oracle/gen_golden.py
+Needs the reference's sources to build that library; the fixtures it writes are committed.
+Usage: python oracle/gen_golden.py [--restatement]
+
+random_cases / batch_map_cases / eigen_sse_cases are the fresh-input comparisons of tests/test_oracle_pin.py; their
+outputs, stored as SHA-256 digests (ref_random.json, ref_batch_map.json, ref_eigen_sse.json), come from the compiled reference, or with --restatement
+from oracle/liboracle.so.  The committed three were made with --restatement; oracle/vsom_oracle.c is unchanged since
+commit 6ccba42, whose tests compared it with the compiled reference on exactly these inputs, bit for bit.
 """
+import hashlib
+import json
 import os
 import sys
 
@@ -26,11 +33,119 @@ CASES = [
 ]
 
 
+def random_cases(make):
+    """Fresh random cases: every transformation and decay, global and local BMU regimes, scoring.  make(W, H, D, tr) -> checker.
+    Returns the outputs by name."""
+    out = {}
+    rng = np.random.default_rng(3)
+    for tr in (po.STANDARD, po.MEDIAN, po.CLR):
+        for dec in (po.EXPONENTIAL, po.INVERSE):
+            W, H, D = int(rng.integers(2, 9)), int(rng.integers(2, 9)), (5 if tr == po.CLR else int(rng.integers(1, 40)))
+            c = make(W, H, D, tr)
+            c.random_initialize(11, 0.7)
+            x = rng.standard_normal((90, D)).astype(np.float32)
+            p = f"tr{tr}_dec{dec}_"
+            for si, sg in enumerate((2.7, 1.01, 1.0, 0.5)):
+                eta = 0.01 if tr == po.CLR else 0.3
+                for k, v in zip(("bmu", "dist", "resid2", "last"), c.train_rows(x, eta, sg, dec)):
+                    out[f"{p}sigma{si}_{k}"] = v
+                for k, v in c.get_state().items():
+                    out[f"{p}sigma{si}_{k}"] = v
+            for start in (0, W * H - 1, W - 1):
+                out[f"{p}local_bmu_from{start}"] = np.int64(c.find_local_bmu(x[0], start))
+            out[p + "umatrix"] = c.update_umatrix()
+            out[p + "bmd"] = c.find_restricted_bmd(x[1], 1)
+            if tr != po.CLR:
+                out[p + "evaluate"] = np.float64(c.evaluate(x))
+                out[p + "similarity"] = np.int64(c.measure_similarity(x[:30], 3, 0))
+    return out
+
+
+def batch_map_cases(make):
+    """The batch-map trainer: non-square maps (the SomIndex(map, index) quirk), several chunks per epoch, U-matrix after each
+    epoch and the early return at sigma < 1."""
+    out = {}
+    rng = np.random.default_rng(21)
+    for tr in (po.STANDARD, po.MEDIAN, po.CLR):
+        for W, H in ((6, 6), (7, 4), (4, 9)):
+            D = 5 if tr == po.CLR else 11
+            c = make(W, H, D, tr)
+            c.random_initialize(3, 1.0)
+            x = rng.standard_normal((90, D)).astype(np.float32)
+            p = f"tr{tr}_{W}x{H}_"
+            out[p + "mse"] = c.train_batch(x, 40, 5, 3.0, 0.35, True)
+            for k, v in c.get_state().items():
+                out[p + k] = v
+            out[p + "umatrix"] = c.update_umatrix()
+    return out
+
+
+def eigen_sse_cases(make):
+    """The whole path in the Eigen SSE2 dot order: training (all transformations, both decays, global and local BMU regimes),
+    scoring, evaluate, measureSimilarity, U-matrix, batch-map trainer.  make(W, H, D, tr) -> checker in that order."""
+    out = {}
+    rng = np.random.default_rng(4)
+    for tr in (po.STANDARD, po.MEDIAN, po.CLR):
+        for dec in (po.EXPONENTIAL, po.INVERSE):
+            W, H, D = int(rng.integers(2, 9)), int(rng.integers(2, 9)), (6 if tr == po.CLR else int(rng.integers(5, 60)))
+            c = make(W, H, D, tr)
+            c.random_initialize(11, 0.7)
+            x = rng.standard_normal((90, D)).astype(np.float32)
+            p = f"tr{tr}_dec{dec}_"
+            for si, sg in enumerate((2.7, 1.01, 1.0, 0.5)):
+                eta = 0.01 if tr == po.CLR else 0.3
+                for k, v in zip(("bmu", "dist", "resid2", "last"), c.train_rows(x, eta, sg, dec)):
+                    out[f"{p}sigma{si}_{k}"] = v
+                for k, v in c.get_state().items():
+                    out[f"{p}sigma{si}_{k}"] = v
+            out[p + "umatrix"] = c.update_umatrix()
+            out[p + "score_bmu"], out[p + "score_dist"] = c.find_bmu(x)
+            out[p + "bmd"] = c.find_restricted_bmd(x[1], 1)
+            if tr != po.CLR:
+                out[p + "evaluate"] = np.float64(c.evaluate(x))
+                out[p + "similarity"] = np.int64(c.measure_similarity(x[:30], 3, 0))
+    for tr in (po.STANDARD, po.CLR):
+        D = 5 if tr == po.CLR else 13
+        c = make(7, 4, D, tr)
+        c.random_initialize(3, 1.0)
+        x = rng.standard_normal((90, D)).astype(np.float32)
+        p = f"batch_tr{tr}_"
+        out[p + "mse"] = c.train_batch(x, 40, 4, 3.0, 0.35, True)
+        for k, v in c.get_state().items():
+            out[p + k] = v
+    return out
+
+
+def digests(outputs):
+    """Outputs by name -> {name: [dtype, shape, SHA-256 of the bytes]}, in the order they were computed."""
+    out = {}
+    for k, v in outputs.items():
+        a = np.ascontiguousarray(v)
+        out[k] = [a.dtype.str, list(np.shape(v)), hashlib.sha256(a.tobytes()).hexdigest()]
+    return out
+
+
+def write_comparison_cases(restatement):
+    if restatement:
+        seq = lambda W, H, D, tr: po.Oracle(W, H, D, tr)  # noqa: E731
+        sse = lambda W, H, D, tr: po.Oracle(W, H, D, tr, po.ORDER_EIGEN_SSE)  # noqa: E731
+    else:
+        seq, sse = po.Reference, po.ReferenceSse
+    for name, fn, make in (("random", random_cases, seq), ("batch_map", batch_map_cases, seq), ("eigen_sse", eigen_sse_cases, sse)):
+        with open(os.path.join(OUT, f"ref_{name}.json"), "w") as f:
+            json.dump(digests(fn(make)), f, indent=0)
+        print(name, "ok")
+
+
 def main():
+    if "--restatement" in sys.argv:
+        write_comparison_cases(True)
+        return
     if not po.Reference.available():
         po.build(quiet=False)
-    assert po.Reference.available(), "oracle/_ref/libvsom_ref.so missing (needs /root/reference)"
+    assert po.Reference.available(), "oracle/_ref/libvsom_ref.so missing (needs the reference's sources, see oracle/Makefile)"
     os.makedirs(OUT, exist_ok=True)
+    write_comparison_cases(False)
     for ci, (name, W, H, Din, tr, dec, eta, rows, sigmas) in enumerate(CASES):
         rng = np.random.default_rng(1000 + ci)
         r = po.Reference(W, H, Din, tr)
