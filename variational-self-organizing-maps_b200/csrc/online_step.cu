@@ -324,6 +324,9 @@ __global__ void __launch_bounds__(kThreads, 1) online_step_kernel(const StepPara
             sProf[i] = 0;
     u64 done = 0;
 
+    // keys carry local node indices (see the exchange below): only the rank holding global node 0 (rank 0, block 0) lets a
+    // NaN distance at its local node 0 win, like findBmu's seed; on other ranks local node 0 is an ordinary node
+    const unsigned nanSeed = p.rank == 0 ? 0u : ~0u;
     int ring = 0; // t % 3
     for (u64 t = 0; t < p.n; ++t, ring = ring == 2 ? 0 : ring + 1)
     {
@@ -502,7 +505,7 @@ __global__ void __launch_bounds__(kThreads, 1) online_step_kernel(const StepPara
                                 sacc = eacc.finish(erest, p.Dm & 7);
                                 if (p.localSearch)
                                     p.distBuf[(t & 1) * static_cast<u64>(p.nodeCount) + static_cast<u64>(l) * G + b] = sacc;
-                                best = u64_min(best, make_key(sacc, static_cast<unsigned>(l * G + b), tag));
+                                best = u64_min(best, make_key(sacc, static_cast<unsigned>(l * G + b), tag, nanSeed));
                             }
                         }
                         else if (l < L)
@@ -533,7 +536,7 @@ __global__ void __launch_bounds__(kThreads, 1) online_step_kernel(const StepPara
                             {
                                 if (p.localSearch)
                                     p.distBuf[(t & 1) * static_cast<u64>(p.nodeCount) + static_cast<u64>(l) * G + b] = sacc;
-                                best = u64_min(best, make_key(sacc, static_cast<unsigned>(l * G + b), tag));
+                                best = u64_min(best, make_key(sacc, static_cast<unsigned>(l * G + b), tag, nanSeed));
                             }
                         }
                         __syncwarp(); // every lane is done with this buffer before it is refilled
@@ -561,7 +564,7 @@ __global__ void __launch_bounds__(kThreads, 1) online_step_kernel(const StepPara
                     const float d = node_dist_reference<TR, ORDER>(mBase + l * stride, xt, p, n4, pi, pj);
                     if (p.localSearch)
                         p.distBuf[(t & 1) * static_cast<u64>(p.nodeCount) + static_cast<u64>(l) * G + b] = d;
-                    best = u64_min(best, make_key(d, static_cast<unsigned>(l * G + b), tag));
+                    best = u64_min(best, make_key(d, static_cast<unsigned>(l * G + b), tag, nanSeed));
                 }
         }
         else
@@ -584,7 +587,7 @@ __global__ void __launch_bounds__(kThreads, 1) online_step_kernel(const StepPara
                 const float d = dist_lanes<TR>(mBase + l * stride, xt, p.Dr, p.P, pi, pj, lane);
                 if (p.localSearch && lane == 0)
                     p.distBuf[(t & 1) * static_cast<u64>(p.nodeCount) + static_cast<u64>(l) * G + b] = d;
-                best = u64_min(best, make_key(d, static_cast<unsigned>(l * G + b), tag));
+                best = u64_min(best, make_key(d, static_cast<unsigned>(l * G + b), tag, nanSeed));
             }
         }
         if (p.localSearch)

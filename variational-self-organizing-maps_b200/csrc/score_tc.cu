@@ -32,6 +32,12 @@
 // statistical recall argument: Delta' only trades list length against the share of rows that need the full scan.  Up to
 // 48 survivors per row go to the exact rescore (which also re-checks min_hits eligibility, so nothing depends on the large
 // constant given to excluded nodes); rows with more (or whose list overflowed) take the exact full scan as well.
+// What the certificate covers: nodes with finite approximate scores.  A NaN score drops out of the epilogue's minima and is
+// never listed, which is right for every node but node 0: findBmu seeds with node 0, so a NaN distance there wins every
+// row (src/Som.cpp:293).  When node 0 has a NaN component (TcScale::nanNode0, set by map_stats_kernel) no row is certified
+// and the probes hand the call to the exact scan.  Rows with a NaN or infinite element, and rows whose best listed distance
+// overflows to inf, fail the certificate on their own (NaN / inf bound); an infinite map component collapses s_m so that
+// every node sits inside every margin.  All of these end in the exact scan.
 //
 // Kernel structure (one CTA per SM, persistent; 384 threads; by default two CTAs — the SMs of a TPC — form a cluster and
 // work as ONE tcgen05 cta_group::2 unit on 256 rows, see score_tc_kernel):
@@ -216,6 +222,7 @@ struct TcScale
     float maxAbs;   // max |m_pk| (bits, via atomicMax) — input of the scale
     float maxNorm2; // max_p |m_p|^2                   — input of the scale
     int split;      // 1: operands are hi / lo pairs of halves (three products per element), 0: one half each
+    int nanNode0;   // node 0 has a NaN component: no row can be certified (see "Candidate rule")
 };
 
 // Error bound E' and list margin Delta' of one row in its scaled units (see "Candidate rule" above).
@@ -692,6 +699,8 @@ __global__ void map_stats_kernel(const float *__restrict__ mean, int N, int D, i
     if (lane == 0)
     {
         norm2[p] = s;
+        if (p == 0 && s != s)
+            scale->nanNode0 = 1;
         atomicMax(reinterpret_cast<int *>(&scale->maxAbs), __float_as_int(fminf(mx, 3.0e38f)));
         if (s == s)
             atomicMax(reinterpret_cast<int *>(&scale->maxNorm2), __float_as_int(fminf(s, 3.0e38f)));
@@ -869,7 +878,7 @@ __global__ void __launch_bounds__(RS_THREADS) rescore_kernel(const float *__rest
     {
         const long long row = row0 + tid;
         const u64 key = sKey[tid];
-        const bool nan = (key & 1ull) != 0;
+        const bool nan = (key & 1ull) != 0 || scale->nanNode0;
         bool certified = false;
         if (cnt != TC_OVERFLOW && !nan && key != ~0ull)
         {
