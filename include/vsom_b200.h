@@ -178,7 +178,11 @@ VSOM_API int vsom_train_chunk_device(vsom_ctx *ctx, const float *x_dev, size_t n
 /* One chunk-epoch of the batch-map trainer: Som::trainBatchSomEpoch (src/Som.cpp:756-879).  Phase A finds every row's BMU
  * (is_first != 0: global search; else the local walk from last_bmu[row]), counts the hits and returns the mean squared
  * residual in *out_mse; phase B replaces every neuron by the incrementally weighted mean of all rows of the chunk (and its
- * sigma and weight).  last_bmu is in/out per row; x is n x d_in row-major on the host. */
+ * sigma and weight).  last_bmu is in/out per row; x is n x d_in row-major on the host.
+ * Limits: Standard / Median need Dm <= 5888; CLR needs P = d_in (d_in - 1) / 2 <= 2944 (d_in <= 77); rows of up to 6400
+ * values fit phase B's shared-memory row buffers.  A call past a limit returns VSOM_ERR_UNSUPPORTED and changes nothing: not
+ * the map, its hit counts or last_bmu.  Afterwards vsom_debug_last_score_tc reports phase A's search: K2's tier when a first
+ * epoch ran the tensor-core search (>= 1024 rows on a shape K2 covers), 0 for the exact scan and for the local walks. */
 VSOM_API int vsom_batch_epoch(vsom_ctx *ctx, const float *x, size_t n, double sigma, int is_first, uint64_t *last_bmu, float *out_mse);
 
 /* -------------------------------------------------------------------------------- scoring */

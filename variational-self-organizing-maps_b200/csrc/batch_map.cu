@@ -355,11 +355,50 @@ int launch_batch_epoch(vsom_ctx *ctx, const float *xDev, size_t n, double sigma,
         return set_error(ctx, VSOM_ERR_UNSUPPORTED, "batch-map trainer needs an unsharded context");
     if (n == 0)
         return VSOM_OK;
+    // ---- phase B's launch shape, first: a shape it cannot run is refused before anything is enqueued (no hits counted)
+    const int Dq = ctx->transform == VSOM_CLR ? ctx->P : ctx->Dm;
+    // chains per thread: the value that wastes the fewest lanes once T is rounded up to whole warps (ties: more chains per thread)
+    const int cptMax = ctx->transform == VSOM_CLR ? 4 : 8, cptMin = ctx->transform == VSOM_CLR ? 2 : 4;
+    int cpt = cptMin, T = 0;
+    long bestCost = -1;
+    for (int c = cptMin; c <= cptMax; ++c)
+    {
+        const int t = ((Dq + c - 1) / c + 31) / 32 * 32;
+        if (t > 736)
+            continue;
+        const long cost = static_cast<long>(t) * c;
+        if (bestCost < 0 || cost <= bestCost)
+        {
+            bestCost = cost;
+            cpt = c;
+            T = t;
+        }
+    }
+    if (bestCost < 0)
+        return set_error(ctx, VSOM_ERR_UNSUPPORTED, "batch-map trainer: model vector longer than 5888 components");
+    // neurons per CTA: as many as keep every SM busy in the fewest rounds (the rows are streamed once per CTA)
+    const int gMax = std::max(1, std::min(BM_MAXNB, 736 / T));
+    int G = 1;
+    long bestRounds = -1;
+    for (int gq = 1; gq <= gMax; ++gq)
+    {
+        const long ctas = (ctx->N + gq - 1) / gq, rounds = (ctas + ctx->numSMs - 1) / ctx->numSMs * gq;
+        if (bestRounds < 0 || rounds <= bestRounds)
+        {
+            bestRounds = rounds;
+            G = gq;
+        }
+    }
+    // rows per batch: two batches of rows in shared memory, at most 96 KB each
+    const int R = std::max(4, std::min(BM_ROWS, static_cast<int>((100 * 1024) / (sizeof(float) * ctx->Din)) & ~3));
+    if (sizeof(float) * 2 * R * ctx->Din > 208 * 1024)
+        return set_error(ctx, VSOM_ERR_UNSUPPORTED, "batch-map trainer: rows longer than 6400 values");
     int rc;
-    // ---- phase A
+    // ---- phase A; last_score_tc reports which search ran (K2's tier, or 0 for the exact scan and the local walks)
     if (isFirst)
     {
-        if (score_tc_supported(ctx) && n >= 1024)
+        ctx->lastScoreTc = score_tc_supported(ctx) && n >= 1024;
+        if (ctx->lastScoreTc)
             rc = launch_find_bmu_tc(ctx, xDev, n, 0, bmuDev, distDev, nullptr);
         else
             rc = launch_find_bmu(ctx, xDev, n, 0, bmuDev, distDev);
@@ -368,6 +407,7 @@ int launch_batch_epoch(vsom_ctx *ctx, const float *xDev, size_t n, double sigma,
     }
     else
     {
+        ctx->lastScoreTc = 0;
         const unsigned grid = static_cast<unsigned>((n + 31) / 32);
         if (ctx->transform == VSOM_CLR)
             local_bmu_rows_kernel<VSOM_CLR><<<grid, 256, 0, ctx->stream>>>(xDev, n, ctx->mean, ctx->W, ctx->H, ctx->Din, ctx->Dr, ctx->P, ctx->rowStride,
@@ -407,43 +447,6 @@ int launch_batch_epoch(vsom_ctx *ctx, const float *xDev, size_t n, double sigma,
     VSOM_CUDA(ctx, cudaMemcpyAsync(lutDev, lutHost.data(), sizeof(float) * lutHost.size(), cudaMemcpyHostToDevice, ctx->stream));
     VSOM_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); // lutHost is a local
     bmu_xy_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, ctx->stream>>>(bmuDev, n, ctx->W, ctx->H, xyDev);
-    const int Dq = ctx->transform == VSOM_CLR ? ctx->P : ctx->Dm;
-    // chains per thread: the value that wastes the fewest lanes once T is rounded up to whole warps (ties: more chains per thread)
-    const int cptMax = ctx->transform == VSOM_CLR ? 4 : 8, cptMin = ctx->transform == VSOM_CLR ? 2 : 4;
-    int cpt = cptMin, T = 0;
-    long bestCost = -1;
-    for (int c = cptMin; c <= cptMax; ++c)
-    {
-        const int t = ((Dq + c - 1) / c + 31) / 32 * 32;
-        if (t > 736)
-            continue;
-        const long cost = static_cast<long>(t) * c;
-        if (bestCost < 0 || cost <= bestCost)
-        {
-            bestCost = cost;
-            cpt = c;
-            T = t;
-        }
-    }
-    if (bestCost < 0)
-        return set_error(ctx, VSOM_ERR_UNSUPPORTED, "batch-map trainer: model vector longer than 5888 components");
-    // neurons per CTA: as many as keep every SM busy in the fewest rounds (the rows are streamed once per CTA)
-    const int gMax = std::max(1, std::min(BM_MAXNB, 736 / T));
-    int G = 1;
-    long bestRounds = -1;
-    for (int gq = 1; gq <= gMax; ++gq)
-    {
-        const long ctas = (ctx->N + gq - 1) / gq, rounds = (ctas + ctx->numSMs - 1) / ctx->numSMs * gq;
-        if (bestRounds < 0 || rounds <= bestRounds)
-        {
-            bestRounds = rounds;
-            G = gq;
-        }
-    }
-    // rows per batch: two batches of rows in shared memory, at most 96 KB each
-    const int R = std::max(4, std::min(BM_ROWS, static_cast<int>((100 * 1024) / (sizeof(float) * ctx->Din)) & ~3));
-    if (sizeof(float) * 2 * R * ctx->Din > 208 * 1024)
-        return set_error(ctx, VSOM_ERR_UNSUPPORTED, "batch-map trainer: rows longer than 6400 values");
     const unsigned grid = static_cast<unsigned>((ctx->N + G - 1) / G);
     const unsigned threads = static_cast<unsigned>(G * T + 32);
     const int lutN = lutHost.size() <= static_cast<size_t>(BM_LUT_SMEM) ? static_cast<int>(lutHost.size()) : 0;
