@@ -1,6 +1,6 @@
 """Small driver for ncu captures of the tensor-core scoring kernel (not a test): scores n rows twice against a 128x128x256
 map (random init, or trained with a decaying sigma when the second argument is "trained").
-Usage: [VSOM_TC_TIER=1|2] [VSOM_TC_PAIR=0|1] [VSOM_TC_STAGGER=3 -> pipeline only] python tests/profile_k2.py [rows] [random|trained]"""
+Usage: [VSOM_TC_TIER=1|2] [VSOM_TC_PAIR=0|1] python tests/profile_k2.py [rows] [random|trained]"""
 import importlib
 import sys
 import time

@@ -109,8 +109,7 @@ static int create_impl(vsom_ctx **out, int device, int width, int height, int d_
         // Node sharding: grid rows are dealt to the ranks round-robin in blocks of shardBlock rows (block b -> rank b % world).
         // Contiguous bands (SURVEY.md §8e's first proposal) put a whole update window (80 x 80 nodes at sigma = 16 on a
         // 512 x 512 map) on one or two GPUs; small blocks spread it over all of them, at the price of more U-matrix halo rows.
-        const char *e = getenv("VSOM_SHARD_BLOCK_ROWS");
-        int block = world == 1 ? height : (e && atoi(e) > 0 ? atoi(e) : 4);
+        int block = world == 1 ? height : 4;
         if (world > 1 && block * world > height)
             block = height / world; // every rank holds at least one row (world <= height was checked above)
         ctx->shardBlock = block;
@@ -890,7 +889,7 @@ int vsom_soft_assign(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits,
     return VSOM_OK;
 }
 
-// per-grid-row pointer tables of K4 (umatrix.cu): [H] mean rows, [H] sigma rows, [localRows] grid rows to compute.  A
+// per-grid-row pointer tables of K4 (umatrix.cu): [H] mean rows, [H] sigma rows, then the tiles to compute.  A
 // node-sharded context reads its neighbours' border rows straight out of the owners' planes (peer-mapped pointers).
 static int umatrix_tables(vsom_ctx *ctx)
 {
@@ -899,31 +898,26 @@ static int umatrix_tables(vsom_ctx *ctx)
     const int H = ctx->H;
     const size_t rowFloats = static_cast<size_t>(ctx->W) * ctx->rowStride;
     std::vector<const float *> rows(2 * static_cast<size_t>(H), nullptr);
-    std::vector<int> halo; // grid rows of other ranks that border this rank's rows
     for (int lr = 0; lr < ctx->localRows; ++lr)
     {
         const int y = ctx->localRowY[lr];
         rows[y] = ctx->mean + lr * rowFloats;
         rows[H + y] = ctx->sigma + lr * rowFloats;
     }
+    // Halo rows (grid rows of other ranks that border this rank's rows) are not copied: their table entries point INTO the
+    // owner's mean plane (peer-mapped over NVLink), and the kernels' cp.async copies read them from there while they
+    // compute — one border row of means per neighbouring block (sigma is the centre's own, SURVEY.md §8e).
     for (int lr = 0; lr < ctx->localRows; ++lr)
         for (int dy = -1; dy <= 1; dy += 2)
         {
             const int y = ctx->localRowY[lr] + dy;
-            if (y >= 0 && y < H && !rows[y] && std::find(halo.begin(), halo.end(), y) == halo.end())
-                halo.push_back(y);
+            if (y < 0 || y >= H || rows[y])
+                continue;
+            const int owner = (y / ctx->shardBlock) % ctx->world, ly = shard_local_row(y, ctx->shardBlock, owner, ctx->world);
+            if (!ctx->peerMean[owner])
+                return set_error(ctx, VSOM_ERR_INVALID, "vsom_update_umatrix: sharded context without vsom_peer_import_planes / vsom_peer_attach for every rank");
+            rows[y] = ctx->peerMean[owner] + ly * rowFloats;
         }
-    // Halo rows are not copied: their table entries point INTO the owner's mean plane (peer-mapped over NVLink), and the
-    // tiled kernel's cp.async copies read them from there while it computes — one border row of means per neighbouring
-    // block (sigma is the centre's own, SURVEY.md §8e).
-    for (int y : halo)
-    {
-        const int owner = (y / ctx->shardBlock) % ctx->world, lr = shard_local_row(y, ctx->shardBlock, owner, ctx->world);
-        if (!ctx->peerMean[owner])
-            return set_error(ctx, VSOM_ERR_INVALID, "vsom_update_umatrix: sharded context without vsom_peer_import_planes / vsom_peer_attach for every rank");
-        rows[y] = ctx->peerMean[owner] + lr * rowFloats;
-    }
-    ctx->haloRows = halo;
     // tiles of the tiled kernel: runs of at most umatrix_tile_rows() consecutive grid rows this context owns
     std::vector<int2> tiles;
     for (int lr = 0; lr < ctx->localRows;)
@@ -934,12 +928,10 @@ static int umatrix_tables(vsom_ctx *ctx)
         tiles.push_back(make_int2(ctx->localRowY[lr], rows_));
         lr += rows_;
     }
-    const size_t ptrBytes = sizeof(float *) * rows.size(), rowBytes = sizeof(int) * ctx->localRowY.size();
-    VSOM_CUDA(ctx, cudaMalloc(&ctx->umTab, ptrBytes + rowBytes + sizeof(int2) * tiles.size() + 16));
+    const size_t ptrBytes = sizeof(float *) * rows.size();
+    VSOM_CUDA(ctx, cudaMalloc(&ctx->umTab, ptrBytes + sizeof(int2) * tiles.size()));
     VSOM_CUDA(ctx, cudaMemcpy(ctx->umTab, rows.data(), ptrBytes, cudaMemcpyHostToDevice));
-    VSOM_CUDA(ctx, cudaMemcpy(static_cast<unsigned char *>(ctx->umTab) + ptrBytes, ctx->localRowY.data(), rowBytes, cudaMemcpyHostToDevice));
-    VSOM_CUDA(ctx, cudaMemcpy(static_cast<unsigned char *>(ctx->umTab) + ptrBytes + ((rowBytes + 7) & ~size_t{7}), tiles.data(), sizeof(int2) * tiles.size(), cudaMemcpyHostToDevice));
-    ctx->umRows = ctx->localRows;
+    VSOM_CUDA(ctx, cudaMemcpy(static_cast<unsigned char *>(ctx->umTab) + ptrBytes, tiles.data(), sizeof(int2) * tiles.size(), cudaMemcpyHostToDevice));
     ctx->umTiles = static_cast<int>(tiles.size());
     return VSOM_OK;
 }
@@ -953,13 +945,7 @@ int vsom_update_umatrix(vsom_ctx *ctx, double *out)
     if (rc)
         return rc;
     const float *const *meanRows = static_cast<const float *const *>(ctx->umTab);
-    const int *rowsDev = reinterpret_cast<const int *>(meanRows + 2 * ctx->H);
-    const char *kenv = getenv("VSOM_UMATRIX_KERNEL"); // "rows": the one-thread-per-pair kernel without shared-memory tiles (A/B measurements)
-    if (kenv && std::string(kenv) == "rows")
-        rc = launch_umatrix_rows(ctx, meanRows, meanRows + ctx->H, rowsDev, ctx->umRows);
-    else
-        rc = launch_umatrix_tiles(ctx, meanRows, meanRows + ctx->H,
-                                  reinterpret_cast<const int2 *>(reinterpret_cast<const unsigned char *>(rowsDev) + ((sizeof(int) * ctx->localRowY.size() + 7) & ~size_t{7})), ctx->umTiles);
+    rc = launch_umatrix_tiles(ctx, meanRows, meanRows + ctx->H, reinterpret_cast<const int2 *>(meanRows + 2 * ctx->H), ctx->umTiles);
     if (rc)
         return rc;
     if (out) // full-map array; a sharded context fills in its own grid rows only

@@ -71,7 +71,7 @@ struct StepParams
     int *rowOf;               // [G] row (die * 160 + slot) every CTA claimed in this launch
     unsigned *rowCtr;         // [0..1] rows claimed per die, [2] arrivals at the one-off grid barrier
     u64 *rowPool;
-    int pollDelay;            // cycles between the pushes and the first poll
+    int pollDelay;            // cycles between the pushes and the first poll: 0 in every launch (without the wait, ptxas gives K1F's PROF builds a register more)
     u64 *distTag;             // K1F, sigma <= 1: [2][N] (distance bits << 32 | step + 1) of every node, self-validating words
     int scanBufs, scanSeg, scanNSeg; // K1 on HBM-resident rows: streamed scan (ring of scanBufs buffers of 32 row segments of scanSeg floats)
     const void *scanMap;      // ... its TMA descriptor of the mean plane (device memory)
@@ -89,7 +89,6 @@ struct vsom_ctx
     std::vector<int> localRowY;   // global grid row of every local row
     float *peerMean[8] = {};      // mean planes of the ranks (U-matrix halo rows), peer-mapped; peerMean[rank] == mean
     bool peerMeanOpened[8] = {};
-    std::vector<int> haloRows;    // grid rows of other ranks that border this rank's rows (read in place for the U-matrix)
     vsom::u64 *rankSlots = nullptr;
     vsom::u64 *peerSlots[8] = {};
     bool peerOpened[8] = {};
@@ -148,8 +147,8 @@ struct vsom_ctx
     vsom::u64 *distTag = nullptr; // K1F local-walk regime: tagged per-step distances
     int scanBufs = 0, scanSeg = 0, scanNSeg = 0; // K1: HBM-resident rows are streamed through a ring of segment buffers
     void *scanMapDev = nullptr;                   // TMA descriptor of the mean plane for that scan
-    void *umTab = nullptr;        // K4: per-grid-row pointer tables (mean rows, sigma rows) + the grid rows this context computes
-    int umRows = 0, umTiles = 0;
+    void *umTab = nullptr;        // K4: per-grid-row pointer tables (mean rows, sigma rows) + the tiles this context computes
+    int umTiles = 0;
     long long *profDev = nullptr; // diagnostics: per-phase cycle sums of the last online-step launch
     size_t profSamples = 0;
     std::string err;
@@ -191,7 +190,6 @@ int launch_similarity_rowmax(vsom_ctx *ctx, const float *xDev, size_t rows, cons
 int similarity_hook(vsom_ctx *ctx, const float *xDev, size_t rows, const unsigned *bmuDev, size_t rowInCall, cudaStream_t stream);
 int launch_umatrix_tiles(vsom_ctx *ctx, const float *const *meanRowDev, const float *const *sigmaRowDev, const int2 *tilesDev, int nTiles);
 int umatrix_tile_rows();
-int launch_umatrix_rows(vsom_ctx *ctx, const float *const *meanRowDev, const float *const *sigmaRowDev, const int *rowsDev, int nRows);
 int launch_build_index(vsom_ctx *ctx, const unsigned *bmuDev, size_t n, u64 *countsDev, u64 *offsetsDev, unsigned *rowIdsDev);
 
 // ------------------------------------------------------------------------------------------ device helpers

@@ -1258,7 +1258,7 @@ static int calibrate_die_map(vsom_ctx *ctx)
     cudaFree(smids);
     float thr = 0.f;
     const bool bimodal = ok && split_bimodal(rt, thr);
-    if (getenv("VSOM_DEBUG_DIE") || !bimodal)
+    if (!bimodal)
     {
         std::vector<float> srt = rt;
         std::sort(srt.begin(), srt.end());
@@ -1335,7 +1335,7 @@ static int build_row_pool(vsom_ctx *ctx)
             for (float v : rt)
                 complete = complete && v > 0.f;
             const bool bimodal = complete && split_bimodal(rt, thr);
-            if (getenv("VSOM_DEBUG_DIE") || !bimodal)
+            if (!bimodal)
             {
                 std::vector<float> srt = rt;
                 std::sort(srt.begin(), srt.end());
@@ -1409,17 +1409,8 @@ int configure_online_step_fast(vsom_ctx *ctx)
     if (Lmax > kFThreads)
         return 0; // one scan lane per owned node
     // Eigen order: eight lanes per node cut the chain from Dr to Dr / 8 dependent adds; worth it when the rows are long or when
-    // all the CTA's nodes still fit one warp (no extra CTA-level reduction).  VSOM_K1F_LANES=1|8 overrides (experiments).
-    {
-        const int Dr = ctx->Dr;
-        int lpn = 1;
-        if (ctx->order == VSOM_ORDER_EIGEN_SSE && Lmax * 8 <= kFThreads && (Lmax * 8 <= 32 || Dr >= 256))
-            lpn = 8;
-        if (const char *e = getenv("VSOM_K1F_LANES"))
-            if (ctx->order == VSOM_ORDER_EIGEN_SSE && Lmax * 8 <= kFThreads && (atoi(e) == 1 || atoi(e) == 8))
-                lpn = atoi(e);
-        ctx->fastLanes = lpn;
-    }
+    // all the CTA's nodes still fit one warp (no extra CTA-level reduction).
+    ctx->fastLanes = ctx->order == VSOM_ORDER_EIGEN_SSE && Lmax * 8 <= kFThreads && (Lmax * 8 <= 32 || ctx->Dr >= 256) ? 8 : 1;
     const int ipw = fast_ipw(ctx, G);
     for (int prof = 0; prof < 2; ++prof)
     {
@@ -1493,10 +1484,6 @@ int launch_online_step_fast(vsom_ctx *ctx, StepParams &p, double sigma)
     VSOM_CUDA(ctx, cudaMemsetAsync(ctr, 0, sizeof(unsigned) * 4, ctx->stream));
     VSOM_CUDA(ctx, cudaMemsetAsync(ctx->errFlag, 0, sizeof(int), ctx->stream));
     p.winTab = ctx->winTab;
-    {
-        const char *e = getenv("VSOM_POLL_DELAY"); // experiment knob: cycles to wait between the pushes and the first poll
-        p.pollDelay = e ? atoi(e) : 0;
-    }
     p.dieOfSm = ctx->rowMeta;
     p.rowBlocks = ctx->rowMeta + 256;
     p.rowOf = ctx->rowMeta + 256 + 2 * 2 * kFMaxCtas;

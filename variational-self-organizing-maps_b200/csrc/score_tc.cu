@@ -995,8 +995,8 @@ bool score_tc_supported(const vsom_ctx *ctx) { return ctx->transform != VSOM_CLR
 // stage slots used: 6 = fp16 map operand + statistics, 7 = fp16 rows of the current slab, 8 = per-row scratch (two sets).
 struct TcCall
 {
-    int D = 0, N = 0, Kpad = 0, kBlocks = 0, kSteps = 0, Npad = 0, nodeTiles = 0, stagger = 1, split = 0;
-    bool overlap = true, pair = true;
+    int D = 0, N = 0, Kpad = 0, kBlocks = 0, kSteps = 0, Npad = 0, nodeTiles = 0, split = 0;
+    bool pair = true;
     uint64_t minHits = 0;
     size_t slabRows = 0, setBytes = 0, slab = 0;
     __half *Xb = nullptr;
@@ -1066,9 +1066,6 @@ static int tc_begin(vsom_ctx *ctx, TcCall &c, size_t maxSlabRows, uint64_t minHi
     // stream converts a slab and runs the tensor-core search; an auxiliary stream re-scores the slab's candidates (and scans
     // the few rows the certificate rejected) while the next slab is already being searched.  Candidate scratch is
     // double-buffered by slab parity; nothing returns to the host in between.
-    const char *ovlEnv = getenv("VSOM_TC_OVERLAP"), *stg = getenv("VSOM_TC_STAGGER"); // experiment knobs
-    c.overlap = ovlEnv ? atoi(ovlEnv) != 0 : true;
-    c.stagger = stg ? atoi(stg) : 1;
     c.slabRows = maxSlabRows;
     rc = stage_reserve(ctx, 7, sizeof(__half) * c.slabRows * c.Kpad);
     if (rc)
@@ -1151,10 +1148,11 @@ static int tc_enqueue(vsom_ctx *ctx, TcCall &c, const float *xs, size_t rows, un
         const int rowsI = static_cast<int>(rows);
         const float *xn = xnorm, *xr = xratio;
         const TcScale *sc = c.scale;
-        VSOM_CUDA(ctx, cudaLaunchKernelEx(&cfg, c.pair ? score_tc_kernel<true> : score_tc_kernel<false>, mapX, c.mapM, c.kSteps, rowsI, rowTiles, c.nodeTiles, c.kBlocks, c.Kpad, c.stagger, c.D,
+        // the kernel's debug word is 1: staggered node-tile starts, none of the timing-only variants
+        VSOM_CUDA(ctx, cudaLaunchKernelEx(&cfg, c.pair ? score_tc_kernel<true> : score_tc_kernel<false>, mapX, c.mapM, c.kSteps, rowsI, rowTiles, c.nodeTiles, c.kBlocks, c.Kpad, 1, c.D,
                                           xn, xr, sc, cand, candCount, bestA, ctx->errFlag));
     }
-    cudaStream_t rs = c.overlap ? ctx->auxStream : ctx->stream;
+    cudaStream_t rs = ctx->auxStream;
     VSOM_CUDA(ctx, cudaEventRecord(ctx->evScore[par], ctx->stream));
     VSOM_CUDA(ctx, cudaStreamWaitEvent(rs, ctx->evScore[par], 0));
     rescore_kernel<<<static_cast<unsigned>((rows + RS_ROWS - 1) / RS_ROWS), RS_THREADS, 0, rs>>>(xs, static_cast<long long>(rows), c.D, ctx->mean, ctx->rowStride, cand, candCount, bestA,
@@ -1218,10 +1216,51 @@ static size_t tc_slab_cap(const vsom_ctx *ctx, int split)
     return std::max<size_t>(TC_BM, ((size_t{5} << 29) / (kpad * 2)) & ~static_cast<size_t>(TC_BM - 1));
 }
 
-static int tc_forced_tier()
+// The tier policy of both forms.  run(r0, rows, tier, fb) scores rows [r0, r0 + rows) through tier 1 or 2 and sets fb to the
+// number of them that took the exact scan.  On return `done` rows have been scored (all n, unless the tier-2 probe chose
+// tier 3: then rows [done, n) are left to the caller's exact scan) and `fallback` of them took the exact scan.
+template <class Run>
+static int tc_score_tiers(vsom_ctx *ctx, size_t n, const Run &run, size_t &done, unsigned long long &fallback)
 {
     const char *e = getenv("VSOM_TC_TIER");
-    return e ? atoi(e) : 0;
+    const int forced = e ? atoi(e) : 0;
+    int tier = forced;
+    unsigned long long fb = 0;
+    done = 0;
+    fallback = 0;
+    if (tier != 1 && tier != 2)
+    {
+        // probe: the first rows through tier 1 (their results stand), then decide
+        done = std::min(n, kTcProbeRows);
+        const int rc = run(0, done, 1, fb);
+        if (rc)
+            return rc;
+        fallback += fb;
+        tier = static_cast<double>(fb) > kTcTierSwitch * static_cast<double>(done) ? 2 : 1;
+    }
+    if (tier == 2 && !forced && n - done > kTcProbeRows)
+    {
+        // second probe: the next rows through tier 2 (their results stand).  Data whose norms dwarf the map's (or a map whose nodes
+        // nearly coincide) leaves more candidates than the lists hold even at 2^-20: the remainder goes straight to the exact scan
+        const int rc = run(done, kTcProbeRows, 2, fb);
+        if (rc)
+            return rc;
+        fallback += fb;
+        done += kTcProbeRows;
+        if (static_cast<double>(fb) > kTcExactSwitch * static_cast<double>(kTcProbeRows))
+            tier = 3;
+    }
+    ctx->lastScoreTier = tier;
+    if (done < n && tier != 3)
+    {
+        const int rc = run(done, n - done, tier, fb);
+        if (rc)
+            return rc;
+        fallback += fb;
+        done = n;
+    }
+    ctx->lastFallbackRows = fallback;
+    return VSOM_OK;
 }
 
 // rows [0, n) of xDev through one tier; slabs of the given size
@@ -1250,53 +1289,30 @@ int launch_find_bmu_tc(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minH
         *fallbackRowsOut = 0;
     if (n == 0)
         return VSOM_OK;
-    const char *slabEnv = getenv("VSOM_TC_SLAB_LOG2"); // experiment knob; smaller slabs measured slower (per-slab ramp and tail of the persistent kernel)
+    // test knob; smaller slabs measured slower (per-slab ramp and tail of the persistent kernel)
+    const char *slabEnv = getenv("VSOM_TC_SLAB_LOG2");
     const size_t slab1 = static_cast<size_t>(1) << (slabEnv ? atoi(slabEnv) : 22), slab2 = std::min<size_t>(slab1, static_cast<size_t>(1) << 20);
-    int tier = tc_forced_tier();
     size_t done = 0;
-    unsigned long long fb = 0, total = 0;
-    if (tier != 1 && tier != 2)
+    unsigned long long total = 0;
+    int rc = tc_score_tiers(
+        ctx, n,
+        [&](size_t r0, size_t rows, int tier, unsigned long long &fb) {
+            return tc_run_device(ctx, xDev + r0 * ctx->Dm, rows, minHits, tier == 2 ? 1 : 0, tier == 2 ? slab2 : slab1, outBmuDev ? outBmuDev + r0 : nullptr,
+                                 outDistDev ? outDistDev + r0 : nullptr, &fb);
+        },
+        done, total);
+    if (rc)
+        return rc;
+    if (done < n) // tier 3
     {
-        // probe: the first rows through tier 1 (their results stand), then decide
-        done = std::min(n, kTcProbeRows);
-        const int rc = tc_run_device(ctx, xDev, done, minHits, 0, slab1, outBmuDev, outDistDev, &fb);
-        if (rc)
-            return rc;
-        total += fb;
-        tier = static_cast<double>(fb) > kTcTierSwitch * static_cast<double>(done) ? 2 : 1;
-    }
-    if (tier == 2 && !tc_forced_tier() && n - done > kTcProbeRows)
-    {
-        // second probe: the next rows through tier 2 (their results stand).  Data whose norms dwarf the map's (or a map whose nodes
-        // nearly coincide) leaves more candidates than the lists hold even at 2^-20: the remainder goes straight to the exact scan
-        const int rc = tc_run_device(ctx, xDev + done * ctx->Dm, kTcProbeRows, minHits, 1, slab2, outBmuDev ? outBmuDev + done : nullptr,
-                                     outDistDev ? outDistDev + done : nullptr, &fb);
-        if (rc)
-            return rc;
-        total += fb;
-        done += kTcProbeRows;
-        if (static_cast<double>(fb) > kTcExactSwitch * static_cast<double>(kTcProbeRows))
-            tier = 3;
-    }
-    ctx->lastScoreTier = tier;
-    if (done < n && tier == 3)
-    {
-        const int rc = launch_find_bmu(ctx, xDev + done * ctx->Dm, n - done, minHits, outBmuDev ? outBmuDev + done : nullptr, outDistDev ? outDistDev + done : nullptr);
+        rc = launch_find_bmu(ctx, xDev + done * ctx->Dm, n - done, minHits, outBmuDev ? outBmuDev + done : nullptr, outDistDev ? outDistDev + done : nullptr);
         if (rc)
             return rc;
         total += n - done;
-    }
-    else if (done < n)
-    {
-        const int rc = tc_run_device(ctx, xDev + done * ctx->Dm, n - done, minHits, tier == 2 ? 1 : 0, tier == 2 ? slab2 : slab1, outBmuDev ? outBmuDev + done : nullptr,
-                                     outDistDev ? outDistDev + done : nullptr, &fb);
-        if (rc)
-            return rc;
-        total += fb;
+        ctx->lastFallbackRows = total;
     }
     if (fallbackRowsOut)
         *fallbackRowsOut = total;
-    ctx->lastFallbackRows = total;
     return VSOM_OK;
 }
 
@@ -1351,7 +1367,7 @@ static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t min
         rc = tc_enqueue(ctx, c, xbuf[b], rows, bmuDev + r0, distDev + r0, outBmuHost ? outBmuHost + r0 : nullptr, outDistHost ? outDistHost + r0 : nullptr, r0, true);
         if (rc)
             return rc;
-        VSOM_CUDA(ctx, cudaEventRecord(ctx->evSlabDone[b], c.overlap ? ctx->auxStream : ctx->stream)); // behind the slab's re-scoring and result copies
+        VSOM_CUDA(ctx, cudaEventRecord(ctx->evSlabDone[b], ctx->auxStream)); // behind the slab's re-scoring and result copies
         // up to two copies ahead, enqueued AFTER the search of slab sl: a pageable source blocks the host here, not the device
         while (issued < std::min(slabs, sl + 3))
         {
@@ -1381,45 +1397,22 @@ int launch_find_bmu_tc_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_
         return VSOM_OK;
     const char *slabEnv = getenv("VSOM_TC_HOST_SLAB_LOG2");
     const size_t slabRows = static_cast<size_t>(1) << (slabEnv ? atoi(slabEnv) : 19);
-    int tier = tc_forced_tier();
     size_t done = 0;
-    unsigned long long fb = 0, total = 0;
-    if (tier != 1 && tier != 2)
-    {
-        done = std::min(n, kTcProbeRows);
-        const int rc = tc_run_host(ctx, xHost, done, minHits, 0, slabRows, outBmuHost, outDistHost, &fb);
-        if (rc)
-            return rc;
-        total += fb;
-        tier = static_cast<double>(fb) > kTcTierSwitch * static_cast<double>(done) ? 2 : 1;
-    }
-    if (tier == 2 && !tc_forced_tier() && n - done > kTcProbeRows)
-    {
-        const int rc = tc_run_host(ctx, xHost + done * ctx->Dm, kTcProbeRows, minHits, 1, slabRows, outBmuHost ? outBmuHost + done : nullptr,
-                                   outDistHost ? outDistHost + done : nullptr, &fb);
-        if (rc)
-            return rc;
-        total += fb;
-        done += kTcProbeRows;
-        if (static_cast<double>(fb) > kTcExactSwitch * static_cast<double>(kTcProbeRows))
-            tier = 3;
-    }
-    ctx->lastScoreTier = tier;
-    if (done < n && tier != 3)
-    {
-        const int rc = tc_run_host(ctx, xHost + done * ctx->Dm, n - done, minHits, tier == 2 ? 1 : 0, slabRows, outBmuHost ? outBmuHost + done : nullptr,
-                                   outDistHost ? outDistHost + done : nullptr, &fb);
-        if (rc)
-            return rc;
-        total += fb;
-        done = n;
-    }
+    unsigned long long total = 0;
+    const int rc = tc_score_tiers(
+        ctx, n,
+        [&](size_t r0, size_t rows, int tier, unsigned long long &fb) {
+            return tc_run_host(ctx, xHost + r0 * ctx->Dm, rows, minHits, tier == 2 ? 1 : 0, slabRows, outBmuHost ? outBmuHost + r0 : nullptr,
+                               outDistHost ? outDistHost + r0 : nullptr, &fb);
+        },
+        done, total);
+    if (rc)
+        return rc;
     // tier 3: rows [done, n) are left to the caller's exact path
     if (rowsDoneOut)
         *rowsDoneOut = done;
     if (fallbackRowsOut)
         *fallbackRowsOut = total;
-    ctx->lastFallbackRows = total;
     return VSOM_OK;
 }
 
