@@ -5,6 +5,7 @@
 //   evaluate / measureSimilarity / mapDataSet         -> vsom_find_bmu / vsom_evaluate: batches of >= 1024 rows run the
 //                                                        tensor-core candidate search + exact rescore (K2), smaller ones
 //                                                        the exact scan (K3); same bits either way
+//   mapDataSetTopTwo / topographicError (additions)   -> vsom_find_bmu2 (K2 / K3 in their top-2 mode)
 //   findBmu / findRestrictedBmu (one row)             -> vsom_find_bmu      (K3)
 //   euclidianWeightedDist / findLocalBmu / findRestrictedBmd -> vsom_all_dists
 //   variationalAutoEncoder / autoEncoder              -> vsom_soft_assign + host sampling
@@ -154,6 +155,13 @@ class Som
     // ---- additions of this implementation (not in the reference)
     // Batch scoring of the loaded chunk in one device pass: BMU index and distance per row.
     void mapDataSet(const DataSet &dataset, std::vector<size_t> &bmuOut, std::vector<float> &distOut, size_t minBmuHits = 0) const;
+    // The same pass with every row's second-best node as well (vsom_find_bmu2): bmuOut / distOut as mapDataSet, bmu2Out / dist2Out the
+    // runner-up among the eligible nodes (smallest (distance, index) key, NaN distances last); SIZE_MAX and NaN for rows without one.
+    void mapDataSetTopTwo(const DataSet &dataset, std::vector<size_t> &bmuOut, std::vector<float> &distOut, std::vector<size_t> &bmu2Out,
+                          std::vector<float> &dist2Out, size_t minBmuHits = 0) const;
+    // Topographic error of the loaded chunk (min_hits 0): the share of rows whose best and second-best nodes are not 8-neighbours
+    // on the grid (max(|dx|, |dy|) == 1, no wrap-around); rows without a runner-up (a 1 x 1 map) are not errors.  0 for an empty chunk.
+    double topographicError(const DataSet &dataset) const;
     // Rows grouped by BMU: counts[N], offsets[N+1], rowIds[n] (the "SomIndex build").
     void buildIndex(const std::vector<size_t> &bmu, std::vector<size_t> &counts, std::vector<size_t> &offsets, std::vector<unsigned> &rowIds) const;
     // Summation order of the distances (vsom_reduction_order of vsom_b200.h): 0 sequential, 1 lanes (online step only, near-tie

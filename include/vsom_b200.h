@@ -207,6 +207,26 @@ VSOM_API int vsom_find_bmu_exact_device(vsom_ctx *ctx, const float *x_dev, size_
 VSOM_API int vsom_find_bmu_batch(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist, uint64_t *fallback_rows);
 VSOM_API int vsom_find_bmu_batch_device(vsom_ctx *ctx, const float *x_dev, size_t n, uint64_t min_hits, uint32_t *out_bmu_dev, float *out_dist_dev,
                                         uint64_t *fallback_rows);
+/* Best AND second-best matching node of every row — what the topographic error needs.  out_bmu / out_dist are exactly what
+ * vsom_find_bmu returns for the same rows and min_hits (the NaN-at-node-0 rule included).  out_bmu2 / out_dist2: the eligible
+ * node (hits >= min_hits, or node 0) other than out_bmu with the smallest (distance, index) key — a smaller distance wins,
+ * equal distances go to the lower index, a NaN distance ranks after every number (lower index first among NaNs).  A row
+ * without such a node (one node, or one eligible node) gets out_bmu2 = 0xFFFFFFFF and a NaN out_dist2.  Every output may be
+ * NULL; fallback_rows (may be NULL) as in vsom_find_bmu_batch.
+ * Topographic error of n rows: the share of rows whose out_bmu and out_bmu2 are not 8-neighbours on the rectangular,
+ * non-wrapping grid (max(|dx|, |dy|) == 1, diagonals included: the U-matrix's neighbourhood); rows without a runner-up are
+ * not errors.  Som::topographicError (include/SOM.hpp) computes it from these outputs.
+ * Dispatch and tiers as vsom_find_bmu: >= 1024 rows on a shape K2 covers run the tensor-core search in its top-2 mode (the list
+ * threshold follows an upper bound of the second-smallest approximate score, and the certificate must clear the runner-up's
+ * exact distance), everything else the exact scan.  vsom_debug_last_score_tc / _pair / _tc_stats report these calls like
+ * vsom_find_bmu's.  Node-sharded contexts return VSOM_ERR_UNSUPPORTED. */
+VSOM_API int vsom_find_bmu2(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist, uint32_t *out_bmu2,
+                            float *out_dist2, uint64_t *fallback_rows);
+VSOM_API int vsom_find_bmu2_device(vsom_ctx *ctx, const float *x_dev, size_t n, uint64_t min_hits, uint32_t *out_bmu_dev, float *out_dist_dev,
+                                   uint32_t *out_bmu2_dev, float *out_dist2_dev, uint64_t *fallback_rows);
+/* Same contract, always the exact scan (K3) — what the tests compare the dispatching calls with. */
+VSOM_API int vsom_find_bmu2_exact(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist, uint32_t *out_bmu2,
+                                  float *out_dist2);
 /* 0 when the last scoring call on ctx ran the exact scan, else the precision tier of its tensor-core search: 1 = one fp16
  * value per operand element, 2 = hi / lo pairs (three products per element; chosen when a probe of the first rows shows that
  * tier 1 cannot separate the BMU from its neighbours on this map), 3 = both probes (8192 rows each, whose results stand)

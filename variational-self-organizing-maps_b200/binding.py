@@ -58,6 +58,9 @@ _PROTOS = {
     "vsom_debug_tc_stats": (C.c_int, [_vp, _u64p]),
     "vsom_find_bmu_batch": (C.c_int, [_vp, _f32p, C.c_size_t, C.c_uint64, _u32p, _f32p, _u64p]),
     "vsom_find_bmu_batch_device": (C.c_int, [_vp, _vp, C.c_size_t, C.c_uint64, _vp, _vp, _u64p]),
+    "vsom_find_bmu2": (C.c_int, [_vp, _f32p, C.c_size_t, C.c_uint64, _u32p, _f32p, _u32p, _f32p, _u64p]),
+    "vsom_find_bmu2_device": (C.c_int, [_vp, _vp, C.c_size_t, C.c_uint64, _vp, _vp, _vp, _vp, _u64p]),
+    "vsom_find_bmu2_exact": (C.c_int, [_vp, _f32p, C.c_size_t, C.c_uint64, _u32p, _f32p, _u32p, _f32p]),
     "vsom_evaluate": (C.c_int, [_vp, _f32p, C.c_size_t, _f64p]),
     "vsom_measure_similarity": (C.c_int, [_vp, _f32p, C.c_size_t, C.c_uint64, C.c_int, _u32p, _f32p]),
     "vsom_soft_assign": (C.c_int, [_vp, _f32p, C.c_size_t, C.c_uint64, _f64p]),
@@ -268,6 +271,35 @@ class VsomContext:
                                                      out_bmu_dev.data_ptr() if out_bmu_dev is not None else None,
                                                      out_dist_dev.data_ptr() if out_dist_dev is not None else None, C.byref(fb)))
         return int(fb.value)
+
+    def find_bmu2(self, x, min_hits=0):
+        """Best and second-best matching node of every row: (bmu, dist, bmu2, dist2, rows that took the exact full scan).
+        bmu2 is 0xFFFFFFFF and dist2 NaN where a row has no runner-up."""
+        x = _f32(x).reshape(-1, self.Din)
+        n = x.shape[0]
+        bmu, bmu2 = np.empty(n, np.uint32), np.empty(n, np.uint32)
+        dist, dist2 = np.empty(n, np.float32), np.empty(n, np.float32)
+        fb = C.c_uint64(0)
+        self._check(lib().vsom_find_bmu2(self._h, _p(x, _f32p), n, min_hits, _p(bmu, _u32p), _p(dist, _f32p), _p(bmu2, _u32p), _p(dist2, _f32p),
+                                         C.byref(fb)))
+        return bmu, dist, bmu2, dist2, int(fb.value)
+
+    def find_bmu2_device(self, x_dev, n, out_bmu_dev=None, out_dist_dev=None, out_bmu2_dev=None, out_dist2_dev=None, min_hits=0):
+        """vsom_find_bmu2 on device arrays; returns the rows that took the exact full scan."""
+        fb = C.c_uint64(0)
+        ptr = lambda t: t.data_ptr() if t is not None else None
+        self._check(lib().vsom_find_bmu2_device(self._h, x_dev.data_ptr(), n, min_hits, ptr(out_bmu_dev), ptr(out_dist_dev), ptr(out_bmu2_dev),
+                                                ptr(out_dist2_dev), C.byref(fb)))
+        return int(fb.value)
+
+    def find_bmu2_exact(self, x, min_hits=0):
+        """find_bmu2 through the exact scan (K3) whatever the batch size: (bmu, dist, bmu2, dist2)."""
+        x = _f32(x).reshape(-1, self.Din)
+        n = x.shape[0]
+        bmu, bmu2 = np.empty(n, np.uint32), np.empty(n, np.uint32)
+        dist, dist2 = np.empty(n, np.float32), np.empty(n, np.float32)
+        self._check(lib().vsom_find_bmu2_exact(self._h, _p(x, _f32p), n, min_hits, _p(bmu, _u32p), _p(dist, _f32p), _p(bmu2, _u32p), _p(dist2, _f32p)))
+        return bmu, dist, bmu2, dist2
 
     def measure_similarity(self, x, number_of_sigmas, min_hits=0):
         """Per-row pass of Som::measureSimilarity: (restricted BMU, largest normalised deviation from it) for every row."""

@@ -15,6 +15,7 @@ LIB = os.path.join(LIB_DIR, "libvsom_b200.so")
 HOST_LIB = os.path.join(LIB_DIR, "libvsom_host.so")
 API_DRIVER = os.path.join(REPO, "tests", "cpp", "api_driver_b200")
 MNIST_TEST = os.path.join(REPO, "tests", "cpp", "mnist_loader_test")
+TOPO_DRIVER = os.path.join(REPO, "tests", "cpp", "topo_driver")
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
@@ -38,9 +39,10 @@ def sources():
 
 
 def up_to_date() -> bool:
-    if not (os.path.exists(LIB) and os.path.exists(HOST_LIB) and os.path.exists(API_DRIVER) and os.path.exists(MNIST_TEST)):
+    outputs = (LIB, HOST_LIB, API_DRIVER, MNIST_TEST, TOPO_DRIVER)
+    if not all(os.path.exists(o) for o in outputs):
         return False
-    t = min(os.path.getmtime(LIB), os.path.getmtime(HOST_LIB), os.path.getmtime(API_DRIVER), os.path.getmtime(MNIST_TEST))
+    t = min(os.path.getmtime(o) for o in outputs)
     deps = sources() + glob.glob(os.path.join(REPO, "tests", "cpp", "*.cpp")) + glob.glob(os.path.join(REPO, "include", "compat", "Eigen", "*")) + glob.glob(os.path.join(PKG, "host", "*.cpp")) + glob.glob(os.path.join(REPO, "include", "*.hpp")) + glob.glob(os.path.join(CSRC, "*.cuh")) + glob.glob(os.path.join(REPO, "include", "*.h")) + [os.path.abspath(__file__)]
     return all(os.path.getmtime(d) <= t for d in deps)
 
@@ -92,7 +94,8 @@ def build_host() -> str:
     if out.returncode != 0:
         raise RuntimeError(f"host library failed to build:\n{out.stdout}")
     for src, exe, defs in ((os.path.join(REPO, "tests", "cpp", "api_driver.cpp"), API_DRIVER, ["-DVSOM_B200_API"]),
-                           (os.path.join(REPO, "tests", "cpp", "mnist_loader_test.cpp"), MNIST_TEST, [])):
+                           (os.path.join(REPO, "tests", "cpp", "mnist_loader_test.cpp"), MNIST_TEST, []),
+                           (os.path.join(REPO, "tests", "cpp", "topo_driver.cpp"), TOPO_DRIVER, [])):
         if os.path.exists(src):
             cmd = [cxx, *flags, *defs, src, "-o", exe, "-L", LIB_DIR, "-lvsom_host", "-lvsom_b200", f"-Wl,-rpath,{LIB_DIR}", *stdcxx]
             out = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)

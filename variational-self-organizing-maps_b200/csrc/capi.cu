@@ -648,8 +648,9 @@ int vsom_batch_epoch(vsom_ctx *ctx, const float *x, size_t n, double sigma, int 
 static const size_t kTcMinRows = 1024;
 static const char *kUnshardedOnly = "this entry point needs an unsharded context (scoring and index run on replicated maps)";
 
+// top = 2 (vsom_find_bmu2*): every row's runner-up as well, to out_bmu2 / out_dist2 (each may be null); same dispatch
 static int find_bmu_device_impl(vsom_ctx *ctx, const float *x_dev, size_t n, uint64_t min_hits, uint32_t *out_bmu_dev, float *out_dist_dev, bool allowTc,
-                                uint64_t *fallback_rows, const char *who)
+                                uint64_t *fallback_rows, const char *who, int top = 1, uint32_t *out_bmu2_dev = nullptr, float *out_dist2_dev = nullptr)
 {
     if (ctx && ctx->world > 1)
         return set_error(ctx, VSOM_ERR_UNSUPPORTED, kUnshardedOnly);
@@ -663,18 +664,20 @@ static int find_bmu_device_impl(vsom_ctx *ctx, const float *x_dev, size_t n, uin
         if (fallback_rows)
             *fallback_rows = n;
         ctx->lastScoreTc = 0;
+        if (top == 2)
+            return launch_find_bmu2(ctx, x_dev, n, min_hits, out_bmu_dev, out_dist_dev, out_bmu2_dev, out_dist2_dev);
         return launch_find_bmu(ctx, x_dev, n, min_hits, out_bmu_dev, out_dist_dev);
     }
     unsigned long long fb = 0;
     ctx->lastScoreTc = 1;
-    const int rc = launch_find_bmu_tc(ctx, x_dev, n, min_hits, out_bmu_dev, out_dist_dev, &fb);
+    const int rc = launch_find_bmu_tc(ctx, x_dev, n, min_hits, out_bmu_dev, out_dist_dev, &fb, top, out_bmu2_dev, out_dist2_dev);
     if (fallback_rows)
         *fallback_rows = fb;
     return rc;
 }
 
 static int find_bmu_host_impl(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist, bool allowTc, uint64_t *fallback_rows,
-                              const char *who)
+                              const char *who, int top = 1, uint32_t *out_bmu2 = nullptr, float *out_dist2 = nullptr)
 {
     if (ctx && ctx->world > 1)
         return set_error(ctx, VSOM_ERR_UNSUPPORTED, kUnshardedOnly);
@@ -691,14 +694,14 @@ static int find_bmu_host_impl(vsom_ctx *ctx, const float *x, size_t n, uint64_t 
         unsigned long long fb = 0;
         size_t done = 0;
         ctx->lastScoreTc = 1;
-        const int rc = launch_find_bmu_tc_host(ctx, x, n, min_hits, out_bmu, out_dist, &fb, &done);
+        const int rc = launch_find_bmu_tc_host(ctx, x, n, min_hits, out_bmu, out_dist, &fb, &done, top, out_bmu2, out_dist2);
         if (rc)
             return rc;
         if (done < n) // the probes found the map / data unsuited to the candidate search: the rest takes the exact path below
         {
             uint64_t rest = 0;
             const int rc2 = find_bmu_host_impl(ctx, x + done * ctx->Din, n - done, min_hits, out_bmu ? out_bmu + done : nullptr, out_dist ? out_dist + done : nullptr, false,
-                                               &rest, who);
+                                               &rest, who, top, out_bmu2 ? out_bmu2 + done : nullptr, out_dist2 ? out_dist2 + done : nullptr);
             ctx->lastScoreTc = 1;
             fb += rest;
             if (rc2)
@@ -724,6 +727,16 @@ static int find_bmu_host_impl(vsom_ctx *ctx, const float *x, size_t n, uint64_t 
     float *xDev = static_cast<float *>(ctx->stage[0]);
     unsigned *bmuDev = static_cast<unsigned *>(ctx->stage[1]);
     float *distDev = static_cast<float *>(ctx->stage[2]);
+    unsigned *bmu2Dev = nullptr; // top = 2: stage slot 4 holds the runner-ups and their distances
+    float *dist2Dev = nullptr;
+    if (top == 2)
+    {
+        rc = stage_reserve(ctx, 4, (sizeof(unsigned) + sizeof(float)) * slab);
+        if (rc)
+            return rc;
+        bmu2Dev = static_cast<unsigned *>(ctx->stage[4]);
+        dist2Dev = reinterpret_cast<float *>(bmu2Dev + slab);
+    }
     if (fallback_rows)
         *fallback_rows = n;
     ctx->lastScoreTc = 0;
@@ -731,7 +744,7 @@ static int find_bmu_host_impl(vsom_ctx *ctx, const float *x, size_t n, uint64_t 
     {
         const size_t rows = std::min(slab, n - r0);
         VSOM_CUDA(ctx, cudaMemcpyAsync(xDev, x + r0 * ctx->Din, sizeof(float) * rows * ctx->Din, cudaMemcpyHostToDevice, ctx->stream));
-        rc = launch_find_bmu(ctx, xDev, rows, min_hits, bmuDev, distDev);
+        rc = top == 2 ? launch_find_bmu2(ctx, xDev, rows, min_hits, bmuDev, distDev, bmu2Dev, dist2Dev) : launch_find_bmu(ctx, xDev, rows, min_hits, bmuDev, distDev);
         if (rc)
             return rc;
         rc = similarity_hook(ctx, xDev, rows, bmuDev, 0, ctx->stream); // armed by vsom_measure_similarity only
@@ -742,6 +755,10 @@ static int find_bmu_host_impl(vsom_ctx *ctx, const float *x, size_t n, uint64_t 
             VSOM_CUDA(ctx, cudaMemcpyAsync(out_bmu + r0, bmuDev, sizeof(unsigned) * rows, cudaMemcpyDeviceToHost, ctx->stream));
         if (out_dist)
             VSOM_CUDA(ctx, cudaMemcpyAsync(out_dist + r0, distDev, sizeof(float) * rows, cudaMemcpyDeviceToHost, ctx->stream));
+        if (out_bmu2)
+            VSOM_CUDA(ctx, cudaMemcpyAsync(out_bmu2 + r0, bmu2Dev, sizeof(unsigned) * rows, cudaMemcpyDeviceToHost, ctx->stream));
+        if (out_dist2)
+            VSOM_CUDA(ctx, cudaMemcpyAsync(out_dist2 + r0, dist2Dev, sizeof(float) * rows, cudaMemcpyDeviceToHost, ctx->stream));
         VSOM_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); // the staging buffers are reused by the next slab
     }
     return VSOM_OK;
@@ -776,6 +793,23 @@ int vsom_find_bmu_batch_device(vsom_ctx *ctx, const float *x_dev, size_t n, uint
 int vsom_find_bmu_batch(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist, uint64_t *fallback_rows)
 {
     return find_bmu_host_impl(ctx, x, n, min_hits, out_bmu, out_dist, true, fallback_rows, "vsom_find_bmu_batch");
+}
+
+int vsom_find_bmu2(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist, uint32_t *out_bmu2, float *out_dist2,
+                   uint64_t *fallback_rows)
+{
+    return find_bmu_host_impl(ctx, x, n, min_hits, out_bmu, out_dist, true, fallback_rows, "vsom_find_bmu2", 2, out_bmu2, out_dist2);
+}
+
+int vsom_find_bmu2_device(vsom_ctx *ctx, const float *x_dev, size_t n, uint64_t min_hits, uint32_t *out_bmu_dev, float *out_dist_dev, uint32_t *out_bmu2_dev,
+                          float *out_dist2_dev, uint64_t *fallback_rows)
+{
+    return find_bmu_device_impl(ctx, x_dev, n, min_hits, out_bmu_dev, out_dist_dev, true, fallback_rows, "vsom_find_bmu2_device", 2, out_bmu2_dev, out_dist2_dev);
+}
+
+int vsom_find_bmu2_exact(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist, uint32_t *out_bmu2, float *out_dist2)
+{
+    return find_bmu_host_impl(ctx, x, n, min_hits, out_bmu, out_dist, false, nullptr, "vsom_find_bmu2_exact", 2, out_bmu2, out_dist2);
 }
 
 int vsom_debug_tc_stats(const vsom_ctx *ctx, uint64_t out[3])

@@ -178,11 +178,15 @@ int configure_online_step_fast(vsom_ctx *ctx);                               // 
 int launch_online_step_fast(vsom_ctx *ctx, StepParams &p, double sigma);      // 1: enqueued, 0: not eligible, < 0: error
 int launch_find_bmu(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, unsigned *outBmuDev, float *outDistDev);
 int launch_find_bmu_list(vsom_ctx *ctx, const float *xDev, size_t n, const unsigned *rowListDev, const unsigned *rowCountDev, uint64_t minHits, unsigned *outBmuDev,
-                         float *outDistDev, cudaStream_t stream, u64 *keyBufDev);
+                         float *outDistDev, cudaStream_t stream, u64 *keyBufDev, int top = 1, unsigned *outBmu2Dev = nullptr, float *outDist2Dev = nullptr);
+// the exact scan with every row's runner-up as well (vsom_find_bmu2)
+int launch_find_bmu2(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, unsigned *outBmuDev, float *outDistDev, unsigned *outBmu2Dev, float *outDist2Dev);
 bool score_tc_supported(const vsom_ctx *ctx);
-int launch_find_bmu_tc(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, unsigned *outBmuDev, float *outDistDev, unsigned long long *fallbackRowsOut);
+// top = 2 (vsom_find_bmu2): the best two nodes of every row; outBmu2 / outDist2 may be null
+int launch_find_bmu_tc(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, unsigned *outBmuDev, float *outDistDev, unsigned long long *fallbackRowsOut,
+                       int top = 1, unsigned *outBmu2Dev = nullptr, float *outDist2Dev = nullptr);
 int launch_find_bmu_tc_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t minHits, unsigned *outBmuHost, float *outDistHost, unsigned long long *fallbackRowsOut,
-                            size_t *rowsDoneOut);
+                            size_t *rowsDoneOut, int top = 1, unsigned *outBmu2Host = nullptr, float *outDist2Host = nullptr);
 int launch_batch_epoch(vsom_ctx *ctx, const float *xDev, size_t n, double sigma, int isFirst, const u64 *lastDev, unsigned *bmuDev, float *distDev);
 int launch_all_dists(vsom_ctx *ctx, const float *vDev, double *outDev);
 int launch_soft_assign(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, double *probDev, double *sumsDev);
@@ -315,6 +319,39 @@ __device__ __forceinline__ u64 make_key(float d, unsigned node, unsigned tag, un
     return (static_cast<u64>(bits) << 32) | (static_cast<u64>(node) << 8) | tag;
 }
 __device__ __forceinline__ unsigned key_node(u64 k) { return static_cast<unsigned>((k >> 8) & 0xffffffu); }
+
+// ---- best and second-best keys (vsom_find_bmu2).  Keys of distinct nodes are distinct, so the pair (k1 < k2) is simply the two
+// smallest keys: k1 is the BMU of findBmu's rule (a NaN at node 0 wins, key 0), k2 the runner-up with NaN distances after every
+// number (0x7fffffff), lower index first.  ~0ull: no key.
+__device__ __forceinline__ u64 u64_max(u64 a, u64 b) { return a > b ? a : b; }
+__device__ __forceinline__ void key_top2_insert(u64 &k1, u64 &k2, u64 k)
+{
+    k2 = u64_min(k2, u64_max(k1, k));
+    k1 = u64_min(k1, k);
+}
+__device__ __forceinline__ void key_top2_merge(u64 &k1, u64 &k2, u64 o1, u64 o2)
+{
+    k2 = u64_min(u64_min(k2, o2), u64_max(k1, o1));
+    k1 = u64_min(k1, o1);
+}
+// (k1, k2) of several producers meeting in global memory (two words per row): whichever of the new k1 and the old one loses
+// the first atomic min is a candidate for the second word, and so is the producer's own k2.  Once every producer has passed,
+// word 0 holds the smallest key and word 1 the smallest of all the others.
+__device__ __forceinline__ void key_top2_atomic(u64 *slot, u64 k1, u64 k2)
+{
+    const u64 old = atomicMin(slot, k1);
+    atomicMin(slot + 1, u64_min(k2, u64_max(old, k1)));
+}
+// distance of a key as the scoring calls return it (a canonical NaN for NaN distances)
+__device__ __forceinline__ float key_dist(u64 k) { return (k & 1ull) ? __uint_as_float(0x7fc00000u) : __uint_as_float(static_cast<unsigned>(k >> 32)); }
+// the second-best outputs of a row: 0xFFFFFFFF and NaN when the row has no runner-up (fewer than two eligible nodes)
+__device__ __forceinline__ void store_second(unsigned *outBmu2, float *outDist2, u64 row, u64 k2)
+{
+    if (outBmu2)
+        outBmu2[row] = k2 == ~0ull ? 0xffffffffu : key_node(k2);
+    if (outDist2)
+        outDist2[row] = k2 == ~0ull ? __uint_as_float(0x7fc00000u) : key_dist(k2);
+}
 
 // ---- node-sharded contexts (BASELINE config 5): block b of `shardBlock` grid rows lives on rank b % world as that rank's
 // local block b / world.  Local node order is global node order restricted to the rank (monotone), so keys compare the same

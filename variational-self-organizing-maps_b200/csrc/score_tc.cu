@@ -258,7 +258,14 @@ struct TcShared
 //   bFull / aFull : the LEADER's; its producer expects both CTAs' bytes, the peer's TMA completes on it (cta_group::2 load)
 //   bEmpty / aEmpty / tFull : each CTA's own, signalled by the leader's tcgen05.commit multicast to both
 //   tEmpty : the leader's; one arrival per epilogue warp of BOTH CTAs (the peer's arrive through shared::cluster)
-template <bool PAIR>
+//
+// TOP = 2 (vsom_find_bmu2): the list must hold the runner-up too, so each thread keeps an upper bound `second` of the
+// second-smallest score it has seen and lists every node below second + Delta'.  Per chunk:
+//     second = min(second, max(best, chunk min), second-smallest of the eight group minima m4[])
+// (each term bounds the second-smallest of the scores seen so far; the group minima are eight different columns), so the
+// threshold still only falls.  The half-row merge combines the two (best, second) pairs the same way, and bestOut receives the
+// final threshold base: every unlisted node had a' >= that base + Delta' (see rescore_kernel's certificate).
+template <bool PAIR, int TOP>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 score_tc_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUtensorMap mapM, int kSteps, int rowsTotal,
                 int numRowTiles, int numNodeTiles, int kBlocks, int kCols, int stagger, int D, const float *__restrict__ xnorm2, const float *__restrict__ xratio, const TcScale *__restrict__ scale,
@@ -496,6 +503,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant_
             float E, delta;
             tc_margins(xn, mm, ratio, kCols, D, scale->split, E, delta);
             float best = inf, thr = inf, thrC = inf; // thrC: threshold at this list's last compaction
+            float second = inf;                      // TOP = 2: upper bound of the second-smallest score so far
             int cnt = 0;
             bool ovf = false;
             unsigned wp = mineAddr; // shared address of the next free entry of this thread's list (2048 bytes apart)
@@ -544,8 +552,33 @@ score_tc_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant_
                         const float cm = fminf(fminf(fminf(m4[0], m4[1]), fminf(m4[2], m4[3])), fminf(fminf(m4[4], m4[5]), fminf(m4[6], m4[7])));
                         const float thrOld = thr; // valid, possibly stale: whatever must be appended lies below it
                         // the chunk's own minimum tightens the threshold BEFORE anything is appended
-                        best = fminf(best, cm);
-                        thr = best + delta;
+                        if (TOP == 2)
+                        {
+                            // second-smallest of the group minima: (min, second) of pairs, merged twice
+                            float lo[4], hi[4];
+#pragma unroll
+                            for (int j = 0; j < 4; ++j)
+                            {
+                                lo[j] = fminf(m4[2 * j], m4[2 * j + 1]);
+                                hi[j] = fmaxf(m4[2 * j], m4[2 * j + 1]);
+                            }
+#pragma unroll
+                            for (int w2 = 2; w2; w2 >>= 1)
+#pragma unroll
+                                for (int j = 0; j < w2; ++j)
+                                {
+                                    hi[j] = fminf(fmaxf(lo[j], lo[j + w2]), fminf(hi[j], hi[j + w2]));
+                                    lo[j] = fminf(lo[j], lo[j + w2]);
+                                }
+                            second = fminf(second, fminf(fmaxf(best, cm), hi[0]));
+                            best = fminf(best, cm);
+                            thr = second + delta;
+                        }
+                        else
+                        {
+                            best = fminf(best, cm);
+                            thr = best + delta;
+                        }
                         if (!__any_sync(0xffffffffu, cm < thrOld))
                             return; // no lane of the warp has a candidate in this chunk (the common case once the rows have settled)
                         // Lists only grow here, so this is where a long one is compacted — and only when the threshold has tightened
@@ -623,9 +656,23 @@ score_tc_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant_
             // merge the two halves of the row: common best -> final threshold -> filter both lists -> candidates
             cnt = static_cast<int>((wp - mineAddr) >> 11);
             sBest[et] = best;
+            if (TOP == 2)
+                reinterpret_cast<float *>(sCnt)[et] = second; // sCnt is free until the counts below
             asm volatile("bar.sync 1, 256;" ::: "memory");
-            const float bestF = fminf(best, sBest[et ^ 128]);
-            const float thrF = bestF + delta;
+            float bestF, thrF;
+            if (TOP == 2)
+            {
+                // the pair's threshold base: an upper bound of the row's second-smallest score, below both halves' thresholds
+                const float bo = sBest[et ^ 128], so = reinterpret_cast<const float *>(sCnt)[et ^ 128];
+                bestF = fminf(fmaxf(best, bo), fminf(second, so));
+                thrF = bestF + delta;
+                asm volatile("bar.sync 1, 256;" ::: "memory"); // both halves have read sCnt's floats
+            }
+            else
+            {
+                bestF = fminf(best, sBest[et ^ 128]);
+                thrF = bestF + delta;
+            }
             compact(cnt, thrF);
             sCnt[et] = ovf ? 1000 : cnt;
             asm volatile("bar.sync 1, 256;" ::: "memory");
@@ -642,7 +689,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant_
                 if (half == 0)
                 {
                     countOut[row] = bad ? TC_OVERFLOW : static_cast<unsigned>(total);
-                    bestOut[row] = bestF; // the certificate's lower bound starts from the best APPROXIMATE score
+                    bestOut[row] = bestF; // the certificate's lower bound starts from the best APPROXIMATE score (TOP = 2: the threshold base)
                 }
             }
             asm volatile("bar.sync 1, 256;" ::: "memory"); // sBest / sCnt are reused by the next row tile
@@ -812,18 +859,24 @@ __global__ void row_operand_kernel(const float *__restrict__ src, long long rows
 // the (distance, node) key in shared memory — lowest index on ties, like the reference.  Then the certificate (see the
 // head of this file): the row is final only if no unlisted node can reach the winner's exact distance.  Rows that fail it,
 // rows whose list overflowed and rows whose winner is NaN go to the fallback list (exact full scan).
+// TOP = 2: the two smallest keys of the row (two shared-memory atomic mins per candidate, key_top2_atomic), and the certificate
+// must clear the RUNNER-UP's exact distance: bestA then holds the kernel's final threshold base, every unlisted node q had
+// a'_q >= bestA + Delta', so S_r d_q >= bestA + S_r |x|^2 + 0.25 E' > S_r d2 >= S_r d1 — no unlisted node can be either of the
+// two or tie with them.  A row without two listed eligible nodes, or with a NaN among its two, takes the exact scan.
 constexpr int RS_ROWS = 128;
 constexpr int RS_THREADS = 256;
+template <int TOP>
 __global__ void __launch_bounds__(RS_THREADS) rescore_kernel(const float *__restrict__ x, long long rows, int D, const float *__restrict__ mean, int rowStride,
                                                              const unsigned *__restrict__ cand, const unsigned *__restrict__ count, const float *__restrict__ bestA,
                                                              const float *__restrict__ xnorm2, const float *__restrict__ xratio, const TcScale *__restrict__ scale,
                                                              int Kpad, int order, int N, const u64 *__restrict__ hits, u64 minHits, unsigned *__restrict__ outBmu,
                                                              float *__restrict__ outDist, unsigned *__restrict__ fallbackRows, unsigned *__restrict__ fallbackCount,
-                                                             unsigned long long *__restrict__ stats)
+                                                             unsigned long long *__restrict__ stats, unsigned *__restrict__ outBmu2, float *__restrict__ outDist2)
 {
     __shared__ unsigned sOff[RS_ROWS + 1];
     __shared__ unsigned sWarpTot[RS_ROWS / 32];
     __shared__ u64 sKey[RS_ROWS];
+    __shared__ u64 sKey2[TOP == 2 ? 2 * RS_ROWS : 1]; // TOP = 2: (best, second) of row r at 2 r
     __shared__ unsigned short sItem[RS_ROWS * TC_TOPK];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const long long row0 = static_cast<long long>(blockIdx.x) * RS_ROWS;
@@ -834,6 +887,8 @@ __global__ void __launch_bounds__(RS_THREADS) rescore_kernel(const float *__rest
         cnt = row < rows ? count[row] : 0u;
         c = cnt == TC_OVERFLOW ? 0u : cnt;
         sKey[tid] = ~0ull;
+        if (TOP == 2)
+            sKey2[2 * tid] = sKey2[2 * tid + 1] = ~0ull;
         unsigned inc = c; // inclusive scan inside the warp
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1)
@@ -871,16 +926,21 @@ __global__ void __launch_bounds__(RS_THREADS) rescore_kernel(const float *__rest
         if (node >= static_cast<unsigned>(N) || !(node == 0 || minHits == 0 || hits[node] >= minHits))
             continue;
         const float s = dist_rows_f32(mean + static_cast<size_t>(node) * rowStride, x + row * D, D, order);
-        atomicMin(&sKey[r], make_key(s, node, (s != s) ? 1u : 0u));
+        if (TOP == 2)
+            key_top2_atomic(&sKey2[2 * r], make_key(s, node, (s != s) ? 1u : 0u), ~0ull);
+        else
+            atomicMin(&sKey[r], make_key(s, node, (s != s) ? 1u : 0u));
     }
     __syncthreads();
     if (tid < RS_ROWS && row0 + tid < rows)
     {
         const long long row = row0 + tid;
-        const u64 key = sKey[tid];
-        const bool nan = (key & 1ull) != 0 || scale->nanNode0;
+        const u64 key = TOP == 2 ? sKey2[2 * tid] : sKey[tid];
+        const u64 key2 = TOP == 2 ? sKey2[2 * tid + 1] : 0ull; // TOP = 2: the runner-up, whose distance the bound must clear
+        const u64 keyC = TOP == 2 ? key2 : key;
+        const bool nan = (key & 1ull) != 0 || (TOP == 2 && (key2 & 1ull) != 0) || scale->nanNode0;
         bool certified = false;
-        if (cnt != TC_OVERFLOW && !nan && key != ~0ull)
+        if (cnt != TC_OVERFLOW && !nan && keyC != ~0ull)
         {
             // unlisted nodes, in the row's scaled units (S_r = s_r s_m = s_m^2 / ratio): S_r d_q >= best approximate score +
             // S_r |x|^2 + Delta' - E' = ... + 0.25 E' + slack (tc_margins)
@@ -888,14 +948,14 @@ __global__ void __launch_bounds__(RS_THREADS) rescore_kernel(const float *__rest
             float E, delta;
             tc_margins(xn, scale->mm, ratio, Kpad, D, scale->split, E, delta);
             const float lower = __fadd_rn(__fadd_rn(bestA[row], __fmul_rn(xn, ratio)), __fmul_rn(0.25f, E));
-            const float sd = __fmul_rn(__fdiv_rn(__fmul_rn(sm, sm), ratio), __uint_as_float(static_cast<unsigned>(key >> 32))); // S_r d*: a power of two times d*
+            const float sd = __fmul_rn(__fdiv_rn(__fmul_rn(sm, sm), ratio), __uint_as_float(static_cast<unsigned>(keyC >> 32))); // S_r d*: a power of two times d*
             certified = lower > sd;
         }
         if (!certified)
         {
             fallbackRows[atomicAdd(fallbackCount, 1u)] = static_cast<unsigned>(row);
             // diagnostics: why (1: list overflow / empty, 2: NaN or nothing eligible, 3: the certificate's bound did not clear d*)
-            atomicAdd(stats + (cnt == TC_OVERFLOW ? 1 : (nan || key == ~0ull ? 2 : 3)), 1ull);
+            atomicAdd(stats + (cnt == TC_OVERFLOW ? 1 : (nan || keyC == ~0ull ? 2 : 3)), 1ull);
         }
         else
         {
@@ -903,6 +963,8 @@ __global__ void __launch_bounds__(RS_THREADS) rescore_kernel(const float *__rest
                 outBmu[row] = key_node(key);
             if (outDist)
                 outDist[row] = __uint_as_float(static_cast<unsigned>(key >> 32));
+            if (TOP == 2)
+                store_second(outBmu2, outDist2, static_cast<u64>(row), key2);
         }
     }
 }
@@ -996,6 +1058,7 @@ bool score_tc_supported(const vsom_ctx *ctx) { return ctx->transform != VSOM_CLR
 struct TcCall
 {
     int D = 0, N = 0, Kpad = 0, kBlocks = 0, kSteps = 0, Npad = 0, nodeTiles = 0, split = 0;
+    int top = 1; // 2: best and second-best node of every row (vsom_find_bmu2)
     bool pair = true;
     uint64_t minHits = 0;
     size_t slabRows = 0, setBytes = 0, slab = 0;
@@ -1005,9 +1068,10 @@ struct TcCall
     CUtensorMap mapM;
 };
 
-static int tc_begin(vsom_ctx *ctx, TcCall &c, size_t maxSlabRows, uint64_t minHits, int split)
+static int tc_begin(vsom_ctx *ctx, TcCall &c, size_t maxSlabRows, uint64_t minHits, int split, int top)
 {
     const int D = ctx->Dm, N = ctx->N;
+    c.top = top;
     c.D = D;
     c.N = N;
     c.split = split;
@@ -1035,8 +1099,10 @@ static int tc_begin(vsom_ctx *ctx, TcCall &c, size_t maxSlabRows, uint64_t minHi
     // co-schedule a cluster of two of these CTAs (it cannot on a partition without whole TPCs; then the single-CTA kernel runs)
     if (!ctx->tcAttrSet)
     {
-        VSOM_CUDA(ctx, cudaFuncSetAttribute(score_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcShared::TOTAL));
-        VSOM_CUDA(ctx, cudaFuncSetAttribute(score_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcShared::TOTAL));
+        VSOM_CUDA(ctx, cudaFuncSetAttribute(score_tc_kernel<false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcShared::TOTAL));
+        VSOM_CUDA(ctx, cudaFuncSetAttribute(score_tc_kernel<true, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcShared::TOTAL));
+        VSOM_CUDA(ctx, cudaFuncSetAttribute(score_tc_kernel<false, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcShared::TOTAL));
+        VSOM_CUDA(ctx, cudaFuncSetAttribute(score_tc_kernel<true, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcShared::TOTAL));
         cudaLaunchConfig_t q = {};
         cudaLaunchAttribute qa[1];
         q.gridDim = dim3(2);
@@ -1049,7 +1115,7 @@ static int tc_begin(vsom_ctx *ctx, TcCall &c, size_t maxSlabRows, uint64_t minHi
         q.attrs = qa;
         q.numAttrs = 1;
         int clusters = 0;
-        const cudaError_t qe = cudaOccupancyMaxActiveClusters(&clusters, score_tc_kernel<true>, &q);
+        const cudaError_t qe = cudaOccupancyMaxActiveClusters(&clusters, score_tc_kernel<true, 1>, &q); // the TOP = 2 kernel has the same launch shape
         if (qe != cudaSuccess)
             cudaGetLastError(); // not an error of the scoring call
         ctx->tcPairOk = qe == cudaSuccess && clusters >= 1 ? 1 : 0;
@@ -1071,7 +1137,7 @@ static int tc_begin(vsom_ctx *ctx, TcCall &c, size_t maxSlabRows, uint64_t minHi
     if (rc)
         return rc;
     // per-row scratch: candidates, their count, |s_r x|^2, s_m / s_r, best approximate score, fallback list; per set: fallback count
-    const size_t perRow = sizeof(unsigned) * TC_TOPK + sizeof(unsigned) + 3 * sizeof(float) + sizeof(unsigned) + sizeof(u64); // + key of the exact scan's node splits
+    const size_t perRow = sizeof(unsigned) * TC_TOPK + sizeof(unsigned) + 3 * sizeof(float) + sizeof(unsigned) + sizeof(u64) * top; // + key(s) of the exact scan's node splits
     c.setBytes = (perRow * c.slabRows + 512 + 255) & ~static_cast<size_t>(255);
     rc = stage_reserve(ctx, 8, 2 * c.setBytes + 256);
     if (rc)
@@ -1101,8 +1167,10 @@ static int tc_begin(vsom_ctx *ctx, TcCall &c, size_t maxSlabRows, uint64_t minHi
 
 // One slab: xs = rows x D f32 in device memory (must stay valid until the slab's evDone event).  Results go to outBmuDev /
 // outDistDev (device, may be null) and, when given, from there to host memory on the re-scoring stream.
+// c.top = 2: the runner-up as well, to outBmu2Dev / outDist2Dev and from there to outBmu2Host / outDist2Host (each may be null).
 static int tc_enqueue(vsom_ctx *ctx, TcCall &c, const float *xs, size_t rows, unsigned *outBmuDev, float *outDistDev, unsigned *outBmuHost, float *outDistHost,
-                      size_t rowInCall = 0, bool hostCall = false)
+                      size_t rowInCall = 0, bool hostCall = false, unsigned *outBmu2Dev = nullptr, float *outDist2Dev = nullptr, unsigned *outBmu2Host = nullptr,
+                      float *outDist2Host = nullptr)
 {
     const int par = static_cast<int>(c.slab & 1);
     unsigned char *set = static_cast<unsigned char *>(ctx->stage[8]) + par * c.setBytes;
@@ -1113,7 +1181,7 @@ static int tc_enqueue(vsom_ctx *ctx, TcCall &c, const float *xs, size_t rows, un
     float *bestA = xratio + c.slabRows;
     unsigned *fbRows = reinterpret_cast<unsigned *>(bestA + c.slabRows);
     u64 *fbKeys = reinterpret_cast<u64 *>(set + ((reinterpret_cast<unsigned char *>(fbRows + c.slabRows) - set + 7) & ~static_cast<size_t>(7)));
-    unsigned *fbCount = reinterpret_cast<unsigned *>(fbKeys + c.slabRows);
+    unsigned *fbCount = reinterpret_cast<unsigned *>(fbKeys + c.slabRows * c.top);
     const int order = ctx->order == VSOM_ORDER_EIGEN_SSE ? VSOM_ORDER_EIGEN_SSE : VSOM_ORDER_REFERENCE;
 
     if (c.slab >= 2)
@@ -1149,17 +1217,19 @@ static int tc_enqueue(vsom_ctx *ctx, TcCall &c, const float *xs, size_t rows, un
         const float *xn = xnorm, *xr = xratio;
         const TcScale *sc = c.scale;
         // the kernel's debug word is 1: staggered node-tile starts, none of the timing-only variants
-        VSOM_CUDA(ctx, cudaLaunchKernelEx(&cfg, c.pair ? score_tc_kernel<true> : score_tc_kernel<false>, mapX, c.mapM, c.kSteps, rowsI, rowTiles, c.nodeTiles, c.kBlocks, c.Kpad, 1, c.D,
-                                          xn, xr, sc, cand, candCount, bestA, ctx->errFlag));
+        auto kern = c.top == 2 ? (c.pair ? score_tc_kernel<true, 2> : score_tc_kernel<false, 2>) : (c.pair ? score_tc_kernel<true, 1> : score_tc_kernel<false, 1>);
+        VSOM_CUDA(ctx, cudaLaunchKernelEx(&cfg, kern, mapX, c.mapM, c.kSteps, rowsI, rowTiles, c.nodeTiles, c.kBlocks, c.Kpad, 1, c.D, xn, xr, sc, cand, candCount, bestA,
+                                          ctx->errFlag));
     }
     cudaStream_t rs = ctx->auxStream;
     VSOM_CUDA(ctx, cudaEventRecord(ctx->evScore[par], ctx->stream));
     VSOM_CUDA(ctx, cudaStreamWaitEvent(rs, ctx->evScore[par], 0));
-    rescore_kernel<<<static_cast<unsigned>((rows + RS_ROWS - 1) / RS_ROWS), RS_THREADS, 0, rs>>>(xs, static_cast<long long>(rows), c.D, ctx->mean, ctx->rowStride, cand, candCount, bestA,
-                                                                                                 xnorm, xratio, c.scale, c.Kpad, order, c.N, ctx->hits, c.minHits, outBmuDev, outDistDev, fbRows, fbCount, c.totalDev);
+    (c.top == 2 ? rescore_kernel<2> : rescore_kernel<1>)<<<static_cast<unsigned>((rows + RS_ROWS - 1) / RS_ROWS), RS_THREADS, 0, rs>>>(
+        xs, static_cast<long long>(rows), c.D, ctx->mean, ctx->rowStride, cand, candCount, bestA, xnorm, xratio, c.scale, c.Kpad, order, c.N, ctx->hits, c.minHits, outBmuDev,
+        outDistDev, fbRows, fbCount, c.totalDev, outBmu2Dev, outDist2Dev);
     // rows the certificate rejected: exact scan (K3 tiles over the row list; the count stays on the device)
     add_count_kernel<<<1, 1, 0, rs>>>(fbCount, c.totalDev);
-    rc = launch_find_bmu_list(ctx, xs, rows, fbRows, fbCount, c.minHits, outBmuDev, outDistDev, rs, fbKeys);
+    rc = launch_find_bmu_list(ctx, xs, rows, fbRows, fbCount, c.minHits, outBmuDev, outDistDev, rs, fbKeys, c.top, outBmu2Dev, outDist2Dev);
     if (rc)
         return rc;
     if (hostCall && outBmuDev) // vsom_measure_similarity: the slab's rows are still on the device and its BMUs are final
@@ -1172,6 +1242,10 @@ static int tc_enqueue(vsom_ctx *ctx, TcCall &c, const float *xs, size_t rows, un
         VSOM_CUDA(ctx, cudaMemcpyAsync(outBmuHost, outBmuDev, sizeof(unsigned) * rows, cudaMemcpyDeviceToHost, rs));
     if (outDistHost && outDistDev)
         VSOM_CUDA(ctx, cudaMemcpyAsync(outDistHost, outDistDev, sizeof(float) * rows, cudaMemcpyDeviceToHost, rs));
+    if (outBmu2Host && outBmu2Dev)
+        VSOM_CUDA(ctx, cudaMemcpyAsync(outBmu2Host, outBmu2Dev, sizeof(unsigned) * rows, cudaMemcpyDeviceToHost, rs));
+    if (outDist2Host && outDist2Dev)
+        VSOM_CUDA(ctx, cudaMemcpyAsync(outDist2Host, outDist2Dev, sizeof(float) * rows, cudaMemcpyDeviceToHost, rs));
     VSOM_CUDA(ctx, cudaEventRecord(ctx->evDone[par], rs));
     ctx->launches += 4;
     VSOM_CUDA(ctx, cudaGetLastError());
@@ -1265,23 +1339,25 @@ static int tc_score_tiers(vsom_ctx *ctx, size_t n, const Run &run, size_t &done,
 
 // rows [0, n) of xDev through one tier; slabs of the given size
 static int tc_run_device(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, int split, size_t slabRows, unsigned *outBmuDev, float *outDistDev,
-                         unsigned long long *fallbackRowsOut)
+                         unsigned long long *fallbackRowsOut, int top, unsigned *outBmu2Dev, float *outDist2Dev)
 {
     slabRows = std::min(n, std::min(slabRows, tc_slab_cap(ctx, split)));
     TcCall c;
-    int rc = tc_begin(ctx, c, slabRows, minHits, split);
+    int rc = tc_begin(ctx, c, slabRows, minHits, split, top);
     if (rc)
         return rc;
     for (size_t r0 = 0; r0 < n; r0 += slabRows)
     {
-        rc = tc_enqueue(ctx, c, xDev + r0 * c.D, std::min(slabRows, n - r0), outBmuDev ? outBmuDev + r0 : nullptr, outDistDev ? outDistDev + r0 : nullptr, nullptr, nullptr);
+        rc = tc_enqueue(ctx, c, xDev + r0 * c.D, std::min(slabRows, n - r0), outBmuDev ? outBmuDev + r0 : nullptr, outDistDev ? outDistDev + r0 : nullptr, nullptr, nullptr, 0,
+                        false, outBmu2Dev ? outBmu2Dev + r0 : nullptr, outDist2Dev ? outDist2Dev + r0 : nullptr);
         if (rc)
             return rc;
     }
     return tc_finish(ctx, c, fallbackRowsOut);
 }
 
-int launch_find_bmu_tc(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, unsigned *outBmuDev, float *outDistDev, unsigned long long *fallbackRowsOut)
+int launch_find_bmu_tc(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, unsigned *outBmuDev, float *outDistDev, unsigned long long *fallbackRowsOut,
+                       int top, unsigned *outBmu2Dev, float *outDist2Dev)
 {
     if (!score_tc_supported(ctx))
         return set_error(ctx, VSOM_ERR_UNSUPPORTED, "score_tc: needs a Standard/Median transformation and Dm <= 2048");
@@ -1298,14 +1374,16 @@ int launch_find_bmu_tc(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minH
         ctx, n,
         [&](size_t r0, size_t rows, int tier, unsigned long long &fb) {
             return tc_run_device(ctx, xDev + r0 * ctx->Dm, rows, minHits, tier == 2 ? 1 : 0, tier == 2 ? slab2 : slab1, outBmuDev ? outBmuDev + r0 : nullptr,
-                                 outDistDev ? outDistDev + r0 : nullptr, &fb);
+                                 outDistDev ? outDistDev + r0 : nullptr, &fb, top, outBmu2Dev ? outBmu2Dev + r0 : nullptr, outDist2Dev ? outDist2Dev + r0 : nullptr);
         },
         done, total);
     if (rc)
         return rc;
     if (done < n) // tier 3
     {
-        rc = launch_find_bmu(ctx, xDev + done * ctx->Dm, n - done, minHits, outBmuDev ? outBmuDev + done : nullptr, outDistDev ? outDistDev + done : nullptr);
+        rc = launch_find_bmu_list(ctx, xDev + done * ctx->Dm, n - done, nullptr, nullptr, minHits, outBmuDev ? outBmuDev + done : nullptr,
+                                  outDistDev ? outDistDev + done : nullptr, ctx->stream, nullptr, top, outBmu2Dev ? outBmu2Dev + done : nullptr,
+                                  outDist2Dev ? outDist2Dev + done : nullptr);
         if (rc)
             return rc;
         total += n - done;
@@ -1318,7 +1396,7 @@ int launch_find_bmu_tc(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minH
 
 // rows [0, n) of xHost through one tier, pipelined over the copy / search / re-scoring streams
 static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t minHits, int split, size_t slabRows, unsigned *outBmuHost, float *outDistHost,
-                       unsigned long long *fallbackRowsOut)
+                       unsigned long long *fallbackRowsOut, int top, unsigned *outBmu2Host, float *outDist2Host)
 {
     slabRows = std::min(n, std::min(slabRows, tc_slab_cap(ctx, split)));
     const size_t D = static_cast<size_t>(ctx->Dm);
@@ -1338,8 +1416,18 @@ static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t min
         xbuf[i] = static_cast<float *>(ctx->stage[0]) + static_cast<size_t>(i) * slabRows * D;
     unsigned *bmuDev = static_cast<unsigned *>(ctx->stage[1]);
     float *distDev = static_cast<float *>(ctx->stage[2]);
+    unsigned *bmu2Dev = nullptr; // top = 2: stage slot 4 holds the runner-ups and their distances
+    float *dist2Dev = nullptr;
+    if (top == 2)
+    {
+        rc = stage_reserve(ctx, 4, (sizeof(unsigned) + sizeof(float)) * n);
+        if (rc)
+            return rc;
+        bmu2Dev = static_cast<unsigned *>(ctx->stage[4]);
+        dist2Dev = reinterpret_cast<float *>(bmu2Dev + n);
+    }
     TcCall c;
-    rc = tc_begin(ctx, c, slabRows, minHits, split);
+    rc = tc_begin(ctx, c, slabRows, minHits, split, top);
     if (rc)
         return rc;
     // the staging buffers may still be in use by earlier work of the context's stream
@@ -1364,7 +1452,9 @@ static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t min
         const size_t r0 = sl * slabRows, rows = std::min(slabRows, n - r0);
         const int b = static_cast<int>(sl % 3);
         VSOM_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->evCopied[b], 0));
-        rc = tc_enqueue(ctx, c, xbuf[b], rows, bmuDev + r0, distDev + r0, outBmuHost ? outBmuHost + r0 : nullptr, outDistHost ? outDistHost + r0 : nullptr, r0, true);
+        rc = tc_enqueue(ctx, c, xbuf[b], rows, bmuDev + r0, distDev + r0, outBmuHost ? outBmuHost + r0 : nullptr, outDistHost ? outDistHost + r0 : nullptr, r0, true,
+                        bmu2Dev ? bmu2Dev + r0 : nullptr, dist2Dev ? dist2Dev + r0 : nullptr, outBmu2Host ? outBmu2Host + r0 : nullptr,
+                        outDist2Host ? outDist2Host + r0 : nullptr);
         if (rc)
             return rc;
         VSOM_CUDA(ctx, cudaEventRecord(ctx->evSlabDone[b], ctx->auxStream)); // behind the slab's re-scoring and result copies
@@ -1387,7 +1477,7 @@ static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t min
 // call is then bound by the slower of PCIe (4 D bytes per row) and the kernel.  stage slots: 0 = three row slabs,
 // 1 / 2 = BMU / distance of the whole call.  Same probe and tier choice as the device form.
 int launch_find_bmu_tc_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t minHits, unsigned *outBmuHost, float *outDistHost, unsigned long long *fallbackRowsOut,
-                            size_t *rowsDoneOut)
+                            size_t *rowsDoneOut, int top, unsigned *outBmu2Host, float *outDist2Host)
 {
     if (!score_tc_supported(ctx))
         return set_error(ctx, VSOM_ERR_UNSUPPORTED, "score_tc: needs a Standard/Median transformation and Dm <= 2048");
@@ -1403,7 +1493,7 @@ int launch_find_bmu_tc_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_
         ctx, n,
         [&](size_t r0, size_t rows, int tier, unsigned long long &fb) {
             return tc_run_host(ctx, xHost + r0 * ctx->Dm, rows, minHits, tier == 2 ? 1 : 0, slabRows, outBmuHost ? outBmuHost + r0 : nullptr,
-                               outDistHost ? outDistHost + r0 : nullptr, &fb);
+                               outDistHost ? outDistHost + r0 : nullptr, &fb, top, outBmu2Host ? outBmu2Host + r0 : nullptr, outDist2Host ? outDist2Host + r0 : nullptr);
         },
         done, total);
     if (rc)

@@ -6,10 +6,12 @@
 
 #include "vsom_b200.h"
 
+#include <algorithm>
 #include <cassert>
 #include <cmath>
 #include <cstdlib>
 #include <cctype>
+#include <cstdint>
 #include <cstdio>
 #include <cstring>
 #include <ctime>
@@ -435,6 +437,42 @@ void Som::mapDataSet(const DataSet &dataset, std::vector<size_t> &bmuOut, std::v
     if (vsom_find_bmu(ctx, dataset.contiguousRows(), rows, minBmuHits, bmu.data(), distOut.data()) != VSOM_OK)
         fail(ctx, "Som::mapDataSet");
     bmuOut.assign(bmu.begin(), bmu.end());
+}
+
+void Som::mapDataSetTopTwo(const DataSet &dataset, std::vector<size_t> &bmuOut, std::vector<float> &distOut, std::vector<size_t> &bmu2Out,
+                           std::vector<float> &dist2Out, size_t minBmuHits) const
+{
+    vsom_ctx *ctx = context();
+    const size_t rows = dataset.size();
+    std::vector<uint32_t> bmu(rows), bmu2(rows);
+    distOut.resize(rows);
+    dist2Out.resize(rows);
+    if (vsom_find_bmu2(ctx, dataset.contiguousRows(), rows, minBmuHits, bmu.data(), distOut.data(), bmu2.data(), dist2Out.data(), nullptr) != VSOM_OK)
+        fail(ctx, "Som::mapDataSetTopTwo");
+    bmuOut.assign(bmu.begin(), bmu.end());
+    bmu2Out.resize(rows);
+    for (size_t i = 0; i < rows; ++i)
+        bmu2Out[i] = bmu2[i] == 0xFFFFFFFFu ? SIZE_MAX : static_cast<size_t>(bmu2[i]);
+}
+
+double Som::topographicError(const DataSet &dataset) const
+{
+    std::vector<size_t> bmu, bmu2;
+    std::vector<float> dist, dist2;
+    mapDataSetTopTwo(dataset, bmu, dist, bmu2, dist2, 0);
+    if (bmu.empty())
+        return 0.0;
+    size_t errors = 0;
+    for (size_t i = 0; i < bmu.size(); ++i)
+    {
+        if (bmu2[i] == SIZE_MAX)
+            continue;
+        const long long dx = static_cast<long long>(bmu[i] % width) - static_cast<long long>(bmu2[i] % width);
+        const long long dy = static_cast<long long>(bmu[i] / width) - static_cast<long long>(bmu2[i] / width);
+        if (std::max(std::llabs(dx), std::llabs(dy)) != 1)
+            ++errors;
+    }
+    return static_cast<double>(errors) / static_cast<double>(bmu.size());
 }
 
 void Som::buildIndex(const std::vector<size_t> &bmu, std::vector<size_t> &counts, std::vector<size_t> &offsets, std::vector<unsigned> &rowIds) const
