@@ -33,7 +33,7 @@ F32 = np.float32
 STD, MED, CLR = 0, 1, 2
 ORDERS = pytest.mark.parametrize("order", [2, 0], ids=["eigen_sse", "seq"])
 VSOM_ERR_INVALID, VSOM_ERR_UNSUPPORTED = -1, -3
-TC_MIN_ROWS = 1024  # smallest first epoch whose BMU search goes through K2 (capi.cu kTcMinRows)
+TC_MIN_ROWS = 1024  # smallest first epoch whose BMU search goes through K2 (score_tc.cu kTcMinRows)
 
 
 # ------------------------------------------------------------------------------------------------ bench.py's generators

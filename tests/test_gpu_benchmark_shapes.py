@@ -27,7 +27,7 @@ pytestmark = [pytest.mark.gpu, pytest.mark.timeout(1800)]
 F32 = np.float32
 TAG_PERIOD = 512     # both online kernels tag their exchange keys with (t >> 1) & 0xff: a (row, tag) pair recurs every 512 steps
 PROBE = 8192         # rows of each K2 probe (score_tc.cu kTcProbeRows)
-TC_MIN_ROWS = 1024   # smallest batch the scoring calls send to K2 (capi.cu kTcMinRows)
+TC_MIN_ROWS = 1024   # smallest batch the scoring calls send to K2 (score_tc.cu kTcMinRows)
 
 
 # ------------------------------------------------------------------------------------------------ bench.py's generators

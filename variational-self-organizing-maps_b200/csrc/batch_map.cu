@@ -397,17 +397,16 @@ int launch_batch_epoch(vsom_ctx *ctx, const float *xDev, size_t n, double sigma,
     // ---- phase A; last_score_tc reports which search ran (K2's tier, or 0 for the exact scan and the local walks)
     if (isFirst)
     {
-        ctx->lastScoreTc = score_tc_supported(ctx) && n >= 1024;
-        if (ctx->lastScoreTc)
-            rc = launch_find_bmu_tc(ctx, xDev, n, 0, bmuDev, distDev, nullptr);
-        else
-            rc = launch_find_bmu(ctx, xDev, n, 0, bmuDev, distDev);
+        ScoreOut out;
+        out.bmu = bmuDev;
+        out.dist = distDev;
+        rc = score_rows(ctx, xDev, false, n, 0, true, out, nullptr);
         if (rc)
             return rc;
     }
     else
     {
-        ctx->lastScoreTc = 0;
+        ctx->lastScoreTier = 0;
         const unsigned grid = static_cast<unsigned>((n + 31) / 32);
         if (ctx->transform == VSOM_CLR)
             local_bmu_rows_kernel<VSOM_CLR><<<grid, 256, 0, ctx->stream>>>(xDev, n, ctx->mean, ctx->W, ctx->H, ctx->Din, ctx->Dr, ctx->P, ctx->rowStride,

@@ -643,173 +643,66 @@ int vsom_batch_epoch(vsom_ctx *ctx, const float *x, size_t n, double sigma, int 
     return VSOM_OK;
 }
 
-// Batches of at least kTcMinRows rows on a shape K2 covers take the tensor-core candidate search + exact rescore (same
-// results, bit for bit); everything else the exact scan.
-static const size_t kTcMinRows = 1024;
 static const char *kUnshardedOnly = "this entry point needs an unsharded context (scoring and index run on replicated maps)";
 
-// top = 2 (vsom_find_bmu2*): every row's runner-up as well, to out_bmu2 / out_dist2 (each may be null); same dispatch
-static int find_bmu_device_impl(vsom_ctx *ctx, const float *x_dev, size_t n, uint64_t min_hits, uint32_t *out_bmu_dev, float *out_dist_dev, bool allowTc,
-                                uint64_t *fallback_rows, const char *who, int top = 1, uint32_t *out_bmu2_dev = nullptr, float *out_dist2_dev = nullptr)
-{
-    if (ctx && ctx->world > 1)
-        return set_error(ctx, VSOM_ERR_UNSUPPORTED, kUnshardedOnly);
-    if (!ctx || (!x_dev && n))
-        return ctx ? set_error(ctx, VSOM_ERR_INVALID, std::string(who) + ": x is NULL") : VSOM_ERR_INVALID;
-    VSOM_CUDA(ctx, cudaSetDevice(ctx->device));
-    if (fallback_rows)
-        *fallback_rows = 0;
-    if (!allowTc || !score_tc_supported(ctx) || n < kTcMinRows)
-    {
-        if (fallback_rows)
-            *fallback_rows = n;
-        ctx->lastScoreTc = 0;
-        if (top == 2)
-            return launch_find_bmu2(ctx, x_dev, n, min_hits, out_bmu_dev, out_dist_dev, out_bmu2_dev, out_dist2_dev);
-        return launch_find_bmu(ctx, x_dev, n, min_hits, out_bmu_dev, out_dist_dev);
-    }
-    unsigned long long fb = 0;
-    ctx->lastScoreTc = 1;
-    const int rc = launch_find_bmu_tc(ctx, x_dev, n, min_hits, out_bmu_dev, out_dist_dev, &fb, top, out_bmu2_dev, out_dist2_dev);
-    if (fallback_rows)
-        *fallback_rows = fb;
-    return rc;
-}
-
-static int find_bmu_host_impl(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist, bool allowTc, uint64_t *fallback_rows,
-                              const char *who, int top = 1, uint32_t *out_bmu2 = nullptr, float *out_dist2 = nullptr)
+// the argument checks of the scoring entry points; score_rows (score_tc.cu) does the rest
+static int score_entry(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, uint64_t min_hits, bool allowTc, const ScoreOut &out, uint64_t *fallback_rows,
+                       const char *who)
 {
     if (ctx && ctx->world > 1)
         return set_error(ctx, VSOM_ERR_UNSUPPORTED, kUnshardedOnly);
     if (!ctx || (!x && n))
         return ctx ? set_error(ctx, VSOM_ERR_INVALID, std::string(who) + ": x is NULL") : VSOM_ERR_INVALID;
-    if (fallback_rows)
-        *fallback_rows = 0;
-    if (n == 0)
-        return VSOM_OK;
     VSOM_CUDA(ctx, cudaSetDevice(ctx->device));
-    if (allowTc && score_tc_supported(ctx) && n >= kTcMinRows)
-    {
-        // pipelined: H2D of slab i + 1, search + re-scoring of slab i and D2H of slab i - 1 overlap (score_tc.cu)
-        unsigned long long fb = 0;
-        size_t done = 0;
-        ctx->lastScoreTc = 1;
-        const int rc = launch_find_bmu_tc_host(ctx, x, n, min_hits, out_bmu, out_dist, &fb, &done, top, out_bmu2, out_dist2);
-        if (rc)
-            return rc;
-        if (done < n) // the probes found the map / data unsuited to the candidate search: the rest takes the exact path below
-        {
-            uint64_t rest = 0;
-            const int rc2 = find_bmu_host_impl(ctx, x + done * ctx->Din, n - done, min_hits, out_bmu ? out_bmu + done : nullptr, out_dist ? out_dist + done : nullptr, false,
-                                               &rest, who, top, out_bmu2 ? out_bmu2 + done : nullptr, out_dist2 ? out_dist2 + done : nullptr);
-            ctx->lastScoreTc = 1;
-            fb += rest;
-            if (rc2)
-                return rc2;
-        }
-        if (fallback_rows)
-            *fallback_rows = fb;
-        return VSOM_OK;
-    }
-    // exact scan from host rows, in slabs (a call can be the remainder of a very large batch that the probes took off the
-    // tensor-core path): staging stays bounded, results return per slab
-    const char *slabEnv = getenv("VSOM_EXACT_HOST_SLAB_LOG2"); // test knob
-    const size_t slab = std::min(n, static_cast<size_t>(1) << (slabEnv ? atoi(slabEnv) : 20));
-    int rc = stage_reserve(ctx, 0, sizeof(float) * slab * ctx->Din);
-    if (rc)
-        return rc;
-    rc = stage_reserve(ctx, 1, sizeof(unsigned) * slab);
-    if (rc)
-        return rc;
-    rc = stage_reserve(ctx, 2, sizeof(float) * slab);
-    if (rc)
-        return rc;
-    float *xDev = static_cast<float *>(ctx->stage[0]);
-    unsigned *bmuDev = static_cast<unsigned *>(ctx->stage[1]);
-    float *distDev = static_cast<float *>(ctx->stage[2]);
-    unsigned *bmu2Dev = nullptr; // top = 2: stage slot 4 holds the runner-ups and their distances
-    float *dist2Dev = nullptr;
-    if (top == 2)
-    {
-        rc = stage_reserve(ctx, 4, (sizeof(unsigned) + sizeof(float)) * slab);
-        if (rc)
-            return rc;
-        bmu2Dev = static_cast<unsigned *>(ctx->stage[4]);
-        dist2Dev = reinterpret_cast<float *>(bmu2Dev + slab);
-    }
-    if (fallback_rows)
-        *fallback_rows = n;
-    ctx->lastScoreTc = 0;
-    for (size_t r0 = 0; r0 < n; r0 += slab)
-    {
-        const size_t rows = std::min(slab, n - r0);
-        VSOM_CUDA(ctx, cudaMemcpyAsync(xDev, x + r0 * ctx->Din, sizeof(float) * rows * ctx->Din, cudaMemcpyHostToDevice, ctx->stream));
-        rc = top == 2 ? launch_find_bmu2(ctx, xDev, rows, min_hits, bmuDev, distDev, bmu2Dev, dist2Dev) : launch_find_bmu(ctx, xDev, rows, min_hits, bmuDev, distDev);
-        if (rc)
-            return rc;
-        rc = similarity_hook(ctx, xDev, rows, bmuDev, 0, ctx->stream); // armed by vsom_measure_similarity only
-        if (rc)
-            return rc;
-        ctx->simRowBase += rows;
-        if (out_bmu)
-            VSOM_CUDA(ctx, cudaMemcpyAsync(out_bmu + r0, bmuDev, sizeof(unsigned) * rows, cudaMemcpyDeviceToHost, ctx->stream));
-        if (out_dist)
-            VSOM_CUDA(ctx, cudaMemcpyAsync(out_dist + r0, distDev, sizeof(float) * rows, cudaMemcpyDeviceToHost, ctx->stream));
-        if (out_bmu2)
-            VSOM_CUDA(ctx, cudaMemcpyAsync(out_bmu2 + r0, bmu2Dev, sizeof(unsigned) * rows, cudaMemcpyDeviceToHost, ctx->stream));
-        if (out_dist2)
-            VSOM_CUDA(ctx, cudaMemcpyAsync(out_dist2 + r0, dist2Dev, sizeof(float) * rows, cudaMemcpyDeviceToHost, ctx->stream));
-        VSOM_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); // the staging buffers are reused by the next slab
-    }
-    return VSOM_OK;
+    return score_rows(ctx, x, hostRows, n, min_hits, allowTc, out, fallback_rows);
 }
 
 int vsom_find_bmu_device(vsom_ctx *ctx, const float *x_dev, size_t n, uint64_t min_hits, uint32_t *out_bmu_dev, float *out_dist_dev)
 {
-    return find_bmu_device_impl(ctx, x_dev, n, min_hits, out_bmu_dev, out_dist_dev, true, nullptr, "vsom_find_bmu_device");
+    return score_entry(ctx, x_dev, false, n, min_hits, true, ScoreOut{out_bmu_dev, out_dist_dev}, nullptr, "vsom_find_bmu_device");
 }
 
 int vsom_find_bmu(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist)
 {
-    return find_bmu_host_impl(ctx, x, n, min_hits, out_bmu, out_dist, true, nullptr, "vsom_find_bmu");
+    return score_entry(ctx, x, true, n, min_hits, true, ScoreOut{out_bmu, out_dist}, nullptr, "vsom_find_bmu");
 }
 
 int vsom_find_bmu_exact_device(vsom_ctx *ctx, const float *x_dev, size_t n, uint64_t min_hits, uint32_t *out_bmu_dev, float *out_dist_dev)
 {
-    return find_bmu_device_impl(ctx, x_dev, n, min_hits, out_bmu_dev, out_dist_dev, false, nullptr, "vsom_find_bmu_exact_device");
+    return score_entry(ctx, x_dev, false, n, min_hits, false, ScoreOut{out_bmu_dev, out_dist_dev}, nullptr, "vsom_find_bmu_exact_device");
 }
 
 int vsom_find_bmu_exact(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist)
 {
-    return find_bmu_host_impl(ctx, x, n, min_hits, out_bmu, out_dist, false, nullptr, "vsom_find_bmu_exact");
+    return score_entry(ctx, x, true, n, min_hits, false, ScoreOut{out_bmu, out_dist}, nullptr, "vsom_find_bmu_exact");
 }
 
 int vsom_find_bmu_batch_device(vsom_ctx *ctx, const float *x_dev, size_t n, uint64_t min_hits, uint32_t *out_bmu_dev, float *out_dist_dev,
                                uint64_t *fallback_rows)
 {
-    return find_bmu_device_impl(ctx, x_dev, n, min_hits, out_bmu_dev, out_dist_dev, true, fallback_rows, "vsom_find_bmu_batch_device");
+    return score_entry(ctx, x_dev, false, n, min_hits, true, ScoreOut{out_bmu_dev, out_dist_dev}, fallback_rows, "vsom_find_bmu_batch_device");
 }
 
 int vsom_find_bmu_batch(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist, uint64_t *fallback_rows)
 {
-    return find_bmu_host_impl(ctx, x, n, min_hits, out_bmu, out_dist, true, fallback_rows, "vsom_find_bmu_batch");
+    return score_entry(ctx, x, true, n, min_hits, true, ScoreOut{out_bmu, out_dist}, fallback_rows, "vsom_find_bmu_batch");
 }
 
 int vsom_find_bmu2(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist, uint32_t *out_bmu2, float *out_dist2,
                    uint64_t *fallback_rows)
 {
-    return find_bmu_host_impl(ctx, x, n, min_hits, out_bmu, out_dist, true, fallback_rows, "vsom_find_bmu2", 2, out_bmu2, out_dist2);
+    return score_entry(ctx, x, true, n, min_hits, true, ScoreOut{out_bmu, out_dist, out_bmu2, out_dist2, 2}, fallback_rows, "vsom_find_bmu2");
 }
 
 int vsom_find_bmu2_device(vsom_ctx *ctx, const float *x_dev, size_t n, uint64_t min_hits, uint32_t *out_bmu_dev, float *out_dist_dev, uint32_t *out_bmu2_dev,
                           float *out_dist2_dev, uint64_t *fallback_rows)
 {
-    return find_bmu_device_impl(ctx, x_dev, n, min_hits, out_bmu_dev, out_dist_dev, true, fallback_rows, "vsom_find_bmu2_device", 2, out_bmu2_dev, out_dist2_dev);
+    return score_entry(ctx, x_dev, false, n, min_hits, true, ScoreOut{out_bmu_dev, out_dist_dev, out_bmu2_dev, out_dist2_dev, 2}, fallback_rows, "vsom_find_bmu2_device");
 }
 
 int vsom_find_bmu2_exact(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist, uint32_t *out_bmu2, float *out_dist2)
 {
-    return find_bmu_host_impl(ctx, x, n, min_hits, out_bmu, out_dist, false, nullptr, "vsom_find_bmu2_exact", 2, out_bmu2, out_dist2);
+    return score_entry(ctx, x, true, n, min_hits, false, ScoreOut{out_bmu, out_dist, out_bmu2, out_dist2, 2}, nullptr, "vsom_find_bmu2_exact");
 }
 
 int vsom_debug_tc_stats(const vsom_ctx *ctx, uint64_t out[3])
@@ -821,8 +714,8 @@ int vsom_debug_tc_stats(const vsom_ctx *ctx, uint64_t out[3])
     return VSOM_OK;
 }
 
-int vsom_debug_last_score_tc(const vsom_ctx *ctx) { return ctx ? (ctx->lastScoreTc ? ctx->lastScoreTier : 0) : 0; }
-int vsom_debug_last_score_pair(const vsom_ctx *ctx) { return ctx ? (ctx->lastScoreTc ? ctx->lastScorePair : 0) : 0; }
+int vsom_debug_last_score_tc(const vsom_ctx *ctx) { return ctx ? ctx->lastScoreTier : 0; }
+int vsom_debug_last_score_pair(const vsom_ctx *ctx) { return ctx && ctx->lastScoreTier ? ctx->lastScorePair : 0; }
 
 int vsom_evaluate(vsom_ctx *ctx, const float *x, size_t n, double *mean_error)
 {
@@ -857,12 +750,12 @@ int vsom_measure_similarity(vsom_ctx *ctx, const float *x, size_t n, uint64_t mi
     int rc = stage_reserve(ctx, 9, sizeof(float) * n);
     if (rc)
         return rc;
-    ctx->simK = static_cast<float>(number_of_sigmas);
-    ctx->simHost = out_row_max;
-    ctx->simRowBase = 0;
-    rc = find_bmu_host_impl(ctx, x, n, min_hits, out_bmu, nullptr, true, nullptr, "vsom_measure_similarity");
-    ctx->simK = 0.0f;
-    ctx->simHost = nullptr;
+    ScoreOut out;
+    out.bmu = out_bmu;
+    out.rowMax = out_row_max;
+    out.rowMaxDev = static_cast<float *>(ctx->stage[9]);
+    out.k = static_cast<float>(number_of_sigmas);
+    rc = score_rows(ctx, x, true, n, min_hits, true, out, nullptr);
     if (rc)
         return rc;
     // the tensor-core path's result copies run on its re-scoring stream; tc_finish joined it to the context's stream

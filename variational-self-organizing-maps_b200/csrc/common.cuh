@@ -103,7 +103,7 @@ struct vsom_ctx
     cudaEvent_t evScore[2] = {}, evDone[2] = {}, evCopied[3] = {}, evSlabDone[3] = {}; // evCopied / evSlabDone: per host staging buffer (three)
     int tcAttrSet = 0;                          // K2's dynamic shared-memory opt-in was set on this context's device
     int tcPairOk = 0;                           // ... and the device can co-schedule a cluster of two K2 CTAs (cta_group::2 kernel)
-    int lastScorePair = 0;                      // the last K2 call ran the CTA-pair kernel
+    int lastScorePair = 0;                      // the last K2 search ran the CTA-pair kernel (reported while lastScoreTier != 0)
     float *mean = nullptr, *S = nullptr, *sigma = nullptr, *weight = nullptr;
     vsom::u64 *hits = nullptr;
     double *umatrix = nullptr;
@@ -122,14 +122,8 @@ struct vsom_ctx
     bool trainEnqueued = false;              // vsom_train_chunk_device work not yet checked for an abort
     bool poisoned = false;                   // an online-step chunk aborted: the context refuses further chunks
     unsigned long long tcStats[3] = {0, 0, 0}; // K2 fallback causes since creation: list overflow, NaN / nothing eligible, certificate
-    int lastScoreTier = 0;                   // precision tier of the last K2 call (1: one half per operand, 2: hi / lo pairs)
-    int lastScoreTc = 0;                     // the last scoring call ran K2 (tensor-core search + exact rescore)
-    unsigned long long lastFallbackRows = 0; // rows of the last tensor-core scoring call that needed the exact full scan
-    // vsom_measure_similarity: while simK != 0 every host-buffer scoring slab also gets its rows' largest normalised deviation
-    // from their BMU (stage slot 9, absolute row index = simRowBase + row inside the running sub-call), copied to simHost
-    float simK = 0.0f;
-    float *simHost = nullptr;
-    size_t simRowBase = 0;
+    int lastScoreTier = 0;                   // path of the last scoring call (score_rows): 0 the exact scan, else K2's tier (1: one half
+                                             // per operand, 2: hi / lo pairs, 3: the probes sent the rest to the exact scan)
     int gridTrain = 0, residentTrain = 0, smStrideTrain = 0;
     size_t smemTrain = 0;
     uint64_t launches = 0;
@@ -170,28 +164,55 @@ int stage_reserve(vsom_ctx *ctx, int slot, size_t bytes);
             return ::vsom::cuda_fail((ctx), _e, #call, __FILE__, __LINE__);    \
     } while (0)
 
+// The per-row results of one scoring call; every pointer may be null.  All of them are in the memory of the call's rows: device
+// memory for device rows, host memory for host rows (rowMaxDev is always device memory).
+struct ScoreOut
+{
+    unsigned *bmu = nullptr;
+    float *dist = nullptr;
+    unsigned *bmu2 = nullptr; // top == 2 (vsom_find_bmu2): every row's runner-up and its distance
+    float *dist2 = nullptr;
+    int top = 1;
+    // vsom_measure_similarity (k != 0, host rows only): each row's largest normalised deviation from its BMU, computed into
+    // rowMaxDev behind the row's final BMU and copied to rowMax
+    float *rowMax = nullptr;
+    float *rowMaxDev = nullptr;
+    float k = 0.0f;
+
+    // the same outputs from row r on
+    ScoreOut at(size_t r) const
+    {
+        ScoreOut o = *this;
+        auto shift = [r](auto *&p) {
+            if (p)
+                p += r;
+        };
+        shift(o.bmu);
+        shift(o.dist);
+        shift(o.bmu2);
+        shift(o.dist2);
+        shift(o.rowMax);
+        shift(o.rowMaxDev);
+        return o;
+    }
+};
+
 // kernels' host launchers (each returns a vsom_status)
 int launch_online_step(vsom_ctx *ctx, const float *xDev, size_t n, double eta, double sigma, int decay, unsigned *outBmuDev, float *outDistDev,
                        const u64 *lastInDev = nullptr);
 int configure_online_step(vsom_ctx *ctx);
 int configure_online_step_fast(vsom_ctx *ctx);                               // 1: K1F eligible for this context
 int launch_online_step_fast(vsom_ctx *ctx, StepParams &p, double sigma);      // 1: enqueued, 0: not eligible, < 0: error
-int launch_find_bmu(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, unsigned *outBmuDev, float *outDistDev);
-int launch_find_bmu_list(vsom_ctx *ctx, const float *xDev, size_t n, const unsigned *rowListDev, const unsigned *rowCountDev, uint64_t minHits, unsigned *outBmuDev,
-                         float *outDistDev, cudaStream_t stream, u64 *keyBufDev, int top = 1, unsigned *outBmu2Dev = nullptr, float *outDist2Dev = nullptr);
-// the exact scan with every row's runner-up as well (vsom_find_bmu2)
-int launch_find_bmu2(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, unsigned *outBmuDev, float *outDistDev, unsigned *outBmu2Dev, float *outDist2Dev);
-bool score_tc_supported(const vsom_ctx *ctx);
-// top = 2 (vsom_find_bmu2): the best two nodes of every row; outBmu2 / outDist2 may be null
-int launch_find_bmu_tc(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, unsigned *outBmuDev, float *outDistDev, unsigned long long *fallbackRowsOut,
-                       int top = 1, unsigned *outBmu2Dev = nullptr, float *outDist2Dev = nullptr);
-int launch_find_bmu_tc_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t minHits, unsigned *outBmuHost, float *outDistHost, unsigned long long *fallbackRowsOut,
-                            size_t *rowsDoneOut, int top = 1, unsigned *outBmu2Host = nullptr, float *outDist2Host = nullptr);
+// Every scoring call: x holds n rows (host memory when hostRows), results go to `out`.  Chooses K2 or the exact scan, runs K2's
+// tiers and the exact scan of the rows K2 leaves, and records the path for vsom_debug_last_score_tc (score_tc.cu).
+int score_rows(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, uint64_t minHits, bool allowTc, const ScoreOut &out, uint64_t *fallbackRows);
+// The exact scan (K3) of rows 0 .. n-1 of xDev, or (rowListDev != null) of the rows rowListDev[0 .. *rowCountDev)
+int launch_find_bmu_list(vsom_ctx *ctx, const float *xDev, size_t n, const unsigned *rowListDev, const unsigned *rowCountDev, uint64_t minHits, const ScoreOut &out,
+                         cudaStream_t stream, u64 *keyBufDev);
 int launch_batch_epoch(vsom_ctx *ctx, const float *xDev, size_t n, double sigma, int isFirst, const u64 *lastDev, unsigned *bmuDev, float *distDev);
 int launch_all_dists(vsom_ctx *ctx, const float *vDev, double *outDev);
 int launch_soft_assign(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, double *probDev, double *sumsDev);
 int launch_similarity_rowmax(vsom_ctx *ctx, const float *xDev, size_t rows, const unsigned *bmuDev, float k, float *outDev, cudaStream_t stream);
-int similarity_hook(vsom_ctx *ctx, const float *xDev, size_t rows, const unsigned *bmuDev, size_t rowInCall, cudaStream_t stream);
 int launch_umatrix_tiles(vsom_ctx *ctx, const float *const *meanRowDev, const float *const *sigmaRowDev, const int2 *tilesDev, int nTiles);
 int umatrix_tile_rows();
 int launch_build_index(vsom_ctx *ctx, const unsigned *bmuDev, size_t n, u64 *countsDev, u64 *offsetsDev, unsigned *rowIdsDev);

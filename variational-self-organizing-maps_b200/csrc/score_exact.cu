@@ -544,10 +544,10 @@ int launch_soft_assign(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minH
 }
 
 // rowListDev == null: rows 0 .. n-1 of xDev.  Otherwise the rows rowListDev[0 .. *rowCountDev) (at most n of them) — the exact
-// scan of the rows a tensor-core slab could not certify, the count staying on the device; keyBufDev: top * n u64 of scratch.
-// top = 2: the runner-up of every row as well (outBmu2Dev / outDist2Dev, each may be null).
-int launch_find_bmu_list(vsom_ctx *ctx, const float *xDev, size_t n, const unsigned *rowListDev, const unsigned *rowCountDev, uint64_t minHits, unsigned *outBmuDev,
-                         float *outDistDev, cudaStream_t stream, u64 *keyBufDev, int top, unsigned *outBmu2Dev, float *outDist2Dev)
+// scan of the rows a tensor-core slab could not certify, the count staying on the device; keyBufDev: out.top * n u64 of scratch.
+// out.top = 2: the runner-up of every row as well.
+int launch_find_bmu_list(vsom_ctx *ctx, const float *xDev, size_t n, const unsigned *rowListDev, const unsigned *rowCountDev, uint64_t minHits, const ScoreOut &out,
+                         cudaStream_t stream, u64 *keyBufDev)
 {
     if (n == 0)
         return VSOM_OK;
@@ -559,8 +559,8 @@ int launch_find_bmu_list(vsom_ctx *ctx, const float *xDev, size_t n, const unsig
     const unsigned grid = list ? static_cast<unsigned>(std::min<size_t>((n + tileRows - 1) / tileRows * splits, static_cast<size_t>(ctx->numSMs) * 4))
                                : static_cast<unsigned>((n + tileRows - 1) / tileRows);
     if (list)
-        VSOM_CUDA(ctx, cudaMemsetAsync(keyBufDev, 0xff, sizeof(u64) * n * (top == 2 ? 2 : 1), stream));
-#define VSOM_SCORE_ARGS xDev, n, rowListDev, rowCountDev, ctx->mean, ctx->hits, minHits, ctx->N, ctx->Din, ctx->Dr, ctx->P, ctx->rowStride, ctx->pairI, ctx->pairJ, outBmuDev, outDistDev, splits, keyBufDev, outBmu2Dev, outDist2Dev
+        VSOM_CUDA(ctx, cudaMemsetAsync(keyBufDev, 0xff, sizeof(u64) * n * (out.top == 2 ? 2 : 1), stream));
+#define VSOM_SCORE_ARGS xDev, n, rowListDev, rowCountDev, ctx->mean, ctx->hits, minHits, ctx->N, ctx->Din, ctx->Dr, ctx->P, ctx->rowStride, ctx->pairI, ctx->pairJ, out.bmu, out.dist, splits, keyBufDev, out.bmu2, out.dist2
 #define VSOM_SCORE_LAUNCH(TOP)                                                                                                   \
     if (eigen)                                                                                                                   \
     {                                                                                                                            \
@@ -573,7 +573,7 @@ int launch_find_bmu_list(vsom_ctx *ctx, const float *xDev, size_t n, const unsig
         find_bmu_exact_kernel<VSOM_CLR, TOP><<<grid, kScoreThreads, 0, stream>>>(VSOM_SCORE_ARGS);                              \
     else /* Standard and Median share the Comparer (src/Transformation.cpp:7-8, :45-46) */                                       \
         find_bmu_exact_kernel<VSOM_STANDARD, TOP><<<grid, kScoreThreads, 0, stream>>>(VSOM_SCORE_ARGS);
-    if (top == 2)
+    if (out.top == 2)
     {
         VSOM_SCORE_LAUNCH(2)
     }
@@ -587,24 +587,14 @@ int launch_find_bmu_list(vsom_ctx *ctx, const float *xDev, size_t n, const unsig
     if (list)
     {
         const unsigned fgrid = std::min(1024u, static_cast<unsigned>((n + 255) / 256));
-        if (top == 2)
-            finalize_list2_kernel<<<fgrid, 256, 0, stream>>>(rowListDev, rowCountDev, keyBufDev, outBmuDev, outDistDev, outBmu2Dev, outDist2Dev);
+        if (out.top == 2)
+            finalize_list2_kernel<<<fgrid, 256, 0, stream>>>(rowListDev, rowCountDev, keyBufDev, out.bmu, out.dist, out.bmu2, out.dist2);
         else
-            finalize_list_kernel<<<fgrid, 256, 0, stream>>>(rowListDev, rowCountDev, keyBufDev, outBmuDev, outDistDev);
+            finalize_list_kernel<<<fgrid, 256, 0, stream>>>(rowListDev, rowCountDev, keyBufDev, out.bmu, out.dist);
         ctx->launches += 1;
     }
     VSOM_CUDA(ctx, cudaGetLastError());
     return VSOM_OK;
-}
-
-int launch_find_bmu(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, unsigned *outBmuDev, float *outDistDev)
-{
-    return launch_find_bmu_list(ctx, xDev, n, nullptr, nullptr, minHits, outBmuDev, outDistDev, ctx->stream, nullptr);
-}
-
-int launch_find_bmu2(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, unsigned *outBmuDev, float *outDistDev, unsigned *outBmu2Dev, float *outDist2Dev)
-{
-    return launch_find_bmu_list(ctx, xDev, n, nullptr, nullptr, minHits, outBmuDev, outDistDev, ctx->stream, nullptr, 2, outBmu2Dev, outDist2Dev);
 }
 
 // ---- Som::measureSimilarity's per-row pass (src/Som.cpp:631-714): delta_n = ((v_n - m_n) / sM_n) / numOfSigmas against the row's BMU,
@@ -648,20 +638,6 @@ int launch_similarity_rowmax(vsom_ctx *ctx, const float *xDev, size_t rows, cons
     similarity_rowmax_kernel<<<static_cast<unsigned>((rows + 7) / 8), 256, 0, stream>>>(xDev, rows, ctx->Din, ctx->mean, ctx->sigma, ctx->rowStride, bmuDev, k, outDev);
     ctx->launches += 1;
     VSOM_CUDA(ctx, cudaGetLastError());
-    return VSOM_OK;
-}
-
-// called by the host-buffer scoring paths behind a slab's final BMUs (stream-ordered); no-op unless vsom_measure_similarity armed it
-int similarity_hook(vsom_ctx *ctx, const float *xDev, size_t rows, const unsigned *bmuDev, size_t rowInCall, cudaStream_t stream)
-{
-    if (ctx->simK == 0.0f || !ctx->stage[9])
-        return VSOM_OK;
-    float *dst = static_cast<float *>(ctx->stage[9]) + ctx->simRowBase + rowInCall;
-    const int rc = launch_similarity_rowmax(ctx, xDev, rows, bmuDev, ctx->simK, dst, stream);
-    if (rc)
-        return rc;
-    if (ctx->simHost)
-        VSOM_CUDA(ctx, cudaMemcpyAsync(ctx->simHost + ctx->simRowBase + rowInCall, dst, sizeof(float) * rows, cudaMemcpyDeviceToHost, stream));
     return VSOM_OK;
 }
 

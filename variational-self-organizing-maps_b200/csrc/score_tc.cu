@@ -50,7 +50,7 @@
 //   warps 4-11 epilogue   : two threads per row (TMEM lane), 128 columns each; tcgen05.ld 32 columns at a time (next
 //                           chunk in flight); per chunk a tree of FMNMX3 (the accumulators ARE the scores), one vote, and
 //                           only for flagged groups of four columns the predicated appends to the thread's list
-// Two precision tiers (one fp16 per operand element / hi-lo pairs, three products) — see launch_find_bmu_tc.
+// Two precision tiers (one fp16 per operand element / hi-lo pairs, three products) — see tc_score_tiers.
 // Measured (round 2, 128x128x256, ncu): pipeline without epilogue 93 % / 97 % tensor-pipe active (tier 1 / 2); an epilogue that only
 // reads the accumulators (tcgen05.ld, no scoring) 92 % / 97 %; the real one 72 % / 95 %.  So the TMEM reads fit under the K = 272
 // contraction of a tile; what costs tier 1 its last 20 % is the latency chain of the scoring code (min tree -> vote -> branch) with two
@@ -1050,9 +1050,6 @@ static int make_map(vsom_ctx *ctx, CUtensorMap *map, void *base, unsigned long l
     return VSOM_OK;
 }
 
-// Standard / Median Comparer (the contraction form of |m - x|^2); rows longer than TC_MAXK stream their A k-blocks
-bool score_tc_supported(const vsom_ctx *ctx) { return ctx->transform != VSOM_CLR && ctx->Dm <= 2048; }
-
 // One batched scoring call: tc_begin (map side, once) -> tc_enqueue per slab of rows (no host synchronisation) -> tc_finish.
 // stage slots used: 6 = fp16 map operand + statistics, 7 = fp16 rows of the current slab, 8 = per-row scratch (two sets).
 struct TcCall
@@ -1165,12 +1162,31 @@ static int tc_begin(vsom_ctx *ctx, TcCall &c, size_t maxSlabRows, uint64_t minHi
     return VSOM_OK;
 }
 
-// One slab: xs = rows x D f32 in device memory (must stay valid until the slab's evDone event).  Results go to outBmuDev /
-// outDistDev (device, may be null) and, when given, from there to host memory on the re-scoring stream.
-// c.top = 2: the runner-up as well, to outBmu2Dev / outDist2Dev and from there to outBmu2Host / outDist2Host (each may be null).
-static int tc_enqueue(vsom_ctx *ctx, TcCall &c, const float *xs, size_t rows, unsigned *outBmuDev, float *outDistDev, unsigned *outBmuHost, float *outDistHost,
-                      size_t rowInCall = 0, bool hostCall = false, unsigned *outBmu2Dev = nullptr, float *outDist2Dev = nullptr, unsigned *outBmu2Host = nullptr,
-                      float *outDist2Host = nullptr)
+// Host rows: the results of a slab are final in `dev` (device staging).  Behind them on `stream`: the similarity pass, then the
+// copies to the caller's buffers in `host`.
+static int slab_to_host(vsom_ctx *ctx, const float *xs, size_t rows, const ScoreOut &dev, const ScoreOut &host, cudaStream_t stream)
+{
+    if (host.k != 0.0f)
+    {
+        const int rc = launch_similarity_rowmax(ctx, xs, rows, dev.bmu, host.k, host.rowMaxDev, stream);
+        if (rc)
+            return rc;
+        VSOM_CUDA(ctx, cudaMemcpyAsync(host.rowMax, host.rowMaxDev, sizeof(float) * rows, cudaMemcpyDeviceToHost, stream));
+    }
+    if (host.bmu)
+        VSOM_CUDA(ctx, cudaMemcpyAsync(host.bmu, dev.bmu, sizeof(unsigned) * rows, cudaMemcpyDeviceToHost, stream));
+    if (host.dist)
+        VSOM_CUDA(ctx, cudaMemcpyAsync(host.dist, dev.dist, sizeof(float) * rows, cudaMemcpyDeviceToHost, stream));
+    if (host.bmu2)
+        VSOM_CUDA(ctx, cudaMemcpyAsync(host.bmu2, dev.bmu2, sizeof(unsigned) * rows, cudaMemcpyDeviceToHost, stream));
+    if (host.dist2)
+        VSOM_CUDA(ctx, cudaMemcpyAsync(host.dist2, dev.dist2, sizeof(float) * rows, cudaMemcpyDeviceToHost, stream));
+    return VSOM_OK;
+}
+
+// One slab: xs = rows x D f32 in device memory (must stay valid until the slab's evDone event).  Results go to `dev` (device
+// memory, top = c.top) and, for host rows, from there to `host` on the re-scoring stream.
+static int tc_enqueue(vsom_ctx *ctx, TcCall &c, const float *xs, size_t rows, const ScoreOut &dev, const ScoreOut *host)
 {
     const int par = static_cast<int>(c.slab & 1);
     unsigned char *set = static_cast<unsigned char *>(ctx->stage[8]) + par * c.setBytes;
@@ -1225,27 +1241,19 @@ static int tc_enqueue(vsom_ctx *ctx, TcCall &c, const float *xs, size_t rows, un
     VSOM_CUDA(ctx, cudaEventRecord(ctx->evScore[par], ctx->stream));
     VSOM_CUDA(ctx, cudaStreamWaitEvent(rs, ctx->evScore[par], 0));
     (c.top == 2 ? rescore_kernel<2> : rescore_kernel<1>)<<<static_cast<unsigned>((rows + RS_ROWS - 1) / RS_ROWS), RS_THREADS, 0, rs>>>(
-        xs, static_cast<long long>(rows), c.D, ctx->mean, ctx->rowStride, cand, candCount, bestA, xnorm, xratio, c.scale, c.Kpad, order, c.N, ctx->hits, c.minHits, outBmuDev,
-        outDistDev, fbRows, fbCount, c.totalDev, outBmu2Dev, outDist2Dev);
+        xs, static_cast<long long>(rows), c.D, ctx->mean, ctx->rowStride, cand, candCount, bestA, xnorm, xratio, c.scale, c.Kpad, order, c.N, ctx->hits, c.minHits, dev.bmu,
+        dev.dist, fbRows, fbCount, c.totalDev, dev.bmu2, dev.dist2);
     // rows the certificate rejected: exact scan (K3 tiles over the row list; the count stays on the device)
     add_count_kernel<<<1, 1, 0, rs>>>(fbCount, c.totalDev);
-    rc = launch_find_bmu_list(ctx, xs, rows, fbRows, fbCount, c.minHits, outBmuDev, outDistDev, rs, fbKeys, c.top, outBmu2Dev, outDist2Dev);
+    rc = launch_find_bmu_list(ctx, xs, rows, fbRows, fbCount, c.minHits, dev, rs, fbKeys);
     if (rc)
         return rc;
-    if (hostCall && outBmuDev) // vsom_measure_similarity: the slab's rows are still on the device and its BMUs are final
+    if (host)
     {
-        rc = similarity_hook(ctx, xs, rows, outBmuDev, rowInCall, rs);
+        rc = slab_to_host(ctx, xs, rows, dev, *host, rs);
         if (rc)
             return rc;
     }
-    if (outBmuHost && outBmuDev)
-        VSOM_CUDA(ctx, cudaMemcpyAsync(outBmuHost, outBmuDev, sizeof(unsigned) * rows, cudaMemcpyDeviceToHost, rs));
-    if (outDistHost && outDistDev)
-        VSOM_CUDA(ctx, cudaMemcpyAsync(outDistHost, outDistDev, sizeof(float) * rows, cudaMemcpyDeviceToHost, rs));
-    if (outBmu2Host && outBmu2Dev)
-        VSOM_CUDA(ctx, cudaMemcpyAsync(outBmu2Host, outBmu2Dev, sizeof(unsigned) * rows, cudaMemcpyDeviceToHost, rs));
-    if (outDist2Host && outDist2Dev)
-        VSOM_CUDA(ctx, cudaMemcpyAsync(outDist2Host, outDist2Dev, sizeof(float) * rows, cudaMemcpyDeviceToHost, rs));
     VSOM_CUDA(ctx, cudaEventRecord(ctx->evDone[par], rs));
     ctx->launches += 4;
     VSOM_CUDA(ctx, cudaGetLastError());
@@ -1253,12 +1261,13 @@ static int tc_enqueue(vsom_ctx *ctx, TcCall &c, const float *xs, size_t rows, un
     return VSOM_OK;
 }
 
-static int tc_finish(vsom_ctx *ctx, TcCall &c, unsigned long long *fallbackRowsOut)
+// fallbackRows: rows of this run that took the exact scan
+static int tc_finish(vsom_ctx *ctx, TcCall &c, unsigned long long &fallbackRows)
 {
     // the context's stream owns the results again
     for (int i = 0; i < 2 && static_cast<size_t>(i) < c.slab; ++i)
         VSOM_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->evDone[i], 0));
-    unsigned long long totalFallback = 0, st[4] = {0, 0, 0, 0};
+    unsigned long long st[4] = {0, 0, 0, 0};
     int flag = 0;
     VSOM_CUDA(ctx, cudaMemcpyAsync(st, c.totalDev, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
     VSOM_CUDA(ctx, cudaMemcpyAsync(&flag, ctx->errFlag, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1266,12 +1275,9 @@ static int tc_finish(vsom_ctx *ctx, TcCall &c, unsigned long long *fallbackRowsO
     if (flag)
         return set_error(ctx, VSOM_ERR_TIMEOUT, "score_tc: pipeline barrier timed out (kernel bug)");
     VSOM_CUDA(ctx, cudaGetLastError());
-    totalFallback = st[0];
+    fallbackRows = st[0];
     for (int i = 0; i < 3; ++i)
         ctx->tcStats[i] += st[i + 1];
-    if (fallbackRowsOut)
-        *fallbackRowsOut = totalFallback;
-    ctx->lastFallbackRows = totalFallback;
     return VSOM_OK;
 }
 
@@ -1291,14 +1297,14 @@ static size_t tc_slab_cap(const vsom_ctx *ctx, int split)
 }
 
 // The tier policy of both forms.  run(r0, rows, tier, fb) scores rows [r0, r0 + rows) through tier 1 or 2 and sets fb to the
-// number of them that took the exact scan.  On return `done` rows have been scored (all n, unless the tier-2 probe chose
-// tier 3: then rows [done, n) are left to the caller's exact scan) and `fallback` of them took the exact scan.
+// number of them that took the exact scan.  On return `tier` is the tier chosen, `done` rows have been scored (all n, unless
+// the tier-2 probe chose tier 3: then rows [done, n) are left to the exact scan) and `fallback` of them took the exact scan.
 template <class Run>
-static int tc_score_tiers(vsom_ctx *ctx, size_t n, const Run &run, size_t &done, unsigned long long &fallback)
+static int tc_score_tiers(size_t n, const Run &run, int &tier, size_t &done, unsigned long long &fallback)
 {
     const char *e = getenv("VSOM_TC_TIER");
     const int forced = e ? atoi(e) : 0;
-    int tier = forced;
+    tier = forced;
     unsigned long long fb = 0;
     done = 0;
     fallback = 0;
@@ -1324,7 +1330,6 @@ static int tc_score_tiers(vsom_ctx *ctx, size_t n, const Run &run, size_t &done,
         if (static_cast<double>(fb) > kTcExactSwitch * static_cast<double>(kTcProbeRows))
             tier = 3;
     }
-    ctx->lastScoreTier = tier;
     if (done < n && tier != 3)
     {
         const int rc = run(done, n - done, tier, fb);
@@ -1333,70 +1338,32 @@ static int tc_score_tiers(vsom_ctx *ctx, size_t n, const Run &run, size_t &done,
         fallback += fb;
         done = n;
     }
-    ctx->lastFallbackRows = fallback;
     return VSOM_OK;
 }
 
 // rows [0, n) of xDev through one tier; slabs of the given size
-static int tc_run_device(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, int split, size_t slabRows, unsigned *outBmuDev, float *outDistDev,
-                         unsigned long long *fallbackRowsOut, int top, unsigned *outBmu2Dev, float *outDist2Dev)
+static int tc_run_device(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, int split, size_t slabRows, const ScoreOut &out, unsigned long long &fallbackRows)
 {
     slabRows = std::min(n, std::min(slabRows, tc_slab_cap(ctx, split)));
     TcCall c;
-    int rc = tc_begin(ctx, c, slabRows, minHits, split, top);
+    int rc = tc_begin(ctx, c, slabRows, minHits, split, out.top);
     if (rc)
         return rc;
     for (size_t r0 = 0; r0 < n; r0 += slabRows)
     {
-        rc = tc_enqueue(ctx, c, xDev + r0 * c.D, std::min(slabRows, n - r0), outBmuDev ? outBmuDev + r0 : nullptr, outDistDev ? outDistDev + r0 : nullptr, nullptr, nullptr, 0,
-                        false, outBmu2Dev ? outBmu2Dev + r0 : nullptr, outDist2Dev ? outDist2Dev + r0 : nullptr);
+        rc = tc_enqueue(ctx, c, xDev + r0 * c.D, std::min(slabRows, n - r0), out.at(r0), nullptr);
         if (rc)
             return rc;
     }
-    return tc_finish(ctx, c, fallbackRowsOut);
+    return tc_finish(ctx, c, fallbackRows);
 }
 
-int launch_find_bmu_tc(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, unsigned *outBmuDev, float *outDistDev, unsigned long long *fallbackRowsOut,
-                       int top, unsigned *outBmu2Dev, float *outDist2Dev)
-{
-    if (!score_tc_supported(ctx))
-        return set_error(ctx, VSOM_ERR_UNSUPPORTED, "score_tc: needs a Standard/Median transformation and Dm <= 2048");
-    if (fallbackRowsOut)
-        *fallbackRowsOut = 0;
-    if (n == 0)
-        return VSOM_OK;
-    // test knob; smaller slabs measured slower (per-slab ramp and tail of the persistent kernel)
-    const char *slabEnv = getenv("VSOM_TC_SLAB_LOG2");
-    const size_t slab1 = static_cast<size_t>(1) << (slabEnv ? atoi(slabEnv) : 22), slab2 = std::min<size_t>(slab1, static_cast<size_t>(1) << 20);
-    size_t done = 0;
-    unsigned long long total = 0;
-    int rc = tc_score_tiers(
-        ctx, n,
-        [&](size_t r0, size_t rows, int tier, unsigned long long &fb) {
-            return tc_run_device(ctx, xDev + r0 * ctx->Dm, rows, minHits, tier == 2 ? 1 : 0, tier == 2 ? slab2 : slab1, outBmuDev ? outBmuDev + r0 : nullptr,
-                                 outDistDev ? outDistDev + r0 : nullptr, &fb, top, outBmu2Dev ? outBmu2Dev + r0 : nullptr, outDist2Dev ? outDist2Dev + r0 : nullptr);
-        },
-        done, total);
-    if (rc)
-        return rc;
-    if (done < n) // tier 3
-    {
-        rc = launch_find_bmu_list(ctx, xDev + done * ctx->Dm, n - done, nullptr, nullptr, minHits, outBmuDev ? outBmuDev + done : nullptr,
-                                  outDistDev ? outDistDev + done : nullptr, ctx->stream, nullptr, top, outBmu2Dev ? outBmu2Dev + done : nullptr,
-                                  outDist2Dev ? outDist2Dev + done : nullptr);
-        if (rc)
-            return rc;
-        total += n - done;
-        ctx->lastFallbackRows = total;
-    }
-    if (fallbackRowsOut)
-        *fallbackRowsOut = total;
-    return VSOM_OK;
-}
-
-// rows [0, n) of xHost through one tier, pipelined over the copy / search / re-scoring streams
-static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t minHits, int split, size_t slabRows, unsigned *outBmuHost, float *outDistHost,
-                       unsigned long long *fallbackRowsOut, int top, unsigned *outBmu2Host, float *outDist2Host)
+// Rows in HOST memory (the call Som::evaluate / measureSimilarity / mapDataSet make), rows [0, n) through one tier: the chunk
+// crosses PCIe in slabs on a copy stream into one of three staging buffers while the previous slabs are searched and re-scored,
+// and each slab's results return to the host behind its re-scoring.  With pinned host memory the three engines (H2D, SMs, D2H)
+// overlap fully; the call is then bound by the slower of PCIe (4 D bytes per row) and the kernel.  stage slots: 0 = three row
+// slabs, 1 / 2 = BMU / distance of the whole run, 4 = runner-ups and their distances (top = 2).
+static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t minHits, int split, size_t slabRows, const ScoreOut &out, unsigned long long &fallbackRows)
 {
     slabRows = std::min(n, std::min(slabRows, tc_slab_cap(ctx, split)));
     const size_t D = static_cast<size_t>(ctx->Dm);
@@ -1414,20 +1381,20 @@ static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t min
     float *xbuf[3];
     for (int i = 0; i < 3; ++i)
         xbuf[i] = static_cast<float *>(ctx->stage[0]) + static_cast<size_t>(i) * slabRows * D;
-    unsigned *bmuDev = static_cast<unsigned *>(ctx->stage[1]);
-    float *distDev = static_cast<float *>(ctx->stage[2]);
-    unsigned *bmu2Dev = nullptr; // top = 2: stage slot 4 holds the runner-ups and their distances
-    float *dist2Dev = nullptr;
-    if (top == 2)
+    ScoreOut dev;
+    dev.bmu = static_cast<unsigned *>(ctx->stage[1]);
+    dev.dist = static_cast<float *>(ctx->stage[2]);
+    dev.top = out.top;
+    if (out.top == 2)
     {
         rc = stage_reserve(ctx, 4, (sizeof(unsigned) + sizeof(float)) * n);
         if (rc)
             return rc;
-        bmu2Dev = static_cast<unsigned *>(ctx->stage[4]);
-        dist2Dev = reinterpret_cast<float *>(bmu2Dev + n);
+        dev.bmu2 = static_cast<unsigned *>(ctx->stage[4]);
+        dev.dist2 = reinterpret_cast<float *>(dev.bmu2 + n);
     }
     TcCall c;
-    rc = tc_begin(ctx, c, slabRows, minHits, split, top);
+    rc = tc_begin(ctx, c, slabRows, minHits, split, out.top);
     if (rc)
         return rc;
     // the staging buffers may still be in use by earlier work of the context's stream
@@ -1452,9 +1419,8 @@ static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t min
         const size_t r0 = sl * slabRows, rows = std::min(slabRows, n - r0);
         const int b = static_cast<int>(sl % 3);
         VSOM_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->evCopied[b], 0));
-        rc = tc_enqueue(ctx, c, xbuf[b], rows, bmuDev + r0, distDev + r0, outBmuHost ? outBmuHost + r0 : nullptr, outDistHost ? outDistHost + r0 : nullptr, r0, true,
-                        bmu2Dev ? bmu2Dev + r0 : nullptr, dist2Dev ? dist2Dev + r0 : nullptr, outBmu2Host ? outBmu2Host + r0 : nullptr,
-                        outDist2Host ? outDist2Host + r0 : nullptr);
+        const ScoreOut host = out.at(r0);
+        rc = tc_enqueue(ctx, c, xbuf[b], rows, dev.at(r0), &host);
         if (rc)
             return rc;
         VSOM_CUDA(ctx, cudaEventRecord(ctx->evSlabDone[b], ctx->auxStream)); // behind the slab's re-scoring and result copies
@@ -1466,43 +1432,96 @@ static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t min
                 return rc;
         }
     }
-    rc = tc_finish(ctx, c, fallbackRowsOut);
-    ctx->simRowBase += n; // the next sub-call of the same scoring call (probe / remainder) continues behind these rows
-    return rc;
+    return tc_finish(ctx, c, fallbackRows);
 }
 
-// Rows in HOST memory (the call Som::evaluate / measureSimilarity / mapDataSet make): the chunk crosses PCIe in slabs on a
-// copy stream into one of three staging buffers while the previous slabs are searched and re-scored, and each slab's results
-// return to the host behind its re-scoring.  With pinned host memory the three engines (H2D, SMs, D2H) overlap fully; the
-// call is then bound by the slower of PCIe (4 D bytes per row) and the kernel.  stage slots: 0 = three row slabs,
-// 1 / 2 = BMU / distance of the whole call.  Same probe and tier choice as the device form.
-int launch_find_bmu_tc_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t minHits, unsigned *outBmuHost, float *outDistHost, unsigned long long *fallbackRowsOut,
-                            size_t *rowsDoneOut, int top, unsigned *outBmu2Host, float *outDist2Host)
+// The exact scan of rows in HOST memory, in slabs (VSOM_EXACT_HOST_SLAB_LOG2, default 2^20 rows): staging stays bounded and each
+// slab's results return before the next slab is copied in.  stage slots as tc_run_host, sized by the slab.
+static int score_exact_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t minHits, const ScoreOut &out)
 {
-    if (!score_tc_supported(ctx))
-        return set_error(ctx, VSOM_ERR_UNSUPPORTED, "score_tc: needs a Standard/Median transformation and Dm <= 2048");
-    if (fallbackRowsOut)
-        *fallbackRowsOut = 0;
-    if (n == 0)
-        return VSOM_OK;
-    const char *slabEnv = getenv("VSOM_TC_HOST_SLAB_LOG2");
-    const size_t slabRows = static_cast<size_t>(1) << (slabEnv ? atoi(slabEnv) : 19);
-    size_t done = 0;
-    unsigned long long total = 0;
-    const int rc = tc_score_tiers(
-        ctx, n,
-        [&](size_t r0, size_t rows, int tier, unsigned long long &fb) {
-            return tc_run_host(ctx, xHost + r0 * ctx->Dm, rows, minHits, tier == 2 ? 1 : 0, slabRows, outBmuHost ? outBmuHost + r0 : nullptr,
-                               outDistHost ? outDistHost + r0 : nullptr, &fb, top, outBmu2Host ? outBmu2Host + r0 : nullptr, outDist2Host ? outDist2Host + r0 : nullptr);
-        },
-        done, total);
+    const char *slabEnv = getenv("VSOM_EXACT_HOST_SLAB_LOG2");
+    const size_t slab = std::min(n, static_cast<size_t>(1) << (slabEnv ? atoi(slabEnv) : 20));
+    int rc = stage_reserve(ctx, 0, sizeof(float) * slab * ctx->Din);
     if (rc)
         return rc;
-    // tier 3: rows [done, n) are left to the caller's exact path
-    if (rowsDoneOut)
-        *rowsDoneOut = done;
-    if (fallbackRowsOut)
-        *fallbackRowsOut = total;
+    rc = stage_reserve(ctx, 1, sizeof(unsigned) * slab);
+    if (rc)
+        return rc;
+    rc = stage_reserve(ctx, 2, sizeof(float) * slab);
+    if (rc)
+        return rc;
+    float *xDev = static_cast<float *>(ctx->stage[0]);
+    ScoreOut dev;
+    dev.bmu = static_cast<unsigned *>(ctx->stage[1]);
+    dev.dist = static_cast<float *>(ctx->stage[2]);
+    dev.top = out.top;
+    if (out.top == 2)
+    {
+        rc = stage_reserve(ctx, 4, (sizeof(unsigned) + sizeof(float)) * slab);
+        if (rc)
+            return rc;
+        dev.bmu2 = static_cast<unsigned *>(ctx->stage[4]);
+        dev.dist2 = reinterpret_cast<float *>(dev.bmu2 + slab);
+    }
+    for (size_t r0 = 0; r0 < n; r0 += slab)
+    {
+        const size_t rows = std::min(slab, n - r0);
+        VSOM_CUDA(ctx, cudaMemcpyAsync(xDev, xHost + r0 * ctx->Din, sizeof(float) * rows * ctx->Din, cudaMemcpyHostToDevice, ctx->stream));
+        rc = launch_find_bmu_list(ctx, xDev, rows, nullptr, nullptr, minHits, dev, ctx->stream, nullptr);
+        if (rc)
+            return rc;
+        rc = slab_to_host(ctx, xDev, rows, dev, out.at(r0), ctx->stream);
+        if (rc)
+            return rc;
+        VSOM_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); // the staging buffers are reused by the next slab
+    }
+    return VSOM_OK;
+}
+
+// Batches of at least kTcMinRows rows on a shape K2 covers take the tensor-core candidate search + exact rescore (same results,
+// bit for bit); everything else the exact scan.  K2 covers the Standard / Median Comparer (the contraction form of |m - x|^2) up to
+// Dm = 2048; rows longer than TC_MAXK stream their A k-blocks.
+static const size_t kTcMinRows = 1024;
+
+int score_rows(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, uint64_t minHits, bool allowTc, const ScoreOut &out, uint64_t *fallbackRows)
+{
+    if (fallbackRows)
+        *fallbackRows = 0;
+    if (hostRows && n == 0)
+        return VSOM_OK; // nothing ran: vsom_debug_last_score_tc keeps reporting the previous call
+    int tier = 0;
+    size_t done = 0;
+    unsigned long long fallback = 0;
+    if (allowTc && ctx->transform != VSOM_CLR && ctx->Dm <= 2048 && n >= kTcMinRows)
+    {
+        // test knobs; smaller device slabs measured slower (per-slab ramp and tail of the persistent kernel)
+        const char *slabEnv = getenv(hostRows ? "VSOM_TC_HOST_SLAB_LOG2" : "VSOM_TC_SLAB_LOG2");
+        const size_t slab1 = static_cast<size_t>(1) << (slabEnv ? atoi(slabEnv) : hostRows ? 19 : 22);
+        const size_t slab2 = hostRows ? slab1 : std::min<size_t>(slab1, static_cast<size_t>(1) << 20);
+        const int rc = tc_score_tiers(
+            n,
+            [&](size_t r0, size_t rows, int t, unsigned long long &fb) {
+                const int split = t == 2 ? 1 : 0;
+                const size_t slab = t == 2 ? slab2 : slab1;
+                return hostRows ? tc_run_host(ctx, x + r0 * ctx->Din, rows, minHits, split, slab, out.at(r0), fb)
+                                : tc_run_device(ctx, x + r0 * ctx->Din, rows, minHits, split, slab, out.at(r0), fb);
+            },
+            tier, done, fallback);
+        if (rc)
+            return rc;
+    }
+    ctx->lastScoreTier = tier;
+    if (done < n) // every row, or the rows the probes sent to the exact scan (tier 3)
+    {
+        const float *xr = x + done * ctx->Din;
+        const int rc = hostRows ? score_exact_host(ctx, xr, n - done, minHits, out.at(done))
+                                : launch_find_bmu_list(ctx, xr, n - done, nullptr, nullptr, minHits, out.at(done), ctx->stream, nullptr);
+        if (rc)
+            return rc;
+        fallback += n - done;
+    }
+    if (fallbackRows)
+        *fallbackRows = fallback;
     return VSOM_OK;
 }
 
