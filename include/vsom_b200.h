@@ -132,9 +132,11 @@ VSOM_API int vsom_planes_resident(const vsom_ctx *ctx);
  * five phases of each sample (wait-for-sample, scan + CTA min, grid-wide min-loc exchange, broadcast barrier,
  * window update); vsom_debug_phase_cycles returns their mean over CTAs in cycles per sample for the last chunk. */
 VSOM_API int vsom_debug_profile(vsom_ctx *ctx, int enable);
-/* Which kernel the last vsom_train_chunk[_device] call ran: 1 = K1F (online_step_fast.cu: Standard / Median, reference
- * order, planes resident in shared memory, sigma > 1, one GPU), 0 = the generic online-step kernel.  The environment
- * variable VSOM_ONLINE_KERNEL=generic, read by vsom_create, keeps a context on the generic kernel (A/B measurements). */
+/* Which kernel the last vsom_train_chunk[_device] call ran: 1 = K1F (online_step_fast.cu), 0 = the generic online-step
+ * kernel.  K1F runs chunks of fewer than 2^32 - 1 samples on one GPU in the reference and Eigen orders, for every
+ * transformation and both sigma regimes, when the map fits on chip (grid sides <= 4096, at most 512 nodes per CTA, planes
+ * in shared memory).  The environment variable VSOM_ONLINE_KERNEL=generic, read by vsom_create, keeps a context on the
+ * generic kernel (A/B measurements). */
 VSOM_API int vsom_debug_last_train_fast(const vsom_ctx *ctx);
 VSOM_API int vsom_debug_phase_cycles(vsom_ctx *ctx, double out[5]);
 /* The unfolded slots of the last launch.  K1F: chain, CTA min, exchange, coefficients, barrier, update, barrier, 0;

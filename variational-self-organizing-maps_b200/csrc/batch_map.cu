@@ -16,7 +16,6 @@
 #include "common.cuh"
 
 #include <algorithm>
-#include <cmath>
 
 namespace vsom
 {
@@ -424,17 +423,7 @@ int launch_batch_epoch(vsom_ctx *ctx, const float *xDev, size_t n, double sigma,
     std::vector<float> lutHost(static_cast<size_t>(lw) * lh);
     for (int dy = 0; dy < lh; ++dy)
         for (int dx = 0; dx < lw; ++dx)
-        {
-            double nw;
-            if (sigma > 1.0)
-            {
-                const double ddx = dx, ddy = dy;
-                nw = std::exp(-(ddx * ddx / 2.0 / sigma / sigma + ddy * ddy / 2.0 / sigma / sigma));
-            }
-            else
-                nw = (dx == 0 && dy == 0) ? 1.0 : 0.0;
-            lutHost[static_cast<size_t>(dy) * lw + dx] = static_cast<float>(nw);
-        }
+            lutHost[static_cast<size_t>(dy) * lw + dx] = static_cast<float>(neighbourhood_weight(dx, dy, sigma));
     rc = stage_reserve(ctx, 6, sizeof(float) * lutHost.size() + 256);
     if (rc)
         return rc;

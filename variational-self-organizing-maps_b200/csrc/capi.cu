@@ -117,7 +117,6 @@ static int create_impl(vsom_ctx **out, int device, int width, int height, int d_
             if ((y / block) % world == rank)
                 ctx->localRowY.push_back(y);
         ctx->localRows = static_cast<int>(ctx->localRowY.size());
-        ctx->node0 = 0;
         ctx->localN = ctx->localRows * width;
     }
 
@@ -143,11 +142,6 @@ static int create_impl(vsom_ctx **out, int device, int width, int height, int d_
         return fail(VSOM_ERR_NO_DEVICE);
     }
     ctx->numSMs = prop.multiProcessorCount;
-    {
-        // diagnostics / A-B measurements: VSOM_ONLINE_KERNEL=generic keeps every online step on the generic kernel
-        const char *e = getenv("VSOM_ONLINE_KERNEL");
-        ctx->fastDisabled = (e && std::string(e) == "generic") ? 1 : 0;
-    }
     ctx->smemOptin = static_cast<int>(prop.sharedMemPerBlockOptin);
     CREATE_CUDA(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
     const size_t plane = sizeof(float) * static_cast<size_t>(ctx->localN) * ctx->rowStride;
@@ -369,9 +363,9 @@ int vsom_depth(const vsom_ctx *ctx) { return ctx ? ctx->Dm : 0; }
 int vsom_node_count(const vsom_ctx *ctx) { return ctx ? ctx->N : 0; }
 void *vsom_stream(const vsom_ctx *ctx) { return ctx ? static_cast<void *>(ctx->stream) : nullptr; }
 uint64_t vsom_launch_count(const vsom_ctx *ctx) { return ctx ? ctx->launches : 0; }
-int vsom_planes_resident(const vsom_ctx *ctx) { return ctx ? ctx->residentTrain : 0; }
+int vsom_planes_resident(const vsom_ctx *ctx) { return ctx ? ctx->k1.resident : 0; }
 
-int vsom_debug_last_train_fast(const vsom_ctx *ctx) { return ctx ? ctx->lastTrainFast : 0; }
+int vsom_debug_last_train_fast(const vsom_ctx *ctx) { return ctx && ctx->lastPlan == &ctx->k1f ? 1 : 0; }
 
 int vsom_debug_profile(vsom_ctx *ctx, int enable)
 {
@@ -392,14 +386,14 @@ int vsom_debug_profile(vsom_ctx *ctx, int enable)
     return VSOM_OK;
 }
 
-// raw per-phase cycle sums of the last online-step launch, averaged over CTAs, per sample: the generic kernel fills
-// 5 slots (stride 5), K1F 7 (stride 8)
+// raw per-phase cycle sums of the last online-step launch, averaged over CTAs, per sample, in the slots of its plan
 static int read_phase_cycles(vsom_ctx *ctx, double raw[8])
 {
-    if (!ctx->profDev || !ctx->profSamples || !ctx->gridTrain)
+    const StepPlan *plan = ctx->lastPlan;
+    if (!ctx->profDev || !plan)
         return set_error(ctx, VSOM_ERR_INVALID, "vsom_debug_phase_cycles: profiling not enabled or no chunk trained yet");
     VSOM_CUDA(ctx, cudaSetDevice(ctx->device));
-    const int stride = ctx->lastTrainFast ? 8 : 5, grid = ctx->lastTrainFast ? ctx->fastGrid : ctx->gridTrain;
+    const int stride = plan->profStride, grid = plan->grid;
     std::vector<long long> h(static_cast<size_t>(stride) * grid);
     VSOM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     VSOM_CUDA(ctx, cudaMemcpy(h.data(), ctx->profDev, sizeof(long long) * h.size(), cudaMemcpyDeviceToHost));
@@ -421,18 +415,13 @@ int vsom_debug_phase_cycles(vsom_ctx *ctx, double out[5])
     int rc = read_phase_cycles(ctx, raw);
     if (rc)
         return rc;
-    if (ctx->lastTrainFast)
+    for (int i = 0; i < 5; ++i)
     {
-        // K1F has no wait-for-sample phase; fold its seven slots into the five documented ones
-        out[0] = 0.0;
-        out[1] = raw[0] + raw[1]; // FADD chain + CTA min
-        out[2] = raw[2];          // grid-wide exchange
-        out[3] = raw[3] + raw[4]; // coefficients + barrier
-        out[4] = raw[5] + raw[6]; // update (+ next sample's squared residuals) + barrier
+        out[i] = 0.0;
+        for (int j = 0; j < 8; ++j)
+            if (ctx->lastPlan->profFold[i] >> j & 1)
+                out[i] += raw[j];
     }
-    else
-        for (int i = 0; i < 5; ++i)
-            out[i] = raw[i];
     return VSOM_OK;
 }
 

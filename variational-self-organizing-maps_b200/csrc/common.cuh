@@ -6,9 +6,11 @@
 // contracts or reassociates; the library is additionally compiled with -fmad=false.
 #pragma once
 
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <cmath>
 #include <string>
 #include <vector>
 
@@ -28,6 +30,18 @@ struct LutEntry
     float cexp; // (float)(nw * eta)  — Exponential decay: added to weightMap and multiplies the step
     float nwf;  // (float)nw          — multiplies the Welford term; added to weightMap in InverseProportional
 };
+
+// Som::calculateNeighbourhoodWeight (src/Som.cpp:949-975) of a node (dx, dy) cells from the BMU, with the division order of
+// :962-963 and the host libm exp() the reference calls (the host code is compiled with -ffp-contract=off)
+inline double neighbourhood_weight(int dx, int dy, double sigma)
+{
+    if (sigma > 1.0)
+    {
+        const double ddx = static_cast<double>(dx), ddy = static_cast<double>(dy);
+        return std::exp(-(ddx * ddx / 2.0 / sigma / sigma + ddy * ddy / 2.0 / sigma / sigma));
+    }
+    return (dx == 0 && dy == 0) ? 1.0 : 0.0;
+}
 
 struct StepParams
 {
@@ -77,6 +91,22 @@ struct StepParams
     const void *scanMap;      // ... its TMA descriptor of the mean plane (device memory)
 };
 
+// How one online-step kernel is launched on a context: K1 (online_step.cu) is always configured, K1F (online_step_fast.cu)
+// only where it is eligible.  Both are fixed at vsom_create; launch_online_step picks one per chunk.
+struct StepPlan
+{
+    void (*kernel[2])(const StepParams) = {}; // [profiling]: K1F has a profiled instantiation, K1 tests p.prof at run time
+    int grid = 0;                             // CTAs; 0: the kernel is not configured on this context
+    int threads = 0;
+    size_t smem = 0;                          // dynamic shared memory without the neighbourhood table
+    size_t smemCap = 0;                       // dynamic shared memory the kernel may use: the table rides behind smem if it fits
+    int resident = 0;                         // StepParams::resident, smStride, lanesPerNode
+    int smStride = 0;
+    int lanesPerNode = 0;
+    int profStride = 0;                       // profiling slots per CTA (StepParams::prof)
+    unsigned char profFold[5] = {};           // vsom_debug_phase_cycles: phase i is the sum of the slots in bit mask profFold[i]
+};
+
 } // namespace vsom
 
 struct vsom_ctx
@@ -84,7 +114,7 @@ struct vsom_ctx
     int device = 0;
     int W = 0, H = 0, N = 0, Din = 0, Dm = 0, Dr = 0, P = 0;
     int rank = 0, world = 1;      // node sharding: grid rows are dealt to the ranks round-robin in blocks of shardBlock rows
-    int node0 = 0, localN = 0;    // node0 stays 0; localN = localRows * W
+    int localN = 0;               // localRows * W
     int shardBlock = 0, localRows = 0;
     std::vector<int> localRowY;   // global grid row of every local row
     float *peerMean[8] = {};      // mean planes of the ranks (U-matrix halo rows), peer-mapped; peerMean[rank] == mean
@@ -124,17 +154,12 @@ struct vsom_ctx
     unsigned long long tcStats[3] = {0, 0, 0}; // K2 fallback causes since creation: list overflow, NaN / nothing eligible, certificate
     int lastScoreTier = 0;                   // path of the last scoring call (score_rows): 0 the exact scan, else K2's tier (1: one half
                                              // per operand, 2: hi / lo pairs, 3: the probes sent the rest to the exact scan)
-    int gridTrain = 0, residentTrain = 0, smStrideTrain = 0;
-    size_t smemTrain = 0;
     uint64_t launches = 0;
-    // K1F (online_step_fast.cu): eligibility and launch geometry, window table of the current sigma
-    int fastTrain = 0, fastGrid = 0, fastStride = 0, fastDisabled = 0;
-    size_t fastSmem = 0;
+    vsom::StepPlan k1, k1f;                  // online step: the generic kernel, and K1F (k1f.grid == 0: not eligible)
+    const vsom::StepPlan *lastPlan = nullptr; // the plan of the last online-step launch
+    // K1F (online_step_fast.cu): window table of the current sigma
     unsigned *winTab = nullptr;
     double winSigma = -1;
-    int lastTrainFast = 0;        // the last online-step launch ran K1F
-    int fastLanes = 1;            // K1F: lanes per node in the scan
-    int fastReg = 0;              // K1F: items per warp whose rows live in registers (0: rows in shared memory)
     vsom::u64 *rowPool = nullptr; // K1F exchange rows: 1024 blocks of 2 KB
     int *rowMeta = nullptr;       // dieOfSm[256] | rowBlocks[640] | rowOf[160] | counters[4]
     int dieAware = 0;             // the row pool was classified by L2 die
@@ -201,8 +226,12 @@ struct ScoreOut
 int launch_online_step(vsom_ctx *ctx, const float *xDev, size_t n, double eta, double sigma, int decay, unsigned *outBmuDev, float *outDistDev,
                        const u64 *lastInDev = nullptr);
 int configure_online_step(vsom_ctx *ctx);
-int configure_online_step_fast(vsom_ctx *ctx);                               // 1: K1F eligible for this context
-int launch_online_step_fast(vsom_ctx *ctx, StepParams &p, double sigma);      // 1: enqueued, 0: not eligible, < 0: error
+void configure_online_step_fast(vsom_ctx *ctx);
+int prepare_online_step_fast(vsom_ctx *ctx, StepParams &p, double sigma); // K1F's per-chunk buffers and StepParams fields
+// cuTensorMapEncodeTiled of the driver, null when the driver does not have it
+typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *, const cuuint32_t *,
+                                  const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+EncodeTiledFn tensor_map_encoder();
 // Every scoring call: x holds n rows (host memory when hostRows), results go to `out`.  Chooses K2 or the exact scan, runs K2's
 // tiers and the exact scan of the rows K2 leaves, and records the path for vsom_debug_last_score_tc (score_tc.cu).
 int score_rows(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, uint64_t minHits, bool allowTc, const ScoreOut &out, uint64_t *fallbackRows);

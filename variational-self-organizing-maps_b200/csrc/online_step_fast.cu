@@ -3,9 +3,8 @@
 //
 // Same contract and the same bits as online_step.cu's generic kernel (Som::trainSingle src/Som.cpp:885-947 =
 // findBmu :291-309 / findLocalBmu :335-454 over euclidianWeightedDist :124-141, window update :899-944,
-// calculateNeighbourhoodWeight :949-975, addBmu :1189-1192), for: all three transformations, reference summation order,
-// planes that fit on chip, one GPU, grid sides <= 4096, at most 512 owned nodes per CTA.  Everything else (LANES order,
-// HBM-resident maps, node-sharded contexts) runs the generic kernel.
+// calculateNeighbourhoodWeight :949-975, addBmu :1189-1192), for maps whose planes fit on chip, on one GPU.  Which chunks
+// it runs is decided in one place, launch_online_step (online_step.cu).
 //
 // Why a second kernel: the generic one measures (profiles/r01_bench_default_final_candidate.json, cycles per sample
 // at 64x64x128) wait 593 + scan 1535 + exchange 3323 + broadcast 248 + update 1643.  The strict per-sample dependency
@@ -1298,7 +1297,7 @@ static int build_row_pool(vsom_ctx *ctx)
         // pairs of die-0 SMs, by SM id
         std::vector<int> pairOf(256, -1), roleOf(256, 0), die0;
         for (int s = 0; s < 256; ++s)
-            if (dm.dieOfSm[s] == 0 && s < 256)
+            if (dm.dieOfSm[s] == 0)
                 die0.push_back(s);
         // dieOfSm defaults to 0 for ids that were never seen; keep only SM ids below the SM count
         die0.erase(std::remove_if(die0.begin(), die0.end(), [&](int s) { return s >= ctx->numSMs; }), die0.end());
@@ -1355,7 +1354,6 @@ static int build_row_pool(vsom_ctx *ctx)
     }
     // rowBlocks[(die * kFMaxCtas + slot) * 2 + buffer] = block index; every (die, slot, buffer) gets its own block
     std::vector<int> rowBlocks(2 * 2 * kFMaxCtas, 0), dieOfSm(256, 0);
-    int next = 0;
     std::vector<int> byDie[2];
     for (int k = 0; k < kFPoolBlocks; ++k)
         byDie[haveHomes ? home[k] : (k & 1)].push_back(k);
@@ -1373,7 +1371,6 @@ static int build_row_pool(vsom_ctx *ctx)
             byDie[k & 1].push_back(k);
         std::fill(dieOfSm.begin(), dieOfSm.end(), 0);
     }
-    (void)next;
     for (int d = 0; d < 2; ++d)
         for (int slot = 0; slot < kFMaxCtas; ++slot)
             for (int buf = 0; buf < 2; ++buf)
@@ -1390,27 +1387,25 @@ static int build_row_pool(vsom_ctx *ctx)
     return VSOM_OK;
 }
 
-// 0: not eligible (the caller runs the generic kernel), 1: configured
-int configure_online_step_fast(vsom_ctx *ctx)
+// K1F's plan, left unset where K1F cannot run the context (launch_online_step states the rule)
+void configure_online_step_fast(vsom_ctx *ctx)
 {
-    ctx->fastTrain = 0;
-    if (ctx->order == VSOM_ORDER_LANES || ctx->world > 1 || ctx->W > 4096 || ctx->H > 4096)
-        return 0;
+    const char *env = getenv("VSOM_ONLINE_KERNEL"); // "generic": every chunk on K1 (A/B measurements)
+    if ((env && std::string(env) == "generic") || ctx->order == VSOM_ORDER_LANES || ctx->world > 1 || ctx->W > 4096 || ctx->H > 4096)
+        return;
     if (ctx->transform == VSOM_CLR && ((ctx->Din + 3) & ~3) + 4 > 65535)
-        return 0; // pair tables are 16-bit
+        return; // pair tables are 16-bit
     int G = ctx->localN < ctx->numSMs ? ctx->localN : ctx->numSMs;
     if (G > kFMaxCtas)
         G = kFMaxCtas;
     const int stride = fast_stride(ctx);
     const size_t bytes = fast_smem(ctx, G, stride);
     if (bytes + kFStaticSmem > static_cast<size_t>(ctx->smemOptin))
-        return 0;
+        return;
     const int Lmax = (ctx->localN + G - 1) / G;
     if (Lmax > kFThreads)
-        return 0; // one scan lane per owned node
-    // Eigen order: eight lanes per node cut the chain from Dr to Dr / 8 dependent adds; worth it when the rows are long or when
-    // all the CTA's nodes still fit one warp (no extra CTA-level reduction).
-    ctx->fastLanes = ctx->order == VSOM_ORDER_EIGEN_SSE && Lmax * 8 <= kFThreads && (Lmax * 8 <= 32 || ctx->Dr >= 256) ? 8 : 1;
+        return; // one scan lane per owned node
+    StepPlan pl;
     const int ipw = fast_ipw(ctx, G);
     for (int prof = 0; prof < 2; ++prof)
     {
@@ -1418,21 +1413,31 @@ int configure_online_step_fast(vsom_ctx *ctx)
         if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, ctx->smemOptin - static_cast<int>(kFStaticSmem)) != cudaSuccess)
         {
             cudaGetLastError();
-            return 0;
+            return;
         }
         int perSm = 0;
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, k, kFThreads, bytes) != cudaSuccess || perSm < 1)
         {
             cudaGetLastError();
-            return 0;
+            return;
         }
+        pl.kernel[prof] = k;
     }
-    ctx->fastTrain = 1;
-    ctx->fastGrid = G;
-    ctx->fastStride = stride;
-    ctx->fastSmem = bytes;
-    ctx->fastReg = ipw;
-    return 1;
+    pl.grid = G;
+    pl.threads = kFThreads;
+    pl.smem = bytes;
+    pl.smemCap = static_cast<size_t>(ctx->smemOptin) - kFStaticSmem;
+    pl.resident = 1;
+    pl.smStride = stride;
+    // Eigen order: eight lanes per node cut the chain from Dr to Dr / 8 dependent adds; worth it when the rows are long or when
+    // all the CTA's nodes still fit one warp (no extra CTA-level reduction).
+    pl.lanesPerNode = ctx->order == VSOM_ORDER_EIGEN_SSE && Lmax * 8 <= kFThreads && (Lmax * 8 <= 32 || ctx->Dr >= 256) ? 8 : 1;
+    // slots: chain, CTA min, exchange, coefficients, barrier, update (+ the next sample's squared residuals), barrier.  No
+    // wait-for-sample phase; the other four phases of the profile are sums of these.
+    pl.profStride = 8;
+    const unsigned char fold[5] = {0, 0x03, 0x04, 0x18, 0x60};
+    std::copy(fold, fold + 5, pl.profFold);
+    ctx->k1f = pl;
 }
 
 // [start,end) of the update window per BMU column and row: the f64 expressions of src/Som.cpp:899-903
@@ -1458,12 +1463,10 @@ static int build_window_table(vsom_ctx *ctx, double sigma)
     return VSOM_OK;
 }
 
-// Called by launch_online_step after the neighbourhood table is in place.  Returns 1 when the chunk was enqueued,
-// 0 when this launch is not eligible (sigma <= 1, ...), < 0 on error.
-int launch_online_step_fast(vsom_ctx *ctx, StepParams &p, double sigma)
+// K1F's per-chunk state: the local walk's tagged distances, the exchange rows (the first chunk measures the L2 dies) and the
+// update window table
+int prepare_online_step_fast(vsom_ctx *ctx, StepParams &p, double sigma)
 {
-    if (!ctx->fastTrain || p.world > 1 || p.n >= (1ull << 32) - 1)
-        return 0;
     if (p.localSearch)
     {
         const size_t bytes = sizeof(u64) * 2 * kWalkReplicas * static_cast<size_t>(ctx->N);
@@ -1478,27 +1481,16 @@ int launch_online_step_fast(vsom_ctx *ctx, StepParams &p, double sigma)
     rc = build_window_table(ctx, sigma);
     if (rc)
         return rc;
-    const int G = ctx->fastGrid;
     VSOM_CUDA(ctx, cudaMemsetAsync(ctx->rowPool, 0xff, static_cast<size_t>(kFPoolBlocks) * 2048, ctx->stream));
     unsigned *ctr = reinterpret_cast<unsigned *>(ctx->rowMeta + 256 + 2 * 2 * kFMaxCtas + kFMaxCtas);
     VSOM_CUDA(ctx, cudaMemsetAsync(ctr, 0, sizeof(unsigned) * 4, ctx->stream));
-    VSOM_CUDA(ctx, cudaMemsetAsync(ctx->errFlag, 0, sizeof(int), ctx->stream));
     p.winTab = ctx->winTab;
     p.dieOfSm = ctx->rowMeta;
     p.rowBlocks = ctx->rowMeta + 256;
     p.rowOf = ctx->rowMeta + 256 + 2 * 2 * kFMaxCtas;
     p.rowCtr = ctr;
     p.rowPool = ctx->rowPool;
-    p.resident = 1;
-    p.lanesPerNode = ctx->fastLanes;
-    p.smStride = ctx->fastStride;
-    const size_t lutBytes = sizeof(LutEntry) * static_cast<size_t>(p.lutCount);
-    p.lutSmem = (ctx->fastSmem + lutBytes + kFStaticSmem <= static_cast<size_t>(ctx->smemOptin)) ? 1 : 0;
-    const size_t smemBytes = ctx->fastSmem + (p.lutSmem ? lutBytes : 0);
-    FastKernel k = pick_fast(ctx->transform, ctx->fastReg, p.prof != nullptr);
-    void *args[] = {&p};
-    VSOM_CUDA(ctx, cudaLaunchCooperativeKernel(reinterpret_cast<void *>(k), dim3(G), dim3(kFThreads), args, smemBytes, ctx->stream));
-    return 1;
+    return VSOM_OK;
 }
 
 } // namespace vsom

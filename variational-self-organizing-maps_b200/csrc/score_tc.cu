@@ -1018,10 +1018,7 @@ __global__ void __launch_bounds__(256) find_bmu_rowwise_kernel(const float *__re
 
 // ------------------------------------------------------------------------------------------------ host side
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *, const cuuint32_t *,
-                                  const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn encode_fn()
+EncodeTiledFn tensor_map_encoder()
 {
     static EncodeTiledFn fn = nullptr;
     if (!fn)
@@ -1036,7 +1033,7 @@ static EncodeTiledFn encode_fn()
 
 static int make_map(vsom_ctx *ctx, CUtensorMap *map, void *base, unsigned long long rows, int Kpad, int boxRows)
 {
-    EncodeTiledFn enc = encode_fn();
+    EncodeTiledFn enc = tensor_map_encoder();
     if (!enc)
         return set_error(ctx, VSOM_ERR_CUDA, "score_tc: cuTensorMapEncodeTiled entry point not available");
     const cuuint64_t dims[2] = {static_cast<cuuint64_t>(Kpad), static_cast<cuuint64_t>(rows)};
