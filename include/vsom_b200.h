@@ -69,6 +69,8 @@ typedef enum vsom_decay_kind
  *              (16,8,4,2,1).  Deterministic; BMUs can differ from the reference only at near-ties (relative
  *              distance gap below 2*Dm*2^-24, see DESIGN.md).  It runs on the generic online-step kernel; since
  *              K1F (online_step_fast.cu) the REFERENCE order is the faster of the two for maps that fit on chip.
+ *              Only the online step sums in the lanes order: every other path of such a context (scoring, all_dists,
+ *              soft assignment, U-matrix, the batch-map trainer) sums in the REFERENCE order and returns its bits.
  *   EIGEN_SSE: the order `dot()` / `squaredNorm()` have when the reference is built against real Eigen (3.3 / 3.4) with
  *              its release flags (-msse2, README.md:64-69, build/Makefile:18): Eigen's vectorised redux over Packet4f —
  *              two 4-wide accumulators over strides of 8 elements (eight interleaved sequential chains), res0 + res1,

@@ -604,11 +604,13 @@ def test_exact_scan_every_residue_of_the_vector_length(vsom, po, tr, Din, order)
 
 
 @pytest.mark.parametrize("order", [0, 2], ids=["seq", "eigen_sse"])
-@pytest.mark.parametrize("Dm", [5, 8, 12, 31, 64, 100])
+@pytest.mark.parametrize("Dm", [1, 5, 7, 8, 9, 12, 31, 32, 33, 63, 64, 65, 72, 100, 127, 129])
 def test_umatrix_division_corner_cases(vsom, po, Dm, order):
     """K4 replaces the reference's IEEE division by a shared reciprocal + one correction step; every term must still be
     the reference's bits.  Sigmas: zero (clamped to 1e-5), tiny, ordinary, huge, 2^100 and beyond, infinite; differences:
-    exact zeros, denormals, tiny, ordinary, huge (the quotient or its square overflows), infinite."""
+    exact zeros, denormals, tiny, ordinary, huge (the quotient or its square overflows), infinite.
+    Model lengths around the kernels' slices (32 elements in the sequential kernel, 64 in the Eigen one), the block of
+    eight and the padded rows (Dm % 4 != 0); at Dm = 65 the Eigen kernel's last slice holds only the rest block."""
     rng = np.random.default_rng(Dm)
     W, H = 19, 6
     N = W * H

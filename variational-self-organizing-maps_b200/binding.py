@@ -181,6 +181,13 @@ class VsomContext:
         self._check(lib().vsom_download_state(self._h, _p(mean, _f32p), _p(S, _f32p), _p(sigma, _f32p), _p(weight, _f32p), _p(hits, _u64p)))
         return dict(mean=mean, S=S, sigma=sigma, weight=weight, hits=hits)
 
+    def get_node(self, node):
+        """Som::getNeuron / Som::getSigmaNeuron: (mean, sigma) rows of one node, Dm floats each."""
+        mean = np.empty(self.Dm, np.float32)
+        sigma = np.empty(self.Dm, np.float32)
+        self._check(lib().vsom_get_node(self._h, node, _p(mean, _f32p), _p(sigma, _f32p)))
+        return mean, sigma
+
     # ---- online training
     def train_chunk(self, x, eta, sigma, decay=EXPONENTIAL, last_bmu=None):
         x = _f32(x).reshape(-1, self.Din)

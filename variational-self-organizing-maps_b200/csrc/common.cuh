@@ -21,6 +21,9 @@ namespace vsom
 
 typedef unsigned long long u64;
 
+// CUDA's limit on gridDim.y (and z): launchers that put rows or tiles on y launch longer ranges in pieces of this size
+constexpr size_t kMaxGridY = 65535;
+
 // One neighbourhood-table entry per (|dy|, |dx|): Som::calculateNeighbourhoodWeight (src/Som.cpp:949-975)
 // evaluated on the host with the same libm exp() the reference calls, then pre-rounded the way
 // Som::trainSingle uses it (src/Som.cpp:922-941).

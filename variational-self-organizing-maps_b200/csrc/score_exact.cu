@@ -530,16 +530,24 @@ int launch_soft_assign(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minH
 {
     if (n == 0)
         return VSOM_OK;
-    dim3 grid((ctx->N + 127) / 128, static_cast<unsigned>(n));
-    if (ctx->transform == VSOM_CLR)
-        soft_assign_terms_kernel<VSOM_CLR><<<grid, 128, 0, ctx->stream>>>(xDev, n, ctx->mean, ctx->hits, minHits, ctx->N, ctx->Din, ctx->Dr, ctx->P, ctx->rowStride, ctx->pairI,
-                                                                          ctx->pairJ, ctx->order, probDev);
-    else
-        soft_assign_terms_kernel<VSOM_STANDARD><<<grid, 128, 0, ctx->stream>>>(xDev, n, ctx->mean, ctx->hits, minHits, ctx->N, ctx->Din, ctx->Dr, ctx->P, ctx->rowStride,
-                                                                               ctx->pairI, ctx->pairJ, ctx->order, probDev);
+    // one grid row per data row: gridDim.y is at most 65 535, so longer batches take several launches
+    for (size_t r0 = 0; r0 < n; r0 += kMaxGridY)
+    {
+        const size_t rows = std::min(n - r0, kMaxGridY);
+        const float *xs = xDev + r0 * ctx->Din;
+        double *out = probDev + r0 * ctx->N;
+        dim3 grid((ctx->N + 127) / 128, static_cast<unsigned>(rows));
+        if (ctx->transform == VSOM_CLR)
+            soft_assign_terms_kernel<VSOM_CLR><<<grid, 128, 0, ctx->stream>>>(xs, rows, ctx->mean, ctx->hits, minHits, ctx->N, ctx->Din, ctx->Dr, ctx->P, ctx->rowStride, ctx->pairI,
+                                                                              ctx->pairJ, ctx->order, out);
+        else
+            soft_assign_terms_kernel<VSOM_STANDARD><<<grid, 128, 0, ctx->stream>>>(xs, rows, ctx->mean, ctx->hits, minHits, ctx->N, ctx->Din, ctx->Dr, ctx->P, ctx->rowStride,
+                                                                                   ctx->pairI, ctx->pairJ, ctx->order, out);
+        ctx->launches += 1;
+    }
     soft_assign_norm_kernel<<<static_cast<unsigned>(n), 256, 0, ctx->stream>>>(n, ctx->N, probDev, sumsDev);
     VSOM_CUDA(ctx, cudaGetLastError());
-    ctx->launches += 2;
+    ctx->launches += 1;
     return VSOM_OK;
 }
 
