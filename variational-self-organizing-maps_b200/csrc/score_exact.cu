@@ -146,69 +146,38 @@ __global__ void __launch_bounds__(kScoreThreads) find_bmu_exact_kernel(const flo
         for (int j = 0; j < 4; ++j)
         {
             const int node = node0 + tx + 16 * j;
-            if (node < N && (node == 0 || minHits == 0 || hits[node] >= minHits))
+            if (node < N && restricted_eligible(node, hits, minHits))
             {
 #pragma unroll
                 for (int i = 0; i < 4; ++i)
                 {
                     const float d = acc[i][j];
                     if (TOP == 2)
-                        key_top2_insert(best[i], second[i], make_key(d, static_cast<unsigned>(node), (d != d) ? 1u : 0u));
+                        key_top2_insert(best[i], second[i], score_key(d, static_cast<unsigned>(node)));
                     else
-                        best[i] = u64_min(best[i], make_key(d, static_cast<unsigned>(node), (d != d) ? 1u : 0u));
+                        best[i] = u64_min(best[i], score_key(d, static_cast<unsigned>(node)));
                 }
             }
         }
     }
     // the 16 threads sharing a row sit in one half-warp: xor offsets 8,4,2,1 stay inside it
-    if (TOP == 2)
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-        {
-            u64 k = best[i], k2 = second[i];
-#pragma unroll
-            for (int o = 8; o; o >>= 1)
-                key_top2_merge(k, k2, __shfl_xor_sync(0xffffffffu, k, o), __shfl_xor_sync(0xffffffffu, k2, o));
-            const u64 item = row0 + ty + 16 * i;
-            if (tx == 0 && item < n)
-            {
-                if (listMode)
-                    key_top2_atomic(keyBuf + 2 * item, k, k2);
-                else
-                {
-                    if (outBmu)
-                        outBmu[item] = key_node(k);
-                    if (outDist)
-                        outDist[item] = key_dist(k);
-                    store_second(outBmu2, outDist2, item, k2);
-                }
-            }
-        }
-    else
 #pragma unroll
     for (int i = 0; i < 4; ++i)
     {
-        u64 k = best[i];
+        u64 k = best[i], k2 = TOP == 2 ? second[i] : ~0ull;
 #pragma unroll
         for (int o = 8; o; o >>= 1)
-            k = u64_min(k, __shfl_xor_sync(0xffffffffu, k, o));
+            if (TOP == 2)
+                key_top2_merge(k, k2, __shfl_xor_sync(0xffffffffu, k, o), __shfl_xor_sync(0xffffffffu, k2, o));
+            else
+                k = u64_min(k, __shfl_xor_sync(0xffffffffu, k, o));
         const u64 item = row0 + ty + 16 * i;
         if (tx == 0 && item < n)
         {
             if (listMode)
-                atomicMin(keyBuf + item, k);
+                list_key_store<TOP>(keyBuf + TOP * item, k, k2);
             else
-            {
-                if (outBmu)
-                    outBmu[item] = key_node(k);
-                if (outDist)
-                {
-                    float d = __uint_as_float(static_cast<unsigned>(k >> 32));
-                    if (k & 1ull)
-                        d = __uint_as_float(0x7fc00000u);
-                    outDist[item] = d;
-                }
-            }
+                store_row_outputs<TOP>(outBmu, outDist, outBmu2, outDist2, item, k, k2);
         }
     }
     __syncthreads(); // the staging arrays are reused by the next work item
@@ -359,7 +328,7 @@ __global__ void __launch_bounds__(kScoreThreads) find_bmu_exact_eigen_kernel(con
         for (int j = 0; j < 4; ++j)
         {
             const int node = node0 + gx + 8 * j;
-            const bool eligible = node < N && (node == 0 || minHits == 0 || hits[node] >= minHits);
+            const bool eligible = node < N && restricted_eligible(node, hits, minHits);
 #pragma unroll
             for (int i = 0; i < 8; ++i)
             {
@@ -379,9 +348,9 @@ __global__ void __launch_bounds__(kScoreThreads) find_bmu_exact_eigen_kernel(con
                 if (eligible)
                 {
                     if (TOP == 2)
-                        key_top2_insert(best[i], second[i], make_key(v, static_cast<unsigned>(node), (v != v) ? 1u : 0u));
+                        key_top2_insert(best[i], second[i], score_key(v, static_cast<unsigned>(node)));
                     else
-                        best[i] = u64_min(best[i], make_key(v, static_cast<unsigned>(node), (v != v) ? 1u : 0u));
+                        best[i] = u64_min(best[i], score_key(v, static_cast<unsigned>(node)));
                 }
             }
         }
@@ -395,80 +364,36 @@ __global__ void __launch_bounds__(kScoreThreads) find_bmu_exact_eigen_kernel(con
                 sSecond[gy + 4 * i][gx] = second[i];
         }
     __syncthreads();
-    if (TOP == 2 && tid < ER && row0 + tid < n)
+    if (tid < ER && row0 + tid < n)
     {
-        u64 k = sBest[tid][0], k2 = sSecond[tid][0];
+        u64 k = sBest[tid][0], k2 = TOP == 2 ? sSecond[tid][0] : ~0ull;
 #pragma unroll
         for (int q = 1; q < 8; ++q)
-            key_top2_merge(k, k2, sBest[tid][q], sSecond[tid][q]);
+            if (TOP == 2)
+                key_top2_merge(k, k2, sBest[tid][q], sSecond[tid][q]);
+            else
+                k = u64_min(k, sBest[tid][q]);
         const u64 item = row0 + tid;
         if (listMode)
-            key_top2_atomic(keyBuf + 2 * item, k, k2);
+            list_key_store<TOP>(keyBuf + TOP * item, k, k2);
         else
-        {
-            if (outBmu)
-                outBmu[item] = key_node(k);
-            if (outDist)
-                outDist[item] = key_dist(k);
-            store_second(outBmu2, outDist2, item, k2);
-        }
-    }
-    if (TOP == 1 && tid < ER && row0 + tid < n)
-    {
-        u64 k = sBest[tid][0];
-#pragma unroll
-        for (int q = 1; q < 8; ++q)
-            k = u64_min(k, sBest[tid][q]);
-        const u64 item = row0 + tid;
-        if (listMode)
-            atomicMin(keyBuf + item, k);
-        else
-        {
-            if (outBmu)
-                outBmu[item] = key_node(k);
-            if (outDist)
-            {
-                float d = __uint_as_float(static_cast<unsigned>(k >> 32));
-                if (k & 1ull)
-                    d = __uint_as_float(0x7fc00000u);
-                outDist[item] = d;
-            }
-        }
+            store_row_outputs<TOP>(outBmu, outDist, outBmu2, outDist2, item, k, k2);
     }
     __syncthreads(); // sBest and the staging arrays are reused by the next work item
   }
 }
 
-// list mode: keys of the work items' splits -> outputs of the listed rows
+// list mode: keys of the work items' splits (TOP per listed row, list_key_store) -> outputs of the listed rows
+template <int TOP>
 __global__ void finalize_list_kernel(const unsigned *__restrict__ rowList, const unsigned *__restrict__ rowCount, const u64 *__restrict__ keyBuf,
-                                     unsigned *__restrict__ outBmu, float *__restrict__ outDist)
+                                     unsigned *__restrict__ outBmu, float *__restrict__ outDist, unsigned *__restrict__ outBmu2, float *__restrict__ outDist2)
 {
     const unsigned n = *rowCount;
     for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
     {
-        const u64 k = keyBuf[i];
-        const unsigned row = rowList[i];
-        if (outBmu)
-            outBmu[row] = key_node(k);
-        if (outDist)
-            outDist[row] = (k & 1ull) ? __uint_as_float(0x7fc00000u) : __uint_as_float(static_cast<unsigned>(k >> 32));
-    }
-}
-
-// the same for the top-2 scan: two keys per listed row (key_top2_atomic)
-__global__ void finalize_list2_kernel(const unsigned *__restrict__ rowList, const unsigned *__restrict__ rowCount, const u64 *__restrict__ keyBuf,
-                                      unsigned *__restrict__ outBmu, float *__restrict__ outDist, unsigned *__restrict__ outBmu2, float *__restrict__ outDist2)
-{
-    const unsigned n = *rowCount;
-    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
-    {
-        const u64 k = keyBuf[2 * static_cast<size_t>(i)];
-        const unsigned row = rowList[i];
-        if (outBmu)
-            outBmu[row] = key_node(k);
-        if (outDist)
-            outDist[row] = key_dist(k);
-        store_second(outBmu2, outDist2, row, keyBuf[2 * static_cast<size_t>(i) + 1]);
+        const u64 *k = keyBuf + TOP * static_cast<size_t>(i);
+        const u64 k1 = k[0];
+        store_row_outputs<TOP>(outBmu, outDist, outBmu2, outDist2, rowList[i], k1, TOP == 2 ? k[1] : k1);
     }
 }
 
@@ -497,7 +422,7 @@ __global__ void soft_assign_terms_kernel(const float *__restrict__ x, u64 n, con
     if (node >= N || row >= n)
         return;
     double pr = 0.0;
-    if (hits[node] >= minHits)
+    if (hits[node] >= minHits) // not restricted_eligible: findRestrictedBmd has no node-0 seed
     {
         const double d = static_cast<double>(dist_ordered<TR>(mean + static_cast<size_t>(node) * rowStride, x + row * Din, Dr, P, pairI, pairJ, order));
         pr = exp(__ddiv_rn(__dmul_rn(-d, d), 2.0));
@@ -596,9 +521,9 @@ int launch_find_bmu_list(vsom_ctx *ctx, const float *xDev, size_t n, const unsig
     {
         const unsigned fgrid = std::min(1024u, static_cast<unsigned>((n + 255) / 256));
         if (out.top == 2)
-            finalize_list2_kernel<<<fgrid, 256, 0, stream>>>(rowListDev, rowCountDev, keyBufDev, out.bmu, out.dist, out.bmu2, out.dist2);
+            finalize_list_kernel<2><<<fgrid, 256, 0, stream>>>(rowListDev, rowCountDev, keyBufDev, out.bmu, out.dist, out.bmu2, out.dist2);
         else
-            finalize_list_kernel<<<fgrid, 256, 0, stream>>>(rowListDev, rowCountDev, keyBufDev, out.bmu, out.dist);
+            finalize_list_kernel<1><<<fgrid, 256, 0, stream>>>(rowListDev, rowCountDev, keyBufDev, out.bmu, out.dist, out.bmu2, out.dist2);
         ctx->launches += 1;
     }
     VSOM_CUDA(ctx, cudaGetLastError());

@@ -794,7 +794,7 @@ __global__ void map_operand_kernel(const float *__restrict__ mean, const float *
     if (lane == 0)
     {
         float c = 60000.0f; // pieces of real nodes stay below 2^13
-        if (p < N && (p == 0 || minHits == 0 || hits[p] >= minHits) && norm2[p] == norm2[p])
+        if (p < N && restricted_eligible(p, hits, minHits) && norm2[p] == norm2[p])
             c = fminf(sm * norm2[p] / tau, 60000.0f);
         const __half hi = __float2half_rn(c);
         const float r1 = c - __half2float(hi);
@@ -923,13 +923,13 @@ __global__ void __launch_bounds__(RS_THREADS) rescore_kernel(const float *__rest
         const unsigned node = cand[row * TC_TOPK + j];
         // eligibility is re-checked here: padding nodes and nodes below min_hits may be listed when their large constant does
         // not dominate (rows much larger than the map); they must not win
-        if (node >= static_cast<unsigned>(N) || !(node == 0 || minHits == 0 || hits[node] >= minHits))
+        if (node >= static_cast<unsigned>(N) || !restricted_eligible(node, hits, minHits))
             continue;
         const float s = dist_rows_f32(mean + static_cast<size_t>(node) * rowStride, x + row * D, D, order);
         if (TOP == 2)
-            key_top2_atomic(&sKey2[2 * r], make_key(s, node, (s != s) ? 1u : 0u), ~0ull);
+            key_top2_atomic(&sKey2[2 * r], score_key(s, node), ~0ull);
         else
-            atomicMin(&sKey[r], make_key(s, node, (s != s) ? 1u : 0u));
+            atomicMin(&sKey[r], score_key(s, node));
     }
     __syncthreads();
     if (tid < RS_ROWS && row0 + tid < rows)
@@ -958,63 +958,11 @@ __global__ void __launch_bounds__(RS_THREADS) rescore_kernel(const float *__rest
             atomicAdd(stats + (cnt == TC_OVERFLOW ? 1 : (nan || keyC == ~0ull ? 2 : 3)), 1ull);
         }
         else
-        {
-            if (outBmu)
-                outBmu[row] = key_node(key);
-            if (outDist)
-                outDist[row] = __uint_as_float(static_cast<unsigned>(key >> 32));
-            if (TOP == 2)
-                store_second(outBmu2, outDist2, static_cast<u64>(row), key2);
-        }
+            store_row_outputs<TOP>(outBmu, outDist, outBmu2, outDist2, static_cast<u64>(row), key, key2);
     }
 }
 
 __global__ void add_count_kernel(const unsigned *count, unsigned long long *total) { *total += *count; }
-
-// Exact full scan for a FEW rows (the rows the candidate lists could not certify): one CTA per row, threads over
-// nodes, every (row, node) distance summed sequentially in f32 like the reference.  Same key rule as K3.
-// Exact full scan of the rows a slab's guard could not certify.  The row count lives in device memory (no host round trip
-// between the slabs of a batch): a fixed grid walks the list, and CTA 0 adds the count to the batch total.
-__global__ void __launch_bounds__(256) find_bmu_rowwise_kernel(const float *__restrict__ x, int D, const unsigned *__restrict__ rows,
-                                                               const unsigned *__restrict__ countPtr, const float *__restrict__ mean, int rowStride, int N,
-                                                               const u64 *__restrict__ hits, u64 minHits, int order, unsigned *__restrict__ outBmu,
-                                                               float *__restrict__ outDist, unsigned long long *__restrict__ total)
-{
-    extern __shared__ float xrow[];
-    __shared__ u64 wkey[8];
-    const unsigned count = *countPtr;
-    if (blockIdx.x == 0 && threadIdx.x == 0 && count)
-        atomicAdd(total, static_cast<unsigned long long>(count));
-    for (unsigned i = blockIdx.x; i < count; i += gridDim.x)
-    {
-        const size_t r = rows[i];
-        __syncthreads(); // xrow / wkey of the previous row are no longer read
-        for (int k = threadIdx.x; k < D; k += blockDim.x)
-            xrow[k] = x[r * D + k];
-        __syncthreads();
-        u64 best = ~0ull;
-        for (int node = threadIdx.x; node < N; node += blockDim.x)
-        {
-            if (!(node == 0 || minHits == 0 || hits[node] >= minHits))
-                continue;
-            const float s = dist_rows_f32(mean + static_cast<size_t>(node) * rowStride, xrow, D, order);
-            best = u64_min(best, make_key(s, static_cast<unsigned>(node), (s != s) ? 1u : 0u));
-        }
-        best = warp_min_u64(best);
-        if ((threadIdx.x & 31) == 0)
-            wkey[threadIdx.x >> 5] = best;
-        __syncthreads();
-        if (threadIdx.x == 0)
-        {
-            for (int w = 1; w < 8; ++w)
-                best = u64_min(best, wkey[w]);
-            if (outBmu)
-                outBmu[r] = key_node(best);
-            if (outDist)
-                outDist[r] = (best & 1ull) ? __uint_as_float(0x7fc00000u) : __uint_as_float(static_cast<unsigned>(best >> 32));
-        }
-    }
-}
 
 // ------------------------------------------------------------------------------------------------ host side
 
