@@ -6,6 +6,7 @@
 //                                                        tensor-core candidate search + exact rescore (K2), smaller ones
 //                                                        the exact scan (K3); same bits either way
 //   mapDataSetTopTwo / topographicError (additions)   -> vsom_find_bmu2 (K2 / K3 in their top-2 mode)
+//   linearInitialize (addition)                       -> vsom_linear_init (co-moment pass + subspace iteration, lininit.cu)
 //   findBmu / findRestrictedBmu (one row)             -> vsom_find_bmu      (K3)
 //   euclidianWeightedDist / findLocalBmu / findRestrictedBmd -> vsom_all_dists
 //   variationalAutoEncoder / autoEncoder              -> vsom_soft_assign + host sampling
@@ -162,6 +163,10 @@ class Som
     // Topographic error of the loaded chunk (min_hits 0): the share of rows whose best and second-best nodes are not 8-neighbours
     // on the grid (max(|dx|, |dy|) == 1, no wrap-around); rows without a runner-up (a 1 x 1 map) are not errors.  0 for an empty chunk.
     double topographicError(const DataSet &dataset) const;
+    // Linear initialisation of the map from the loaded chunk (vsom_linear_init): the mean plane spans the plane of the rows' two
+    // principal components, the first axis along the longer side of the grid; S, sigma, weight, hits and the U-matrix are zeroed and
+    // the metrics reset, as randomInitialize does.  Standard / Median maps only (a CLR map throws), at least two finite rows.
+    void linearInitialize(const DataSet &dataset);
     // Rows grouped by BMU: counts[N], offsets[N+1], rowIds[n] (the "SomIndex build").
     void buildIndex(const std::vector<size_t> &bmu, std::vector<size_t> &counts, std::vector<size_t> &offsets, std::vector<unsigned> &rowIds) const;
     // Summation order of the distances (vsom_reduction_order of vsom_b200.h): 0 sequential, 1 lanes (online step only, near-tie

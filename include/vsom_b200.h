@@ -159,6 +159,33 @@ VSOM_API int vsom_debug_measure_peaks(vsom_ctx *ctx, double out[4]);
 VSOM_API int vsom_upload_state(vsom_ctx *ctx, const float *mean, const float *S, const float *sigma, const float *weight, const uint64_t *hits);
 VSOM_API int vsom_download_state(vsom_ctx *ctx, float *mean, float *S, float *sigma, float *weight, uint64_t *hits);
 
+/* Linear initialisation (not in the reference; SOM_PAK lininit / SOM Toolbox som_lininit): the map's mean plane spans the
+ * plane of the data's two leading principal components.  Standard and Median contexts (D = d_in = Dm).
+ *   1. mu = (1/n) sum_r x_r and C = (1/(n-1)) sum_r (x_r - mu)(x_r - mu)^T, both in f64.
+ *   2. lambda_1 >= lambda_2: the two largest eigenvalues of C, each clamped at 0; v_1, v_2 orthonormal eigenvectors for them, each
+ *      signed so that its component of largest magnitude is positive (the lowest index among equal magnitudes).  D = 1: v_1 = [1],
+ *      lambda_2 = 0, v_2 = 0.
+ *   3. The first axis runs along the longer side of the grid: with W >= H, x goes with (lambda_1, v_1) and y with (lambda_2, v_2);
+ *      otherwise the two are swapped.  Grid coordinate c_L(i) = (2i - (L-1)) / (L-1) for L >= 2, c_1(0) = 0.
+ *   4. m[y*W + x][k] = f32( (mu_k + (c_W(x) * s_x) * v_x[k]) + (c_H(y) * s_y) * v_y[k] ), s = sqrt(lambda), evaluated in f64 with
+ *      round-to-nearest in exactly that order and rounded to f32 once (so the plane can be recomputed bit for bit from the call's own
+ *      out_mean, out_lambda and out_axes).
+ *   5. S, sigma, weight and hits are set to 0 (the state Som::randomInitialize leaves).
+ * The bits depend only on the rows: not on the device, the summation order, Standard vs Median, or node sharding.  On node-sharded
+ * contexts every rank calls with the same rows and writes only its own grid rows (no communication).
+ * Method: one f64 pass over the rows shifted by the first row (host rows stream in slabs of VSOM_LINEAR_INIT_SLAB_ROWS rows), then
+ * subspace iteration on min(D, 8) vectors until |C v_i - lambda_i v_i| <= 1e-11 lambda_1 for i = 1, 2, or 300 iterations.  When the
+ * cap ends it (lambda_1, lambda_2, lambda_3 nearly equal: the data does not determine the axes) the call still succeeds with the Ritz
+ * pairs it has.
+ * x: n x d_in host rows (pageable or pinned).  out_mean[D], out_lambda[2], out_axes[2*D] (axis 1, then axis 2); each may be NULL.
+ * Errors: n < 2 or a non-finite element -> VSOM_ERR_INVALID; a CLR context -> VSOM_ERR_UNSUPPORTED (its model vector holds regression
+ * coefficients, not a point in data space).  A refused call leaves the state unchanged. */
+#define VSOM_LINEAR_INIT_SLAB_ROWS 16384
+VSOM_API int vsom_linear_init(vsom_ctx *ctx, const float *x, size_t n, double *out_mean, double *out_lambda, double *out_axes);
+/* Host wall time of the three phases of the last vsom_linear_init on ctx (ms): out[0] co-moment pass (including the copies of the
+ * rows), out[1] eigen step, out[2] fill; out[3] subspace iterations. */
+VSOM_API int vsom_debug_linear_init_phases(const vsom_ctx *ctx, double out[4]);
+
 /* One node's rows: Som::getNeuron / Som::getSigmaNeuron (src/Som.cpp:194-212).  Either output may be NULL. */
 VSOM_API int vsom_get_node(vsom_ctx *ctx, size_t node, float *mean, float *sigma);
 

@@ -46,6 +46,8 @@ _PROTOS = {
     "vsom_upload_state": (C.c_int, [_vp, _f32p, _f32p, _f32p, _f32p, _u64p]),
     "vsom_download_state": (C.c_int, [_vp, _f32p, _f32p, _f32p, _f32p, _u64p]),
     "vsom_get_node": (C.c_int, [_vp, C.c_size_t, _f32p, _f32p]),
+    "vsom_linear_init": (C.c_int, [_vp, _f32p, C.c_size_t, _f64p, _f64p, _f64p]),
+    "vsom_debug_linear_init_phases": (C.c_int, [_vp, _f64p]),
     "vsom_train_chunk": (C.c_int, [_vp, _f32p, C.c_size_t, C.c_double, C.c_double, C.c_int, _u64p, _u32p, _f32p, _f32p]),
     "vsom_train_chunk_device": (C.c_int, [_vp, _vp, C.c_size_t, C.c_double, C.c_double, C.c_int, _vp, _vp]),
     "vsom_batch_epoch": (C.c_int, [_vp, _f32p, C.c_size_t, C.c_double, C.c_int, _u64p, _f32p]),
@@ -187,6 +189,26 @@ class VsomContext:
         sigma = np.empty(self.Dm, np.float32)
         self._check(lib().vsom_get_node(self._h, node, _p(mean, _f32p), _p(sigma, _f32p)))
         return mean, sigma
+
+    def linear_init(self, x):
+        """Linear initialisation along the rows' two principal components (vsom_linear_init): sets the mean plane, zeroes S, sigma,
+        weight and hits; returns (mean[Din], lambda[2], axes[2, Din]) in f64."""
+        x = _f32(x).reshape(-1, self.Din)
+        mean = np.empty(self.Din, np.float64)
+        lam = np.empty(2, np.float64)
+        axes = np.empty((2, self.Din), np.float64)
+        self._check(lib().vsom_linear_init(self._h, _p(x, _f32p), x.shape[0], _p(mean, _f64p), _p(lam, _f64p), _p(axes, _f64p)))
+        return mean, lam, axes
+
+    def linear_init_host_ptr(self, x_ptr: int, n: int):
+        """vsom_linear_init on raw HOST rows (e.g. a pinned torch tensor); no outputs."""
+        self._check(lib().vsom_linear_init(self._h, C.cast(x_ptr, _f32p), n, None, None, None))
+
+    def linear_init_phases(self):
+        """Host wall time (ms) of the last linear_init: co-moment pass (with the row copies), eigen step, fill; and its iterations."""
+        out = np.zeros(4, np.float64)
+        self._check(lib().vsom_debug_linear_init_phases(self._h, _p(out, _f64p)))
+        return {"pass_ms": out[0], "eigen_ms": out[1], "fill_ms": out[2], "iterations": int(out[3])}
 
     # ---- online training
     def train_chunk(self, x, eta, sigma, decay=EXPONENTIAL, last_bmu=None):

@@ -496,6 +496,48 @@ int vsom_download_state(vsom_ctx *ctx, float *mean, float *S, float *sigma, floa
     return copy_state(ctx, false, mean, S, sigma, weight, hits);
 }
 
+int vsom_linear_init(vsom_ctx *ctx, const float *x, size_t n, double *out_mean, double *out_lambda, double *out_axes)
+{
+    if (!ctx)
+        return VSOM_ERR_INVALID;
+    if (ctx->transform == VSOM_CLR)
+        return set_error(ctx, VSOM_ERR_UNSUPPORTED, "vsom_linear_init: a CLR model vector holds regression coefficients, not a point in data space");
+    if (n < 2 || !x)
+        return set_error(ctx, VSOM_ERR_INVALID, "vsom_linear_init: needs x with at least two rows");
+    VSOM_CUDA(ctx, cudaSetDevice(ctx->device));
+    // the planes are written only once the pass (which refuses non-finite rows) and the eigen step have succeeded
+    LinearFit fit;
+    int rc = linear_init_fit(ctx, x, n, fit);
+    if (rc)
+        return rc;
+    rc = launch_linear_fill(ctx, fit);
+    if (rc)
+        return rc;
+    const size_t D = static_cast<size_t>(ctx->Din);
+    if (out_mean)
+        std::copy(fit.mean.begin(), fit.mean.end(), out_mean);
+    if (out_lambda)
+    {
+        out_lambda[0] = fit.lambda[0];
+        out_lambda[1] = fit.lambda[1];
+    }
+    if (out_axes)
+    {
+        std::copy(fit.axis1.begin(), fit.axis1.end(), out_axes);
+        std::copy(fit.axis2.begin(), fit.axis2.end(), out_axes + D);
+    }
+    return VSOM_OK;
+}
+
+int vsom_debug_linear_init_phases(const vsom_ctx *ctx, double out[4])
+{
+    if (!ctx || !out)
+        return VSOM_ERR_INVALID;
+    for (int i = 0; i < 4; ++i)
+        out[i] = ctx->linInitPhase[i];
+    return VSOM_OK;
+}
+
 int vsom_get_node(vsom_ctx *ctx, size_t node, float *mean, float *sigma)
 {
     if (ctx && ctx->world > 1)

@@ -173,6 +173,7 @@ struct vsom_ctx
     int umTiles = 0;
     long long *profDev = nullptr; // diagnostics: per-phase cycle sums of the last online-step launch
     size_t profSamples = 0;
+    double linInitPhase[4] = {};  // vsom_debug_linear_init_phases: pass, eigen step and fill (ms), iterations of the last call
     std::string err;
 };
 
@@ -248,6 +249,14 @@ int launch_similarity_rowmax(vsom_ctx *ctx, const float *xDev, size_t rows, cons
 int launch_umatrix_tiles(vsom_ctx *ctx, const float *const *meanRowDev, const float *const *sigmaRowDev, const int2 *tilesDev, int nTiles);
 int umatrix_tile_rows();
 int launch_build_index(vsom_ctx *ctx, const unsigned *bmuDev, size_t n, u64 *countsDev, u64 *offsetsDev, unsigned *rowIdsDev);
+// vsom_linear_init (lininit.cu): the mean and the two leading principal axes of n host rows (sign rule applied), then the planes
+struct LinearFit
+{
+    std::vector<double> mean, axis1, axis2;
+    double lambda[2] = {0.0, 0.0};
+};
+int linear_init_fit(vsom_ctx *ctx, const float *x, size_t n, LinearFit &fit);
+int launch_linear_fill(vsom_ctx *ctx, const LinearFit &fit);
 
 // ------------------------------------------------------------------------------------------ device helpers
 #ifdef __CUDACC__

@@ -277,6 +277,20 @@ void Som::randomInitialize(int seed, float sigma)
     deviceIsStale = true;
 }
 
+// Linear initialisation (an addition, not in the reference): vsom_linear_init on the loaded chunk writes the device planes; the
+// host mirror is refreshed from them on demand.
+void Som::linearInitialize(const DataSet &dataset)
+{
+    if (dataset.vectorLength() != inputLength())
+        throw std::invalid_argument("Som::linearInitialize: the rows' length differs from the map's input length");
+    vsom_ctx *ctx = context();
+    if (vsom_linear_init(ctx, dataset.contiguousRows(), dataset.size(), nullptr, nullptr, nullptr) != VSOM_OK)
+        fail(ctx, "Som::linearInitialize");
+    metrics = Metrics{depth};
+    std::fill(uMatrix.begin(), uMatrix.end(), 0.0);
+    hostIsStale = true;
+}
+
 // ------------------------------------------------------------------------------------------------ training
 
 void Som::train(DataSet &data, size_t numberOfEpochs, double eta0, double etaDecay, double sigma0, double sigmaDecay,
