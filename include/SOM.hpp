@@ -7,6 +7,7 @@
 //                                                        the exact scan (K3); same bits either way
 //   mapDataSetTopTwo / topographicError (additions)   -> vsom_find_bmu2 (K2 / K3 in their top-2 mode)
 //   linearInitialize (addition)                       -> vsom_linear_init (co-moment pass + subspace iteration, lininit.cu)
+//   clusterNodes (addition)                           -> vsom_cluster_nodes (k-means++ seeding + Lloyd over the mean plane, cluster.cu)
 //   findBmu / findRestrictedBmu (one row)             -> vsom_find_bmu      (K3)
 //   euclidianWeightedDist / findLocalBmu / findRestrictedBmd -> vsom_all_dists
 //   variationalAutoEncoder / autoEncoder              -> vsom_soft_assign + host sampling
@@ -167,6 +168,12 @@ class Som
     // principal components, the first axis along the longer side of the grid; S, sigma, weight, hits and the U-matrix are zeroed and
     // the metrics reset, as randomInitialize does.  Standard / Median maps only (a CLR map throws), at least two finite rows.
     void linearInitialize(const DataSet &dataset);
+    // k-means over the map's nodes (vsom_cluster_nodes): k-means++ seeding from `seed`, then at most maxIterations Lloyd iterations over
+    // the mean plane, each node weighted by 1 or (weightByHits) by its hit count.  labels[N] gets every node's cluster, centroids the k
+    // centroids (Dm values each, f64); returns the inertia (the weighted sum of the nodes' f32 distances to their centroids).  Throws
+    // on a refused call (k outside 1..N, a non-finite plane, fewer than k distinct nodes carrying weight).  Reads the map only.
+    double clusterNodes(size_t k, std::vector<int> &labels, std::vector<Eigen::VectorXd> &centroids, uint64_t seed = 0, bool weightByHits = false,
+                        int maxIterations = 300) const;
     // Rows grouped by BMU: counts[N], offsets[N+1], rowIds[n] (the "SomIndex build").
     void buildIndex(const std::vector<size_t> &bmu, std::vector<size_t> &counts, std::vector<size_t> &offsets, std::vector<unsigned> &rowIds) const;
     // Summation order of the distances (vsom_reduction_order of vsom_b200.h): 0 sequential, 1 lanes (online step only, near-tie

@@ -186,6 +186,45 @@ VSOM_API int vsom_linear_init(vsom_ctx *ctx, const float *x, size_t n, double *o
  * rows), out[1] eigen step, out[2] fill; out[3] subspace iterations. */
 VSOM_API int vsom_debug_linear_init_phases(const vsom_ctx *ctx, double out[4]);
 
+/* Clustering of the map's nodes (not in the reference; SOM Toolbox som_kmeans / kmeans_clusters after Vesanto & Alhoniemi (2000),
+ * somoclu's Somoclu.cluster): k-means++ seeding, then Lloyd iterations, over the N rows of the mean plane (Dm floats each; on a CLR
+ * context the regression coefficients, so the call clusters the regression models).  Read-only: the planes, hits and U-matrix are
+ * unchanged afterwards.  Weights: w_p = 1 under VSOM_CLUSTER_UNIFORM, (double)hits[p] under VSOM_CLUSTER_HITS.
+ *   Distance: d(p, c) = sum_k (m_p[k] - c[k])^2 in f32 in the context's summation order (a LANES context sums in the REFERENCE
+ *     order, as every path but the online step does), c = the f32 rounding (RN) of the f64 centroid: the bits vsom_find_bmu_exact
+ *     returns for the row m_p on a Standard context of k nodes whose mean plane holds those f32 centroids.
+ *   Seeding: splitmix64 with state = seed (state += 0x9E3779B97F4A7C15; z = state; z = (z ^ z>>30) * 0xBF58476D1CE4E5B9;
+ *     z = (z ^ z>>27) * 0x94D049BB133111EB; draw z ^ z>>31).  Pick j = 0 .. k-1 takes one draw, u_j = (draw >> 11) * 2^-53.  Pick
+ *     weights: q_p = w_p for pick 0, q_p = w_p * D_p (f64) after, D_p = (double) min over the earlier centroids i of d(p, c_i).
+ *     T_b = sequential f64 sum of q over nodes [VSOM_CLUSTER_BLOCK b, VSOM_CLUSTER_BLOCK (b + 1)) in node order; total = sequential
+ *     sum of the T_b; target = u_j * total.  The block: the first b whose running sum over blocks (running + T_b) exceeds the target,
+ *     else the last block with T_b > 0.  The node: inside it, from the sum of the earlier blocks, add q_p in node order and take the
+ *     first p whose sum exceeds the target, else the last p with q_p > 0.  Centroid j = that row, exact in f64.  A total of 0 (fewer
+ *     than k distinct nodes carry weight; under HITS a map that has seen no data) or one that is not finite -> VSOM_ERR_INVALID.
+ *   Lloyd, i = 1 .. max_iter: (1) label(p) = the j with the smallest (d(p, c_j), j).  (2) Stop when i > 1 and no label changed
+ *     (converged = 1), else when i = max_iter (converged = 0).  (3) Update: c_j[k] = (sum of w_p * (double)m_p[k]) / W_j,
+ *     W_j = sum of w_p, over the members in ascending node order, in consecutive groups of VSOM_CLUSTER_BLOCK members, each group
+ *     summed sequentially from 0 and the group sums added sequentially from 0; one f64 division.  A cluster with W_j = 0 keeps its
+ *     centroid.  Stopping before the update keeps the outputs consistent: the labels are the assignment to the returned centroids.
+ *   Outputs (each may be NULL): out_label[N], out_centroids[k * Dm] (f64), out_weight[k] = W_j of the final labels, out_inertia =
+ *     sum_p w_p * (double)d(p, c_label(p)) in the seeding's block order, out_iterations = the number of assignments, out_converged.
+ * Errors (no output written, no state changed): k < 1, k > N, max_iter < 1, an unknown weighting or a NaN / infinite element of the
+ * mean plane -> VSOM_ERR_INVALID; a node-sharded context -> VSOM_ERR_UNSUPPORTED.
+ * Device work: the seeding streams the plane once per pick with the block sums and the pick on the device; the assignment is the exact
+ * scan (K3) with the centroids as its map; the update groups the members with the index build (K5). */
+#define VSOM_CLUSTER_BLOCK 1024
+typedef enum vsom_cluster_weighting
+{
+    VSOM_CLUSTER_UNIFORM = 0,
+    VSOM_CLUSTER_HITS = 1
+} vsom_cluster_weighting;
+VSOM_API int vsom_cluster_nodes(vsom_ctx *ctx, int k, uint64_t seed, int weighting, int max_iter, int32_t *out_label, double *out_centroids, double *out_weight,
+                                double *out_inertia, int *out_iterations, int *out_converged);
+/* Device time (CUDA events on the context's stream, ms) of the phases of the last successful vsom_cluster_nodes on ctx: out[0] the
+ * seeding (the plane check included), out[1] all assignments, out[2] all updates, out[3] the outputs (the weights of the final
+ * labels and the inertia); out[4] the number of assignments (updates: one fewer). */
+VSOM_API int vsom_debug_cluster_phases(const vsom_ctx *ctx, double out[5]);
+
 /* One node's rows: Som::getNeuron / Som::getSigmaNeuron (src/Som.cpp:194-212).  Either output may be NULL. */
 VSOM_API int vsom_get_node(vsom_ctx *ctx, size_t node, float *mean, float *sigma);
 

@@ -7,6 +7,8 @@ B200 every call fails loudly.
 """
 from .binding import (  # noqa: F401
     CLR,
+    CLUSTER_HITS,
+    CLUSTER_UNIFORM,
     EXPONENTIAL,
     INVERSE_PROPORTIONAL,
     MEDIAN,

@@ -12,11 +12,13 @@ from . import build as _build
 STANDARD, MEDIAN, CLR = 0, 1, 2
 EXPONENTIAL, INVERSE_PROPORTIONAL = 0, 1
 ORDER_REFERENCE, ORDER_LANES, ORDER_EIGEN_SSE = 0, 1, 2
+CLUSTER_UNIFORM, CLUSTER_HITS = 0, 1
 
 _f32p = C.POINTER(C.c_float)
 _f64p = C.POINTER(C.c_double)
 _u32p = C.POINTER(C.c_uint32)
 _u64p = C.POINTER(C.c_uint64)
+_i32p = C.POINTER(C.c_int32)
 _vp = C.c_void_p
 
 _PROTOS = {
@@ -48,6 +50,8 @@ _PROTOS = {
     "vsom_get_node": (C.c_int, [_vp, C.c_size_t, _f32p, _f32p]),
     "vsom_linear_init": (C.c_int, [_vp, _f32p, C.c_size_t, _f64p, _f64p, _f64p]),
     "vsom_debug_linear_init_phases": (C.c_int, [_vp, _f64p]),
+    "vsom_debug_cluster_phases": (C.c_int, [_vp, _f64p]),
+    "vsom_cluster_nodes": (C.c_int, [_vp, C.c_int, C.c_uint64, C.c_int, C.c_int, _i32p, _f64p, _f64p, _f64p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "vsom_train_chunk": (C.c_int, [_vp, _f32p, C.c_size_t, C.c_double, C.c_double, C.c_int, _u64p, _u32p, _f32p, _f32p]),
     "vsom_train_chunk_device": (C.c_int, [_vp, _vp, C.c_size_t, C.c_double, C.c_double, C.c_int, _vp, _vp]),
     "vsom_batch_epoch": (C.c_int, [_vp, _f32p, C.c_size_t, C.c_double, C.c_int, _u64p, _f32p]),
@@ -209,6 +213,25 @@ class VsomContext:
         out = np.zeros(4, np.float64)
         self._check(lib().vsom_debug_linear_init_phases(self._h, _p(out, _f64p)))
         return {"pass_ms": out[0], "eigen_ms": out[1], "fill_ms": out[2], "iterations": int(out[3])}
+
+    def cluster_nodes(self, k, seed=0, weighting=CLUSTER_UNIFORM, max_iter=300):
+        """k-means over the map's nodes (vsom_cluster_nodes): k-means++ seeding from `seed`, then Lloyd iterations over the mean plane,
+        each node weighted by 1 (CLUSTER_UNIFORM) or its hit count (CLUSTER_HITS).  Returns (labels[N] int32, centroids[k, Dm] f64,
+        weight[k] f64, inertia, iterations, converged)."""
+        labels = np.empty(self.N, np.int32)
+        centroids = np.empty((k, self.Dm), np.float64)
+        weight = np.empty(k, np.float64)
+        inertia, iterations, converged = C.c_double(0), C.c_int(0), C.c_int(0)
+        self._check(lib().vsom_cluster_nodes(self._h, int(k), int(seed), int(weighting), int(max_iter), _p(labels, _i32p), _p(centroids, _f64p),
+                                             _p(weight, _f64p), C.byref(inertia), C.byref(iterations), C.byref(converged)))
+        return labels, centroids, weight, inertia.value, iterations.value, bool(converged.value)
+
+    def cluster_phases(self):
+        """Device time (ms) of the last cluster_nodes call's phases: seeding, all assignments, all updates, the outputs; and its number
+        of assignments (updates: one fewer)."""
+        out = np.zeros(5, np.float64)
+        self._check(lib().vsom_debug_cluster_phases(self._h, _p(out, _f64p)))
+        return {"seeding_ms": out[0], "assign_ms": out[1], "update_ms": out[2], "outputs_ms": out[3], "assignments": int(out[4])}
 
     # ---- online training
     def train_chunk(self, x, eta, sigma, decay=EXPONENTIAL, last_bmu=None):

@@ -17,6 +17,7 @@ API_DRIVER = os.path.join(REPO, "tests", "cpp", "api_driver_b200")
 MNIST_TEST = os.path.join(REPO, "tests", "cpp", "mnist_loader_test")
 TOPO_DRIVER = os.path.join(REPO, "tests", "cpp", "topo_driver")
 LININIT_DRIVER = os.path.join(REPO, "tests", "cpp", "lininit_driver")
+CLUSTER_DRIVER = os.path.join(REPO, "tests", "cpp", "cluster_driver")
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
@@ -40,7 +41,7 @@ def sources():
 
 
 def up_to_date() -> bool:
-    outputs = (LIB, HOST_LIB, API_DRIVER, MNIST_TEST, TOPO_DRIVER, LININIT_DRIVER)
+    outputs = (LIB, HOST_LIB, API_DRIVER, MNIST_TEST, TOPO_DRIVER, LININIT_DRIVER, CLUSTER_DRIVER)
     if not all(os.path.exists(o) for o in outputs):
         return False
     t = min(os.path.getmtime(o) for o in outputs)
@@ -97,7 +98,8 @@ def build_host() -> str:
     for src, exe, defs in ((os.path.join(REPO, "tests", "cpp", "api_driver.cpp"), API_DRIVER, ["-DVSOM_B200_API"]),
                            (os.path.join(REPO, "tests", "cpp", "mnist_loader_test.cpp"), MNIST_TEST, []),
                            (os.path.join(REPO, "tests", "cpp", "topo_driver.cpp"), TOPO_DRIVER, []),
-                           (os.path.join(REPO, "tests", "cpp", "lininit_driver.cpp"), LININIT_DRIVER, [])):
+                           (os.path.join(REPO, "tests", "cpp", "lininit_driver.cpp"), LININIT_DRIVER, []),
+                           (os.path.join(REPO, "tests", "cpp", "cluster_driver.cpp"), CLUSTER_DRIVER, [])):
         if os.path.exists(src):
             cmd = [cxx, *flags, *defs, src, "-o", exe, "-L", LIB_DIR, "-lvsom_host", "-lvsom_b200", f"-Wl,-rpath,{LIB_DIR}", *stdcxx]
             out = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)

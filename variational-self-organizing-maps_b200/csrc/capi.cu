@@ -538,6 +538,48 @@ int vsom_debug_linear_init_phases(const vsom_ctx *ctx, double out[4])
     return VSOM_OK;
 }
 
+int vsom_cluster_nodes(vsom_ctx *ctx, int k, uint64_t seed, int weighting, int max_iter, int32_t *out_label, double *out_centroids, double *out_weight,
+                       double *out_inertia, int *out_iterations, int *out_converged)
+{
+    if (ctx && ctx->world > 1)
+        return set_error(ctx, VSOM_ERR_UNSUPPORTED, "vsom_cluster_nodes: needs an unsharded context");
+    if (!ctx)
+        return VSOM_ERR_INVALID;
+    if (k < 1 || k > ctx->N || max_iter < 1 || (weighting != VSOM_CLUSTER_UNIFORM && weighting != VSOM_CLUSTER_HITS))
+        return set_error(ctx, VSOM_ERR_INVALID, "vsom_cluster_nodes: needs 1 <= k <= width*height, max_iter >= 1 and a known weighting");
+    VSOM_CUDA(ctx, cudaSetDevice(ctx->device));
+    // the outputs are written only once the whole call has succeeded
+    ClusterResult res;
+    const int rc = cluster_nodes(ctx, k, seed, weighting, max_iter, res);
+    if (rc)
+        return rc;
+    if (out_label)
+        std::copy(res.label.begin(), res.label.end(), out_label);
+    if (out_centroids)
+        std::copy(res.centroids.begin(), res.centroids.end(), out_centroids);
+    if (out_weight)
+        std::copy(res.weight.begin(), res.weight.end(), out_weight);
+    if (out_inertia)
+        *out_inertia = res.inertia;
+    if (out_iterations)
+        *out_iterations = res.iterations;
+    if (out_converged)
+        *out_converged = res.converged;
+    for (int i = 0; i < 4; ++i)
+        ctx->clusterPhase[i] = res.phaseMs[i];
+    ctx->clusterPhase[4] = res.iterations;
+    return VSOM_OK;
+}
+
+int vsom_debug_cluster_phases(const vsom_ctx *ctx, double out[5])
+{
+    if (!ctx || !out)
+        return VSOM_ERR_INVALID;
+    for (int i = 0; i < 5; ++i)
+        out[i] = ctx->clusterPhase[i];
+    return VSOM_OK;
+}
+
 int vsom_get_node(vsom_ctx *ctx, size_t node, float *mean, float *sigma)
 {
     if (ctx && ctx->world > 1)
@@ -927,7 +969,7 @@ int vsom_build_index_device(vsom_ctx *ctx, const uint32_t *bmu_dev, size_t n, ui
     if (!ctx || (!bmu_dev && n) || !counts_dev || !offsets_dev)
         return ctx ? set_error(ctx, VSOM_ERR_INVALID, "vsom_build_index_device: NULL argument") : VSOM_ERR_INVALID;
     VSOM_CUDA(ctx, cudaSetDevice(ctx->device));
-    return launch_build_index(ctx, bmu_dev, n, reinterpret_cast<u64 *>(counts_dev), reinterpret_cast<u64 *>(offsets_dev), row_ids_dev);
+    return launch_build_index(ctx, bmu_dev, n, ctx->N, reinterpret_cast<u64 *>(counts_dev), reinterpret_cast<u64 *>(offsets_dev), row_ids_dev);
 }
 
 int vsom_build_index(vsom_ctx *ctx, const uint32_t *bmu, size_t n, uint64_t *counts, uint64_t *offsets, uint32_t *row_ids)
@@ -953,7 +995,7 @@ int vsom_build_index(vsom_ctx *ctx, const uint32_t *bmu, size_t n, uint64_t *cou
     u64 *offsetsDev = countsDev + N;
     if (n)
         VSOM_CUDA(ctx, cudaMemcpyAsync(bmuDev, bmu, sizeof(unsigned) * n, cudaMemcpyHostToDevice, ctx->stream));
-    rc = launch_build_index(ctx, bmuDev, n, countsDev, offsetsDev, row_ids ? rowDev : nullptr);
+    rc = launch_build_index(ctx, bmuDev, n, ctx->N, countsDev, offsetsDev, row_ids ? rowDev : nullptr);
     if (rc)
         return rc;
     if (counts)

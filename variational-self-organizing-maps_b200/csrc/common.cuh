@@ -174,6 +174,7 @@ struct vsom_ctx
     long long *profDev = nullptr; // diagnostics: per-phase cycle sums of the last online-step launch
     size_t profSamples = 0;
     double linInitPhase[4] = {};  // vsom_debug_linear_init_phases: pass, eigen step and fill (ms), iterations of the last call
+    double clusterPhase[5] = {};  // vsom_debug_cluster_phases: seeding, assignments, updates, outputs (device ms), assignments of the last call
     std::string err;
 };
 
@@ -239,16 +240,43 @@ EncodeTiledFn tensor_map_encoder();
 // Every scoring call: x holds n rows (host memory when hostRows), results go to `out`.  Chooses K2 or the exact scan, runs K2's
 // tiers and the exact scan of the rows K2 leaves, and records the path for vsom_debug_last_score_tc (score_tc.cu).
 int score_rows(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, uint64_t minHits, bool allowTc, const ScoreOut &out, uint64_t *fallbackRows);
-// The exact scan (K3) of rows 0 .. n-1 of xDev, or (rowListDev != null) of the rows rowListDev[0 .. *rowCountDev)
+// The map operand of the exact scan (K3): the nodes every row is scored against, and how the rows are read.  scan_map(ctx) is the
+// context's own mean plane; vsom_cluster_nodes scores the plane's rows against its f32 centroids as a Standard map (cluster.cu).
+struct ScanMap
+{
+    const float *mean = nullptr; // N rows, rowStride floats apart
+    const u64 *hits = nullptr;   // per-node hit counts for min_hits > 0; null: every node competes (min_hits must be 0)
+    int N = 0, rowStride = 0;
+    int transform = VSOM_STANDARD; // the kernel's Comparer: CLR, or Standard (Standard and Median)
+    int Din = 0;                   // floats between consecutive rows of x
+    int Dr = 0, P = 0;             // residual length, CLR pair count
+};
+inline ScanMap scan_map(const vsom_ctx *ctx)
+{
+    ScanMap m;
+    m.mean = ctx->mean;
+    m.hits = ctx->hits;
+    m.N = ctx->N;
+    m.rowStride = ctx->rowStride;
+    m.transform = ctx->transform == VSOM_CLR ? VSOM_CLR : VSOM_STANDARD;
+    m.Din = ctx->Din;
+    m.Dr = ctx->Dr;
+    m.P = ctx->P;
+    return m;
+}
+// The exact scan (K3) of rows 0 .. n-1 of xDev, or (rowListDev != null) of the rows rowListDev[0 .. *rowCountDev), against `map`
 int launch_find_bmu_list(vsom_ctx *ctx, const float *xDev, size_t n, const unsigned *rowListDev, const unsigned *rowCountDev, uint64_t minHits, const ScoreOut &out,
-                         cudaStream_t stream, u64 *keyBufDev);
+                         cudaStream_t stream, u64 *keyBufDev, const ScanMap &map);
 int launch_batch_epoch(vsom_ctx *ctx, const float *xDev, size_t n, double sigma, int isFirst, const u64 *lastDev, unsigned *bmuDev, float *distDev);
 int launch_all_dists(vsom_ctx *ctx, const float *vDev, double *outDev);
 int launch_soft_assign(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, double *probDev, double *sumsDev);
 int launch_similarity_rowmax(vsom_ctx *ctx, const float *xDev, size_t rows, const unsigned *bmuDev, float k, float *outDev, cudaStream_t stream);
 int launch_umatrix_tiles(vsom_ctx *ctx, const float *const *meanRowDev, const float *const *sigmaRowDev, const int2 *tilesDev, int nTiles);
 int umatrix_tile_rows();
-int launch_build_index(vsom_ctx *ctx, const unsigned *bmuDev, size_t n, u64 *countsDev, u64 *offsetsDev, unsigned *rowIdsDev);
+// ids are bins 0 .. bins-1: the context's nodes (vsom_build_index), or the clusters of vsom_cluster_nodes
+int launch_build_index(vsom_ctx *ctx, const unsigned *bmuDev, size_t n, int bins, u64 *countsDev, u64 *offsetsDev, unsigned *rowIdsDev);
+// exclusive scan of countsDev[count] into offsetsDev[count + 1] (one CTA, som_index.cu)
+int launch_offsets_scan(vsom_ctx *ctx, const u64 *countsDev, int count, u64 *offsetsDev);
 // vsom_linear_init (lininit.cu): the mean and the two leading principal axes of n host rows (sign rule applied), then the planes
 struct LinearFit
 {
@@ -257,6 +285,16 @@ struct LinearFit
 };
 int linear_init_fit(vsom_ctx *ctx, const float *x, size_t n, LinearFit &fit);
 int launch_linear_fill(vsom_ctx *ctx, const LinearFit &fit);
+// vsom_cluster_nodes (cluster.cu): k-means++ seeding and Lloyd iterations over the mean plane; the outputs are host arrays
+struct ClusterResult
+{
+    std::vector<int32_t> label;
+    std::vector<double> centroids, weight;
+    double inertia = 0.0;
+    int iterations = 0, converged = 0;
+    double phaseMs[4] = {}; // device time of the seeding, the assignments, the updates and the outputs (vsom_debug_cluster_phases)
+};
+int cluster_nodes(vsom_ctx *ctx, int k, uint64_t seed, int weighting, int maxIter, ClusterResult &res);
 
 // ------------------------------------------------------------------------------------------ device helpers
 #ifdef __CUDACC__

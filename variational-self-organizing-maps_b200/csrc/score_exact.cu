@@ -480,7 +480,7 @@ int launch_soft_assign(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minH
 // scan of the rows a tensor-core slab could not certify, the count staying on the device; keyBufDev: out.top * n u64 of scratch.
 // out.top = 2: the runner-up of every row as well.
 int launch_find_bmu_list(vsom_ctx *ctx, const float *xDev, size_t n, const unsigned *rowListDev, const unsigned *rowCountDev, uint64_t minHits, const ScoreOut &out,
-                         cudaStream_t stream, u64 *keyBufDev)
+                         cudaStream_t stream, u64 *keyBufDev, const ScanMap &map)
 {
     if (n == 0)
         return VSOM_OK;
@@ -488,21 +488,21 @@ int launch_find_bmu_list(vsom_ctx *ctx, const float *xDev, size_t n, const unsig
     const bool eigen = ctx->order == VSOM_ORDER_EIGEN_SSE;
     const int tileRows = eigen ? ER : RT, tileNodes = eigen ? EN : NT;
     // list mode: a fixed grid (a few CTAs per SM) walks (row tile, node split) work items; 32 splits of the node range
-    const int nodeTiles = (ctx->N + tileNodes - 1) / tileNodes, splits = list ? std::max(1, std::min(32, nodeTiles)) : 1;
+    const int nodeTiles = (map.N + tileNodes - 1) / tileNodes, splits = list ? std::max(1, std::min(32, nodeTiles)) : 1;
     const unsigned grid = list ? static_cast<unsigned>(std::min<size_t>((n + tileRows - 1) / tileRows * splits, static_cast<size_t>(ctx->numSMs) * 4))
                                : static_cast<unsigned>((n + tileRows - 1) / tileRows);
     if (list)
         VSOM_CUDA(ctx, cudaMemsetAsync(keyBufDev, 0xff, sizeof(u64) * n * (out.top == 2 ? 2 : 1), stream));
-#define VSOM_SCORE_ARGS xDev, n, rowListDev, rowCountDev, ctx->mean, ctx->hits, minHits, ctx->N, ctx->Din, ctx->Dr, ctx->P, ctx->rowStride, ctx->pairI, ctx->pairJ, out.bmu, out.dist, splits, keyBufDev, out.bmu2, out.dist2
+#define VSOM_SCORE_ARGS xDev, n, rowListDev, rowCountDev, map.mean, map.hits, minHits, map.N, map.Din, map.Dr, map.P, map.rowStride, ctx->pairI, ctx->pairJ, out.bmu, out.dist, splits, keyBufDev, out.bmu2, out.dist2
 #define VSOM_SCORE_LAUNCH(TOP)                                                                                                   \
     if (eigen)                                                                                                                   \
     {                                                                                                                            \
-        if (ctx->transform == VSOM_CLR)                                                                                          \
+        if (map.transform == VSOM_CLR)                                                                                           \
             find_bmu_exact_eigen_kernel<VSOM_CLR, TOP><<<grid, kScoreThreads, 0, stream>>>(VSOM_SCORE_ARGS);                    \
         else                                                                                                                     \
             find_bmu_exact_eigen_kernel<VSOM_STANDARD, TOP><<<grid, kScoreThreads, 0, stream>>>(VSOM_SCORE_ARGS);               \
     }                                                                                                                            \
-    else if (ctx->transform == VSOM_CLR)                                                                                         \
+    else if (map.transform == VSOM_CLR)                                                                                          \
         find_bmu_exact_kernel<VSOM_CLR, TOP><<<grid, kScoreThreads, 0, stream>>>(VSOM_SCORE_ARGS);                              \
     else /* Standard and Median share the Comparer (src/Transformation.cpp:7-8, :45-46) */                                       \
         find_bmu_exact_kernel<VSOM_STANDARD, TOP><<<grid, kScoreThreads, 0, stream>>>(VSOM_SCORE_ARGS);

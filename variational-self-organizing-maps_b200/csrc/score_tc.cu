@@ -1190,7 +1190,7 @@ static int tc_enqueue(vsom_ctx *ctx, TcCall &c, const float *xs, size_t rows, co
         dev.dist, fbRows, fbCount, c.totalDev, dev.bmu2, dev.dist2);
     // rows the certificate rejected: exact scan (K3 tiles over the row list; the count stays on the device)
     add_count_kernel<<<1, 1, 0, rs>>>(fbCount, c.totalDev);
-    rc = launch_find_bmu_list(ctx, xs, rows, fbRows, fbCount, c.minHits, dev, rs, fbKeys);
+    rc = launch_find_bmu_list(ctx, xs, rows, fbRows, fbCount, c.minHits, dev, rs, fbKeys, scan_map(ctx));
     if (rc)
         return rc;
     if (host)
@@ -1412,7 +1412,7 @@ static int score_exact_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_
     {
         const size_t rows = std::min(slab, n - r0);
         VSOM_CUDA(ctx, cudaMemcpyAsync(xDev, xHost + r0 * ctx->Din, sizeof(float) * rows * ctx->Din, cudaMemcpyHostToDevice, ctx->stream));
-        rc = launch_find_bmu_list(ctx, xDev, rows, nullptr, nullptr, minHits, dev, ctx->stream, nullptr);
+        rc = launch_find_bmu_list(ctx, xDev, rows, nullptr, nullptr, minHits, dev, ctx->stream, nullptr, scan_map(ctx));
         if (rc)
             return rc;
         rc = slab_to_host(ctx, xDev, rows, dev, out.at(r0), ctx->stream);
@@ -1460,7 +1460,7 @@ int score_rows(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, uint64_t 
     {
         const float *xr = x + done * ctx->Din;
         const int rc = hostRows ? score_exact_host(ctx, xr, n - done, minHits, out.at(done))
-                                : launch_find_bmu_list(ctx, xr, n - done, nullptr, nullptr, minHits, out.at(done), ctx->stream, nullptr);
+                                : launch_find_bmu_list(ctx, xr, n - done, nullptr, nullptr, minHits, out.at(done), ctx->stream, nullptr, scan_map(ctx));
         if (rc)
             return rc;
         fallback += n - done;

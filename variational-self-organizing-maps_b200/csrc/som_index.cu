@@ -252,9 +252,17 @@ __global__ void __launch_bounds__(kSortThreads) radix_scatter_kernel(const unsig
     }
 }
 
-int launch_build_index(vsom_ctx *ctx, const unsigned *bmuDev, size_t n, u64 *countsDev, u64 *offsetsDev, unsigned *rowIdsDev)
+int launch_offsets_scan(vsom_ctx *ctx, const u64 *countsDev, int count, u64 *offsetsDev)
 {
-    const int N = ctx->N;
+    index_scan_kernel<<<1, 1024, 0, ctx->stream>>>(countsDev, count, offsetsDev);
+    ctx->launches += 1;
+    VSOM_CUDA(ctx, cudaGetLastError());
+    return VSOM_OK;
+}
+
+int launch_build_index(vsom_ctx *ctx, const unsigned *bmuDev, size_t n, int bins, u64 *countsDev, u64 *offsetsDev, unsigned *rowIdsDev)
+{
+    const int N = bins;
     if (n >= (1ull << 32))
         return set_error(ctx, VSOM_ERR_INVALID, "build_index: row ids are 32-bit; split the pass");
     // counts + offsets
@@ -276,9 +284,9 @@ int launch_build_index(vsom_ctx *ctx, const unsigned *bmuDev, size_t n, u64 *cou
         }
         ctx->launches += 1;
     }
-    index_scan_kernel<<<1, 1024, 0, ctx->stream>>>(countsDev, N, offsetsDev);
-    ctx->launches += 1;
-    VSOM_CUDA(ctx, cudaGetLastError());
+    int rc = launch_offsets_scan(ctx, countsDev, N, offsetsDev);
+    if (rc)
+        return rc;
     if (n == 0 || !rowIdsDev)
         return VSOM_OK;
 
@@ -290,7 +298,7 @@ int launch_build_index(vsom_ctx *ctx, const unsigned *bmuDev, size_t n, u64 *cou
     const unsigned nblocks = static_cast<unsigned>((n + kSortChunk - 1) / kSortChunk);
     const size_t tableLen = static_cast<size_t>(256) * nblocks;
     const unsigned scanChunks = static_cast<unsigned>((tableLen + kScanChunk - 1) / kScanChunk);
-    int rc = stage_reserve(ctx, 3, sizeof(unsigned) * (tableLen + scanChunks + 64));
+    rc = stage_reserve(ctx, 3, sizeof(unsigned) * (tableLen + scanChunks + 64));
     if (rc)
         return rc;
     rc = stage_reserve(ctx, 4, sizeof(unsigned) * n * 3); // keys ping, keys pong, vals pong

@@ -291,6 +291,26 @@ void Som::linearInitialize(const DataSet &dataset)
     hostIsStale = true;
 }
 
+// Clustering of the nodes (an addition, not in the reference): vsom_cluster_nodes over the device planes, which it leaves unchanged.
+double Som::clusterNodes(size_t k, std::vector<int> &labels, std::vector<Eigen::VectorXd> &centroids, uint64_t seed, bool weightByHits, int maxIterations) const
+{
+    const size_t nodes = width * height;
+    if (k < 1 || k > nodes)
+        throw std::invalid_argument("Som::clusterNodes: k must lie in 1 .. width*height");
+    vsom_ctx *ctx = context();
+    std::vector<int32_t> lab(nodes);
+    std::vector<double> cent(k * depth);
+    double inertia = 0.0;
+    if (vsom_cluster_nodes(ctx, static_cast<int>(k), seed, weightByHits ? VSOM_CLUSTER_HITS : VSOM_CLUSTER_UNIFORM, maxIterations, lab.data(), cent.data(), nullptr,
+                           &inertia, nullptr, nullptr) != VSOM_OK)
+        fail(ctx, "Som::clusterNodes");
+    labels.assign(lab.begin(), lab.end());
+    centroids.assign(k, Eigen::VectorXd(static_cast<Eigen::Index>(depth)));
+    for (size_t j = 0; j < k; ++j)
+        std::memcpy(centroids[j].data(), cent.data() + j * depth, depth * sizeof(double));
+    return inertia;
+}
+
 // ------------------------------------------------------------------------------------------------ training
 
 void Som::train(DataSet &data, size_t numberOfEpochs, double eta0, double etaDecay, double sigma0, double sigmaDecay,
