@@ -8,6 +8,7 @@
 //   mapDataSetTopTwo / topographicError (additions)   -> vsom_find_bmu2 (K2 / K3 in their top-2 mode)
 //   linearInitialize (addition)                       -> vsom_linear_init (co-moment pass + subspace iteration, lininit.cu)
 //   clusterNodes (addition)                           -> vsom_cluster_nodes (k-means++ seeding + Lloyd over the mean plane, cluster.cu)
+//   predictColumns (addition)                         -> vsom_predict_columns (K2 / K3 over the matched columns, predict.cu)
 //   findBmu / findRestrictedBmu (one row)             -> vsom_find_bmu      (K3)
 //   euclidianWeightedDist / findLocalBmu / findRestrictedBmd -> vsom_all_dists
 //   variationalAutoEncoder / autoEncoder              -> vsom_soft_assign + host sampling
@@ -174,6 +175,13 @@ class Som
     // on a refused call (k outside 1..N, a non-finite plane, fewer than k distinct nodes carrying weight).  Reads the map only.
     double clusterNodes(size_t k, std::vector<int> &labels, std::vector<Eigen::VectorXd> &centroids, uint64_t seed = 0, bool weightByHits = false,
                         int maxIterations = 300) const;
+    // Prediction of unobserved columns for the loaded chunk (vsom_predict_columns): each row's BMU over the columns whose matchColumns
+    // entry is true (bmuOut / distOut, as mapDataSet on a map of those columns only), and that node's mean and sigma at the other
+    // columns, q = getDepth() - (matched columns) values per row in ascending column order (meanOut / sigmaOut, n * q).  The rows'
+    // unmatched columns are never read.  Throws on a CLR map, on a mask whose length is not getDepth() and on a mask with no matched
+    // column.  Reads the map only.
+    void predictColumns(const DataSet &dataset, const std::vector<bool> &matchColumns, std::vector<size_t> &bmuOut, std::vector<float> &distOut,
+                        std::vector<float> &meanOut, std::vector<float> &sigmaOut, size_t minBmuHits = 0) const;
     // Rows grouped by BMU: counts[N], offsets[N+1], rowIds[n] (the "SomIndex build").
     void buildIndex(const std::vector<size_t> &bmu, std::vector<size_t> &counts, std::vector<size_t> &offsets, std::vector<unsigned> &rowIds) const;
     // Summation order of the distances (vsom_reduction_order of vsom_b200.h): 0 sequential, 1 lanes (online step only, near-tie

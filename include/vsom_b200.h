@@ -272,6 +272,29 @@ VSOM_API int vsom_find_bmu_device(vsom_ctx *ctx, const float *x_dev, size_t n, u
 /* Same contract, always the exact scan (K3) — what the tests compare the dispatching calls with. */
 VSOM_API int vsom_find_bmu_exact(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist);
 VSOM_API int vsom_find_bmu_exact_device(vsom_ctx *ctx, const float *x_dev, size_t n, uint64_t min_hits, uint32_t *out_bmu_dev, float *out_dist_dev);
+/* Prediction of unobserved columns (not in the reference; SOM Toolbox som_fillnans, kohonen predict(whatmap=)).
+ * match[Dm]: 1 = the column is observed and is matched, 0 = the column is predicted; any other value -> VSOM_ERR_INVALID.
+ * S = the matched columns in ascending order (|S| >= 1), Q = the predicted ones in ascending order (q = Dm - |S| >= 0).
+ * Per row r of x (n x d_in, full width; the columns in Q are never read and may hold anything, NaN included):
+ *   out_bmu[r], out_dist[r]: exactly what vsom_find_bmu_exact returns, with the same min_hits, on a Standard context of the
+ *     same grid and summation order whose mean plane is the columns S of this map, for the row x[r][S].  That is
+ *     d_S(p) = sum over j of (m_p[S_j] - x_r[S_j])^2 in f32 in the context's order over the compacted sequence (a LANES
+ *     context sums in the REFERENCE order, as every path but the online step does).  It inherits findRestrictedBmu's
+ *     eligibility (hits >= min_hits, node 0 always) and the NaN-at-node-0 rule.
+ *   out_mean[r*q + j] = mean[out_bmu[r]][Q_j], out_sigma[r*q + j] = sigma[out_bmu[r]][Q_j] (copies of the plane's f32 bits).
+ * Every output may be NULL.  |S| = Dm gives vsom_find_bmu's bits.  Read-only: planes, hits and U-matrix are unchanged.
+ * Errors (nothing written): match NULL, no matched column, a value other than 0 / 1 -> VSOM_ERR_INVALID; a CLR context
+ * (its model vector holds regression coefficients, not data columns) or a node-sharded one -> VSOM_ERR_UNSUPPORTED.
+ * Dispatch as vsom_find_bmu, over the compacted operands: >= 1024 rows with |S| <= 2048 run K2 (tiers, probes, exact
+ * rescore, certificate, exact scan of the rows it leaves); everything else runs K3.  vsom_debug_last_score_tc / _pair /
+ * _tc_stats report these calls like vsom_find_bmu's.  The host form copies full-width rows in vsom_find_bmu's slabs and
+ * gathers the columns S on the device; the predictions return per slab through 2 q floats per row of device staging for three
+ * slabs (one slab on the exact scan), on a stream of their own.  The device form gathers all n rows once (n x |S| floats of
+ * staging).  Staging is grow-only: it is kept until the context is destroyed. */
+VSOM_API int vsom_predict_columns(vsom_ctx *ctx, const float *x, size_t n, const uint8_t *match, uint64_t min_hits,
+                                  uint32_t *out_bmu, float *out_dist, float *out_mean, float *out_sigma);
+VSOM_API int vsom_predict_columns_device(vsom_ctx *ctx, const float *x_dev, size_t n, const uint8_t *match /* host */, uint64_t min_hits,
+                                         uint32_t *out_bmu_dev, float *out_dist_dev, float *out_mean_dev, float *out_sigma_dev);
 /* vsom_find_bmu[_device] that also reports how many rows took the exact full scan (fallback_rows, may be NULL; = n when
  * the whole batch ran on the exact scan). */
 VSOM_API int vsom_find_bmu_batch(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist, uint64_t *fallback_rows);

@@ -59,6 +59,8 @@ _PROTOS = {
     "vsom_find_bmu_device": (C.c_int, [_vp, _vp, C.c_size_t, C.c_uint64, _vp, _vp]),
     "vsom_find_bmu_exact": (C.c_int, [_vp, _f32p, C.c_size_t, C.c_uint64, _u32p, _f32p]),
     "vsom_find_bmu_exact_device": (C.c_int, [_vp, _vp, C.c_size_t, C.c_uint64, _vp, _vp]),
+    "vsom_predict_columns": (C.c_int, [_vp, _f32p, C.c_size_t, C.POINTER(C.c_uint8), C.c_uint64, _u32p, _f32p, _f32p, _f32p]),
+    "vsom_predict_columns_device": (C.c_int, [_vp, _vp, C.c_size_t, C.POINTER(C.c_uint8), C.c_uint64, _vp, _vp, _vp, _vp]),
     "vsom_debug_last_score_tc": (C.c_int, [_vp]),
     "vsom_debug_last_score_pair": (C.c_int, [_vp]),
     "vsom_debug_tc_stats": (C.c_int, [_vp, _u64p]),
@@ -286,6 +288,38 @@ class VsomContext:
         self._check(lib().vsom_find_bmu_exact_device(self._h, x_dev.data_ptr(), n, min_hits,
                                                      out_bmu_dev.data_ptr() if out_bmu_dev is not None else None,
                                                      out_dist_dev.data_ptr() if out_dist_dev is not None else None))
+
+    def _match(self, match):
+        """The mask of predict_columns[_device] as Dm bytes: the library reads exactly Dm of them and sizes the outputs from them.
+        None goes through as NULL (the library refuses it)."""
+        if match is None:
+            return None
+        match = np.ascontiguousarray(match, dtype=np.uint8)
+        if match.shape != (self.Dm,):
+            raise ValueError(f"match must hold one 0 / 1 entry per model column: shape ({self.Dm},), got {match.shape}")
+        return match
+
+    def predict_columns(self, x, match, min_hits=0):
+        """BMU of every row over the matched columns (match[Dm]: 1 matched, 0 predicted) and that node's mean and sigma at the
+        predicted ones: (bmu, dist, mean[n, q], sigma[n, q]).  The predicted columns of x are never read."""
+        x = _f32(x).reshape(-1, self.Din)
+        match = self._match(match)
+        n = x.shape[0]
+        q = 0 if match is None else int(self.Dm - np.count_nonzero(match == 1))
+        bmu = np.empty(n, np.uint32)
+        dist = np.empty(n, np.float32)
+        mean = np.empty((n, q), np.float32)
+        sigma = np.empty((n, q), np.float32)
+        self._check(lib().vsom_predict_columns(self._h, _p(x, _f32p), n, _p(match, C.POINTER(C.c_uint8)), min_hits, _p(bmu, _u32p), _p(dist, _f32p),
+                                               _p(mean, _f32p), _p(sigma, _f32p)))
+        return bmu, dist, mean, sigma
+
+    def predict_columns_device(self, x_dev, n, match, out_bmu_dev=None, out_dist_dev=None, out_mean_dev=None, out_sigma_dev=None, min_hits=0):
+        """vsom_predict_columns on device arrays (match stays a host array); out_mean_dev / out_sigma_dev hold n x q values."""
+        match = self._match(match)
+        ptr = lambda t: t.data_ptr() if t is not None else None
+        self._check(lib().vsom_predict_columns_device(self._h, x_dev.data_ptr(), n, _p(match, C.POINTER(C.c_uint8)), min_hits, ptr(out_bmu_dev),
+                                                      ptr(out_dist_dev), ptr(out_mean_dev), ptr(out_sigma_dev)))
 
     def find_bmu_host_ptr(self, x_ptr: int, n: int, bmu_ptr: int, dist_ptr: int, min_hits=0):
         """vsom_find_bmu on raw HOST addresses (e.g. pinned torch tensors): no numpy conversion in the way."""

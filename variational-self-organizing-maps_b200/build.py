@@ -18,6 +18,7 @@ MNIST_TEST = os.path.join(REPO, "tests", "cpp", "mnist_loader_test")
 TOPO_DRIVER = os.path.join(REPO, "tests", "cpp", "topo_driver")
 LININIT_DRIVER = os.path.join(REPO, "tests", "cpp", "lininit_driver")
 CLUSTER_DRIVER = os.path.join(REPO, "tests", "cpp", "cluster_driver")
+PREDICT_DRIVER = os.path.join(REPO, "tests", "cpp", "predict_driver")
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
@@ -41,7 +42,7 @@ def sources():
 
 
 def up_to_date() -> bool:
-    outputs = (LIB, HOST_LIB, API_DRIVER, MNIST_TEST, TOPO_DRIVER, LININIT_DRIVER, CLUSTER_DRIVER)
+    outputs = (LIB, HOST_LIB, API_DRIVER, MNIST_TEST, TOPO_DRIVER, LININIT_DRIVER, CLUSTER_DRIVER, PREDICT_DRIVER)
     if not all(os.path.exists(o) for o in outputs):
         return False
     t = min(os.path.getmtime(o) for o in outputs)
@@ -99,7 +100,8 @@ def build_host() -> str:
                            (os.path.join(REPO, "tests", "cpp", "mnist_loader_test.cpp"), MNIST_TEST, []),
                            (os.path.join(REPO, "tests", "cpp", "topo_driver.cpp"), TOPO_DRIVER, []),
                            (os.path.join(REPO, "tests", "cpp", "lininit_driver.cpp"), LININIT_DRIVER, []),
-                           (os.path.join(REPO, "tests", "cpp", "cluster_driver.cpp"), CLUSTER_DRIVER, [])):
+                           (os.path.join(REPO, "tests", "cpp", "cluster_driver.cpp"), CLUSTER_DRIVER, []),
+                           (os.path.join(REPO, "tests", "cpp", "predict_driver.cpp"), PREDICT_DRIVER, [])):
         if os.path.exists(src):
             cmd = [cxx, *flags, *defs, src, "-o", exe, "-L", LIB_DIR, "-lvsom_host", "-lvsom_b200", f"-Wl,-rpath,{LIB_DIR}", *stdcxx]
             out = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)

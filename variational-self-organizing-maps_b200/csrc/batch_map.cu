@@ -399,7 +399,7 @@ int launch_batch_epoch(vsom_ctx *ctx, const float *xDev, size_t n, double sigma,
         ScoreOut out;
         out.bmu = bmuDev;
         out.dist = distDev;
-        rc = score_rows(ctx, xDev, false, n, 0, true, out, nullptr);
+        rc = score_rows(ctx, xDev, false, n, 0, true, out, nullptr, scan_map(ctx));
         if (rc)
             return rc;
     }

@@ -342,6 +342,12 @@ void vsom_destroy(vsom_ctx *ctx)
             cudaStreamSynchronize(ctx->copyStream);
             cudaStreamDestroy(ctx->copyStream);
         }
+        if (ctx->outStream)
+        {
+            cudaStreamSynchronize(ctx->outStream);
+            cudaStreamDestroy(ctx->outStream);
+            cudaEventDestroy(ctx->evOut);
+        }
         for (int i = 0; i < 2; ++i)
         {
             cudaEventDestroy(ctx->evScore[i]);
@@ -727,7 +733,7 @@ static int score_entry(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, u
     if (!ctx || (!x && n))
         return ctx ? set_error(ctx, VSOM_ERR_INVALID, std::string(who) + ": x is NULL") : VSOM_ERR_INVALID;
     VSOM_CUDA(ctx, cudaSetDevice(ctx->device));
-    return score_rows(ctx, x, hostRows, n, min_hits, allowTc, out, fallback_rows);
+    return score_rows(ctx, x, hostRows, n, min_hits, allowTc, out, fallback_rows, scan_map(ctx));
 }
 
 int vsom_find_bmu_device(vsom_ctx *ctx, const float *x_dev, size_t n, uint64_t min_hits, uint32_t *out_bmu_dev, float *out_dist_dev)
@@ -748,6 +754,50 @@ int vsom_find_bmu_exact_device(vsom_ctx *ctx, const float *x_dev, size_t n, uint
 int vsom_find_bmu_exact(vsom_ctx *ctx, const float *x, size_t n, uint64_t min_hits, uint32_t *out_bmu, float *out_dist)
 {
     return score_entry(ctx, x, true, n, min_hits, false, ScoreOut{out_bmu, out_dist}, nullptr, "vsom_find_bmu_exact");
+}
+
+// the argument checks of vsom_predict_columns[_device]; predict_columns (predict.cu) does the rest
+static int predict_entry(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, const uint8_t *match, uint64_t min_hits, const ScoreOut &out, const char *who)
+{
+    if (!ctx)
+        return VSOM_ERR_INVALID;
+    if (ctx->world > 1)
+        return set_error(ctx, VSOM_ERR_UNSUPPORTED, kUnshardedOnly);
+    if (ctx->transform == VSOM_CLR)
+        return set_error(ctx, VSOM_ERR_UNSUPPORTED, std::string(who) + ": a CLR model vector holds regression coefficients, not data columns");
+    if (!x && n)
+        return set_error(ctx, VSOM_ERR_INVALID, std::string(who) + ": x is NULL");
+    if (!match)
+        return set_error(ctx, VSOM_ERR_INVALID, std::string(who) + ": match is NULL");
+    int matched = 0;
+    for (int j = 0; j < ctx->Dm; ++j)
+    {
+        if (match[j] > 1)
+            return set_error(ctx, VSOM_ERR_INVALID, std::string(who) + ": match[" + std::to_string(j) + "] is neither 0 nor 1");
+        matched += match[j];
+    }
+    if (!matched)
+        return set_error(ctx, VSOM_ERR_INVALID, std::string(who) + ": no matched column");
+    VSOM_CUDA(ctx, cudaSetDevice(ctx->device));
+    return predict_columns(ctx, x, hostRows, n, match, min_hits, out);
+}
+
+int vsom_predict_columns(vsom_ctx *ctx, const float *x, size_t n, const uint8_t *match, uint64_t min_hits, uint32_t *out_bmu, float *out_dist, float *out_mean,
+                         float *out_sigma)
+{
+    ScoreOut out{out_bmu, out_dist};
+    out.mean = out_mean;
+    out.sigma = out_sigma;
+    return predict_entry(ctx, x, true, n, match, min_hits, out, "vsom_predict_columns");
+}
+
+int vsom_predict_columns_device(vsom_ctx *ctx, const float *x_dev, size_t n, const uint8_t *match, uint64_t min_hits, uint32_t *out_bmu_dev, float *out_dist_dev,
+                                float *out_mean_dev, float *out_sigma_dev)
+{
+    ScoreOut out{out_bmu_dev, out_dist_dev};
+    out.mean = out_mean_dev;
+    out.sigma = out_sigma_dev;
+    return predict_entry(ctx, x_dev, false, n, match, min_hits, out, "vsom_predict_columns_device");
 }
 
 int vsom_find_bmu_batch_device(vsom_ctx *ctx, const float *x_dev, size_t n, uint64_t min_hits, uint32_t *out_bmu_dev, float *out_dist_dev,
@@ -828,7 +878,7 @@ int vsom_measure_similarity(vsom_ctx *ctx, const float *x, size_t n, uint64_t mi
     out.rowMax = out_row_max;
     out.rowMaxDev = static_cast<float *>(ctx->stage[9]);
     out.k = static_cast<float>(number_of_sigmas);
-    rc = score_rows(ctx, x, true, n, min_hits, true, out, nullptr);
+    rc = score_rows(ctx, x, true, n, min_hits, true, out, nullptr, scan_map(ctx));
     if (rc)
         return rc;
     // the tensor-core path's result copies run on its re-scoring stream; tc_finish joined it to the context's stream

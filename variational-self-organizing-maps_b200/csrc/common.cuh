@@ -133,6 +133,8 @@ struct vsom_ctx
     cudaStream_t stream = nullptr;
     cudaStream_t auxStream = nullptr;           // K2: re-scoring of slab i overlaps the search of slab i + 1
     cudaStream_t copyStream = nullptr;          // host-buffer scoring: H2D of slab i + 1 overlaps the search of slab i
+    cudaStream_t outStream = nullptr;           // vsom_predict_columns, host rows: the fill and D2H of slab i's predictions overlap the
+    cudaEvent_t evOut = nullptr;                // re-scoring of slab i + 1 and the H2D copies (created on first use)
     cudaEvent_t evScore[2] = {}, evDone[2] = {}, evCopied[3] = {}, evSlabDone[3] = {}; // evCopied / evSlabDone: per host staging buffer (three)
     int tcAttrSet = 0;                          // K2's dynamic shared-memory opt-in was set on this context's device
     int tcPairOk = 0;                           // ... and the device can co-schedule a cluster of two K2 CTAs (cta_group::2 kernel)
@@ -149,9 +151,9 @@ struct vsom_ctx
     std::vector<vsom::LutEntry> lutHost;
     double lutEta = -1, lutSigma = -1;
     int lutW = 0, lutH = 0;
-    // grow-only device staging for the host entry points
-    void *stage[10] = {};
-    size_t stageCap[10] = {};
+    // grow-only device staging for the host entry points (10..12: vsom_predict_columns, predict.cu)
+    void *stage[13] = {};
+    size_t stageCap[13] = {};
     bool trainEnqueued = false;              // vsom_train_chunk_device work not yet checked for an abort
     bool poisoned = false;                   // an online-step chunk aborted: the context refuses further chunks
     unsigned long long tcStats[3] = {0, 0, 0}; // K2 fallback causes since creation: list overflow, NaN / nothing eligible, certificate
@@ -208,21 +210,31 @@ struct ScoreOut
     float *rowMax = nullptr;
     float *rowMaxDev = nullptr;
     float k = 0.0f;
+    // vsom_predict_columns (q != 0): the mean and sigma of each row's final BMU at the columns predCols[0 .. q) (device), q values per
+    // row.  Device rows: written to mean / sigma after the search; host rows: computed into meanDev / sigmaDev behind each slab's BMUs
+    // and copied to mean / sigma.  meanDev / sigmaDev are slab staging that the host paths point at per slab (at() leaves them)
+    const int *predCols = nullptr;
+    int q = 0;
+    float *mean = nullptr, *sigma = nullptr;
+    float *meanDev = nullptr, *sigmaDev = nullptr;
 
     // the same outputs from row r on
     ScoreOut at(size_t r) const
     {
         ScoreOut o = *this;
-        auto shift = [r](auto *&p) {
+        auto shift = [](auto *&p, size_t by) {
             if (p)
-                p += r;
+                p += by;
         };
-        shift(o.bmu);
-        shift(o.dist);
-        shift(o.bmu2);
-        shift(o.dist2);
-        shift(o.rowMax);
-        shift(o.rowMaxDev);
+        shift(o.bmu, r);
+        shift(o.dist, r);
+        shift(o.bmu2, r);
+        shift(o.dist2, r);
+        shift(o.rowMax, r);
+        shift(o.rowMaxDev, r);
+        const size_t rq = r * static_cast<size_t>(q);
+        shift(o.mean, rq);
+        shift(o.sigma, rq);
         return o;
     }
 };
@@ -237,9 +249,6 @@ int prepare_online_step_fast(vsom_ctx *ctx, StepParams &p, double sigma); // K1F
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *, const cuuint32_t *,
                                   const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 EncodeTiledFn tensor_map_encoder();
-// Every scoring call: x holds n rows (host memory when hostRows), results go to `out`.  Chooses K2 or the exact scan, runs K2's
-// tiers and the exact scan of the rows K2 leaves, and records the path for vsom_debug_last_score_tc (score_tc.cu).
-int score_rows(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, uint64_t minHits, bool allowTc, const ScoreOut &out, uint64_t *fallbackRows);
 // The map operand of the exact scan (K3): the nodes every row is scored against, and how the rows are read.  scan_map(ctx) is the
 // context's own mean plane; vsom_cluster_nodes scores the plane's rows against its f32 centroids as a Standard map (cluster.cu).
 struct ScanMap
@@ -250,6 +259,10 @@ struct ScanMap
     int transform = VSOM_STANDARD; // the kernel's Comparer: CLR, or Standard (Standard and Median)
     int Din = 0;                   // floats between consecutive rows of x
     int Dr = 0, P = 0;             // residual length, CLR pair count
+    // host rows of vsom_predict_columns: the caller's rows are srcDin floats apart, and each host slab is gathered on the device to its
+    // columns cols[0 .. Din) (device memory) before the search reads it.  Null: the rows are read as they are (device rows always are).
+    const int *cols = nullptr;
+    int srcDin = 0;
 };
 inline ScanMap scan_map(const vsom_ctx *ctx)
 {
@@ -264,6 +277,11 @@ inline ScanMap scan_map(const vsom_ctx *ctx)
     m.P = ctx->P;
     return m;
 }
+// Every scoring call: x holds n rows (host memory when hostRows), results go to `out`, the nodes are those of `map` (scan_map(ctx),
+// or the compacted plane of vsom_predict_columns).  Chooses K2 or the exact scan, runs K2's tiers and the exact scan of the rows K2
+// leaves, and records the path for vsom_debug_last_score_tc (score_tc.cu).
+int score_rows(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, uint64_t minHits, bool allowTc, const ScoreOut &out, uint64_t *fallbackRows,
+               const ScanMap &map);
 // The exact scan (K3) of rows 0 .. n-1 of xDev, or (rowListDev != null) of the rows rowListDev[0 .. *rowCountDev), against `map`
 int launch_find_bmu_list(vsom_ctx *ctx, const float *xDev, size_t n, const unsigned *rowListDev, const unsigned *rowCountDev, uint64_t minHits, const ScoreOut &out,
                          cudaStream_t stream, u64 *keyBufDev, const ScanMap &map);
@@ -295,6 +313,11 @@ struct ClusterResult
     double phaseMs[4] = {}; // device time of the seeding, the assignments, the updates and the outputs (vsom_debug_cluster_phases)
 };
 int cluster_nodes(vsom_ctx *ctx, int k, uint64_t seed, int weighting, int maxIter, ClusterResult &res);
+// vsom_predict_columns (predict.cu): rows[r][cols[j]] -> out[r * outStride + j] for j < m, zeros up to outStride; and the BMU's mean
+// and sigma at out.predCols behind each row's BMU (into out.meanDev / sigmaDev when toStaging, else out.mean / sigma)
+int launch_gather_columns(vsom_ctx *ctx, const float *src, size_t rows, size_t srcStride, const int *colsDev, int m, int outStride, float *outDev, cudaStream_t stream);
+int launch_predict_fill(vsom_ctx *ctx, const unsigned *bmuDev, size_t rows, const ScoreOut &out, bool toStaging, cudaStream_t stream);
+int predict_columns(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, const uint8_t *match, uint64_t minHits, const ScoreOut &out);
 
 // ------------------------------------------------------------------------------------------ device helpers
 #ifdef __CUDACC__

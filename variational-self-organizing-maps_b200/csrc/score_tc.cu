@@ -1008,11 +1008,13 @@ struct TcCall
     TcScale *scale = nullptr;
     unsigned long long *totalDev = nullptr;
     CUtensorMap mapM;
+    ScanMap map; // the nodes the rows are scored against
 };
 
-static int tc_begin(vsom_ctx *ctx, TcCall &c, size_t maxSlabRows, uint64_t minHits, int split, int top)
+static int tc_begin(vsom_ctx *ctx, TcCall &c, const ScanMap &map, size_t maxSlabRows, uint64_t minHits, int split, int top)
 {
-    const int D = ctx->Dm, N = ctx->N;
+    const int D = map.Dr, N = map.N;
+    c.map = map;
     c.top = top;
     c.D = D;
     c.N = N;
@@ -1033,9 +1035,9 @@ static int tc_begin(vsom_ctx *ctx, TcCall &c, size_t maxSlabRows, uint64_t minHi
     float *mnorm = reinterpret_cast<float *>(static_cast<unsigned char *>(ctx->stage[6]) + mbBytes);
     c.scale = reinterpret_cast<TcScale *>(mnorm + c.Npad);
     VSOM_CUDA(ctx, cudaMemsetAsync(c.scale, 0, sizeof(TcScale), ctx->stream));
-    map_stats_kernel<<<(N + 7) / 8, 256, 0, ctx->stream>>>(ctx->mean, N, D, ctx->rowStride, mnorm, c.scale);
+    map_stats_kernel<<<(N + 7) / 8, 256, 0, ctx->stream>>>(map.mean, N, D, map.rowStride, mnorm, c.scale);
     tc_scale_kernel<<<1, 1, 0, ctx->stream>>>(c.scale, split);
-    map_operand_kernel<<<(c.Npad + 7) / 8, 256, 0, ctx->stream>>>(ctx->mean, mnorm, ctx->hits, minHits, N, c.Npad, D, ctx->rowStride, c.scale, Mb, c.Kpad);
+    map_operand_kernel<<<(c.Npad + 7) / 8, 256, 0, ctx->stream>>>(map.mean, mnorm, map.hits, minHits, N, c.Npad, D, map.rowStride, c.scale, Mb, c.Kpad);
     ctx->launches += 3;
     // function attributes are per device: set them for every context (not once per process), and ask once whether the device can
     // co-schedule a cluster of two of these CTAs (it cannot on a partition without whole TPCs; then the single-CTA kernel runs)
@@ -1108,8 +1110,10 @@ static int tc_begin(vsom_ctx *ctx, TcCall &c, size_t maxSlabRows, uint64_t minHi
 }
 
 // Host rows: the results of a slab are final in `dev` (device staging).  Behind them on `stream`: the similarity pass, then the
-// copies to the caller's buffers in `host`.
-static int slab_to_host(vsom_ctx *ctx, const float *xs, size_t rows, const ScoreOut &dev, const ScoreOut &host, cudaStream_t stream)
+// copies to the caller's buffers in `host`.  The predicted columns (host.q) are filled into host.meanDev / sigmaDev and copied out on
+// `outStream` behind the slab's BMUs: on the pipelined path a stream of their own, so that copying out 8q bytes per row overlaps the
+// next slab's re-scoring and the H2D copies instead of queuing in front of them.
+static int slab_to_host(vsom_ctx *ctx, const float *xs, size_t rows, const ScoreOut &dev, const ScoreOut &host, cudaStream_t stream, cudaStream_t outStream)
 {
     if (host.k != 0.0f)
     {
@@ -1117,6 +1121,22 @@ static int slab_to_host(vsom_ctx *ctx, const float *xs, size_t rows, const Score
         if (rc)
             return rc;
         VSOM_CUDA(ctx, cudaMemcpyAsync(host.rowMax, host.rowMaxDev, sizeof(float) * rows, cudaMemcpyDeviceToHost, stream));
+    }
+    if (host.q && (host.mean || host.sigma))
+    {
+        if (outStream != stream)
+        {
+            VSOM_CUDA(ctx, cudaEventRecord(ctx->evOut, stream));
+            VSOM_CUDA(ctx, cudaStreamWaitEvent(outStream, ctx->evOut, 0));
+        }
+        const int rc = launch_predict_fill(ctx, dev.bmu, rows, host, true, outStream);
+        if (rc)
+            return rc;
+        const size_t bytes = sizeof(float) * rows * static_cast<size_t>(host.q);
+        if (host.mean)
+            VSOM_CUDA(ctx, cudaMemcpyAsync(host.mean, host.meanDev, bytes, cudaMemcpyDeviceToHost, outStream));
+        if (host.sigma)
+            VSOM_CUDA(ctx, cudaMemcpyAsync(host.sigma, host.sigmaDev, bytes, cudaMemcpyDeviceToHost, outStream));
     }
     if (host.bmu)
         VSOM_CUDA(ctx, cudaMemcpyAsync(host.bmu, dev.bmu, sizeof(unsigned) * rows, cudaMemcpyDeviceToHost, stream));
@@ -1186,16 +1206,16 @@ static int tc_enqueue(vsom_ctx *ctx, TcCall &c, const float *xs, size_t rows, co
     VSOM_CUDA(ctx, cudaEventRecord(ctx->evScore[par], ctx->stream));
     VSOM_CUDA(ctx, cudaStreamWaitEvent(rs, ctx->evScore[par], 0));
     (c.top == 2 ? rescore_kernel<2> : rescore_kernel<1>)<<<static_cast<unsigned>((rows + RS_ROWS - 1) / RS_ROWS), RS_THREADS, 0, rs>>>(
-        xs, static_cast<long long>(rows), c.D, ctx->mean, ctx->rowStride, cand, candCount, bestA, xnorm, xratio, c.scale, c.Kpad, order, c.N, ctx->hits, c.minHits, dev.bmu,
+        xs, static_cast<long long>(rows), c.D, c.map.mean, c.map.rowStride, cand, candCount, bestA, xnorm, xratio, c.scale, c.Kpad, order, c.N, c.map.hits, c.minHits, dev.bmu,
         dev.dist, fbRows, fbCount, c.totalDev, dev.bmu2, dev.dist2);
     // rows the certificate rejected: exact scan (K3 tiles over the row list; the count stays on the device)
     add_count_kernel<<<1, 1, 0, rs>>>(fbCount, c.totalDev);
-    rc = launch_find_bmu_list(ctx, xs, rows, fbRows, fbCount, c.minHits, dev, rs, fbKeys, scan_map(ctx));
+    rc = launch_find_bmu_list(ctx, xs, rows, fbRows, fbCount, c.minHits, dev, rs, fbKeys, c.map);
     if (rc)
         return rc;
     if (host)
     {
-        rc = slab_to_host(ctx, xs, rows, dev, *host, rs);
+        rc = slab_to_host(ctx, xs, rows, dev, *host, rs, ctx->outStream);
         if (rc)
             return rc;
     }
@@ -1235,9 +1255,9 @@ static const double kTcTierSwitch = 0.04;
 static const double kTcExactSwitch = 0.25; // tier-2 probe fallback above this: the tensor cores select nothing useful, the rest is scanned exactly (tier "3")
 
 // rows per slab such that the fp16 operand staging of a slab stays below 2.5 GiB
-static size_t tc_slab_cap(const vsom_ctx *ctx, int split)
+static size_t tc_slab_cap(const ScanMap &map, int split)
 {
-    const size_t kext = static_cast<size_t>(split ? 3 * ctx->Dm : ctx->Dm) + 3, kpad = (kext + 15) / 16 * 16;
+    const size_t kext = static_cast<size_t>(split ? 3 * map.Dr : map.Dr) + 3, kpad = (kext + 15) / 16 * 16;
     return std::max<size_t>(TC_BM, ((size_t{5} << 29) / (kpad * 2)) & ~static_cast<size_t>(TC_BM - 1));
 }
 
@@ -1287,11 +1307,12 @@ static int tc_score_tiers(size_t n, const Run &run, int &tier, size_t &done, uns
 }
 
 // rows [0, n) of xDev through one tier; slabs of the given size
-static int tc_run_device(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t minHits, int split, size_t slabRows, const ScoreOut &out, unsigned long long &fallbackRows)
+static int tc_run_device(vsom_ctx *ctx, const ScanMap &map, const float *xDev, size_t n, uint64_t minHits, int split, size_t slabRows, const ScoreOut &out,
+                         unsigned long long &fallbackRows)
 {
-    slabRows = std::min(n, std::min(slabRows, tc_slab_cap(ctx, split)));
+    slabRows = std::min(n, std::min(slabRows, tc_slab_cap(map, split)));
     TcCall c;
-    int rc = tc_begin(ctx, c, slabRows, minHits, split, out.top);
+    int rc = tc_begin(ctx, c, map, slabRows, minHits, split, out.top);
     if (rc)
         return rc;
     for (size_t r0 = 0; r0 < n; r0 += slabRows)
@@ -1307,16 +1328,28 @@ static int tc_run_device(vsom_ctx *ctx, const float *xDev, size_t n, uint64_t mi
 // crosses PCIe in slabs on a copy stream into one of three staging buffers while the previous slabs are searched and re-scored,
 // and each slab's results return to the host behind its re-scoring.  With pinned host memory the three engines (H2D, SMs, D2H)
 // overlap fully; the call is then bound by the slower of PCIe (4 D bytes per row) and the kernel.  stage slots: 0 = three row
-// slabs, 1 / 2 = BMU / distance of the whole run, 4 = runner-ups and their distances (top = 2).
-static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t minHits, int split, size_t slabRows, const ScoreOut &out, unsigned long long &fallbackRows)
+// slabs, 1 / 2 = BMU / distance of the whole run, 4 = runner-ups and their distances (top = 2), 11 = the three slabs gathered to the
+// map's columns (map.cols: the copies carry srcDin floats per row, the search reads D), 12 = three slabs of predicted columns (out.q).
+// The predictions of slab s go out on ctx->outStream; the fill of slab s + 3 reuses slab s's staging behind its copies there.
+static int tc_run_host(vsom_ctx *ctx, const ScanMap &map, const float *xHost, size_t n, uint64_t minHits, int split, size_t slabRows, const ScoreOut &out,
+                       unsigned long long &fallbackRows)
 {
-    slabRows = std::min(n, std::min(slabRows, tc_slab_cap(ctx, split)));
-    const size_t D = static_cast<size_t>(ctx->Dm);
+    slabRows = std::min(n, std::min(slabRows, tc_slab_cap(map, split)));
+    const size_t D = static_cast<size_t>(map.Din), xD = map.cols ? static_cast<size_t>(map.srcDin) : D;
     // THREE staging buffers: the copy of slab s + 1 must not wait for the re-scoring (and the exact scan of the rejected rows) of
     // slab s - 1, which with two buffers sat on the critical path (measured: 14.6 ms per 512 K-row slab instead of 11.5)
-    int rc = stage_reserve(ctx, 0, sizeof(float) * 3 * slabRows * D);
+    int rc = stage_reserve(ctx, 0, sizeof(float) * 3 * slabRows * xD);
     if (rc)
         return rc;
+    float *cbuf[3] = {};
+    if (map.cols)
+    {
+        rc = stage_reserve(ctx, 11, sizeof(float) * 3 * slabRows * D);
+        if (rc)
+            return rc;
+        for (int i = 0; i < 3; ++i)
+            cbuf[i] = static_cast<float *>(ctx->stage[11]) + static_cast<size_t>(i) * slabRows * D;
+    }
     rc = stage_reserve(ctx, 1, sizeof(unsigned) * n);
     if (rc)
         return rc;
@@ -1325,7 +1358,7 @@ static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t min
         return rc;
     float *xbuf[3];
     for (int i = 0; i < 3; ++i)
-        xbuf[i] = static_cast<float *>(ctx->stage[0]) + static_cast<size_t>(i) * slabRows * D;
+        xbuf[i] = static_cast<float *>(ctx->stage[0]) + static_cast<size_t>(i) * slabRows * xD;
     ScoreOut dev;
     dev.bmu = static_cast<unsigned *>(ctx->stage[1]);
     dev.dist = static_cast<float *>(ctx->stage[2]);
@@ -1338,8 +1371,21 @@ static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t min
         dev.bmu2 = static_cast<unsigned *>(ctx->stage[4]);
         dev.dist2 = reinterpret_cast<float *>(dev.bmu2 + n);
     }
+    const bool predict = out.q && (out.mean || out.sigma);
+    const size_t slabVals = slabRows * static_cast<size_t>(out.q);
+    if (predict)
+    {
+        rc = stage_reserve(ctx, 12, sizeof(float) * 2 * 3 * slabVals);
+        if (rc)
+            return rc;
+        if (!ctx->outStream)
+        {
+            VSOM_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->outStream, cudaStreamNonBlocking));
+            VSOM_CUDA(ctx, cudaEventCreateWithFlags(&ctx->evOut, cudaEventDisableTiming));
+        }
+    }
     TcCall c;
-    rc = tc_begin(ctx, c, slabRows, minHits, split, out.top);
+    rc = tc_begin(ctx, c, map, slabRows, minHits, split, out.top);
     if (rc)
         return rc;
     // the staging buffers may still be in use by earlier work of the context's stream
@@ -1350,7 +1396,7 @@ static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t min
         const int b = static_cast<int>(slab % 3);
         if (slab >= 3)
             VSOM_CUDA(ctx, cudaStreamWaitEvent(ctx->copyStream, ctx->evSlabDone[b], 0)); // slab - 3 (same buffer) is fully re-scored
-        VSOM_CUDA(ctx, cudaMemcpyAsync(xbuf[b], xHost + r0 * D, sizeof(float) * rows * D, cudaMemcpyHostToDevice, ctx->copyStream));
+        VSOM_CUDA(ctx, cudaMemcpyAsync(xbuf[b], xHost + r0 * xD, sizeof(float) * rows * xD, cudaMemcpyHostToDevice, ctx->copyStream));
         VSOM_CUDA(ctx, cudaEventRecord(ctx->evCopied[b], ctx->copyStream));
         return VSOM_OK;
     };
@@ -1364,8 +1410,22 @@ static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t min
         const size_t r0 = sl * slabRows, rows = std::min(slabRows, n - r0);
         const int b = static_cast<int>(sl % 3);
         VSOM_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->evCopied[b], 0));
-        const ScoreOut host = out.at(r0);
-        rc = tc_enqueue(ctx, c, xbuf[b], rows, dev.at(r0), &host);
+        const float *xs = xbuf[b];
+        if (map.cols)
+        {
+            // cbuf[b] is free: slab sl - 3 was re-scored before the copy of this slab began (evSlabDone -> evCopied)
+            rc = launch_gather_columns(ctx, xbuf[b], rows, xD, map.cols, static_cast<int>(D), static_cast<int>(D), cbuf[b], ctx->stream);
+            if (rc)
+                return rc;
+            xs = cbuf[b];
+        }
+        ScoreOut host = out.at(r0);
+        if (predict)
+        {
+            host.meanDev = static_cast<float *>(ctx->stage[12]) + 2 * static_cast<size_t>(b) * slabVals;
+            host.sigmaDev = host.meanDev + slabVals;
+        }
+        rc = tc_enqueue(ctx, c, xs, rows, dev.at(r0), &host);
         if (rc)
             return rc;
         VSOM_CUDA(ctx, cudaEventRecord(ctx->evSlabDone[b], ctx->auxStream)); // behind the slab's re-scoring and result copies
@@ -1377,18 +1437,33 @@ static int tc_run_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t min
                 return rc;
         }
     }
+    if (predict)
+    {
+        // the context's stream owns the predictions again once they have been copied out
+        VSOM_CUDA(ctx, cudaEventRecord(ctx->evOut, ctx->outStream));
+        VSOM_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->evOut, 0));
+    }
     return tc_finish(ctx, c, fallbackRows);
 }
 
 // The exact scan of rows in HOST memory, in slabs (VSOM_EXACT_HOST_SLAB_LOG2, default 2^20 rows): staging stays bounded and each
-// slab's results return before the next slab is copied in.  stage slots as tc_run_host, sized by the slab.
-static int score_exact_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_t minHits, const ScoreOut &out)
+// slab's results return before the next slab is copied in.  stage slots as tc_run_host, sized by the slab (one buffer each).
+static int score_exact_host(vsom_ctx *ctx, const ScanMap &map, const float *xHost, size_t n, uint64_t minHits, const ScoreOut &out)
 {
     const char *slabEnv = getenv("VSOM_EXACT_HOST_SLAB_LOG2");
     const size_t slab = std::min(n, static_cast<size_t>(1) << (slabEnv ? atoi(slabEnv) : 20));
-    int rc = stage_reserve(ctx, 0, sizeof(float) * slab * ctx->Din);
+    const size_t D = static_cast<size_t>(map.Din), xD = map.cols ? static_cast<size_t>(map.srcDin) : D;
+    int rc = stage_reserve(ctx, 0, sizeof(float) * slab * xD);
     if (rc)
         return rc;
+    float *cDev = nullptr;
+    if (map.cols)
+    {
+        rc = stage_reserve(ctx, 11, sizeof(float) * slab * D);
+        if (rc)
+            return rc;
+        cDev = static_cast<float *>(ctx->stage[11]);
+    }
     rc = stage_reserve(ctx, 1, sizeof(unsigned) * slab);
     if (rc)
         return rc;
@@ -1396,6 +1471,14 @@ static int score_exact_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_
     if (rc)
         return rc;
     float *xDev = static_cast<float *>(ctx->stage[0]);
+    float *predDev = nullptr;
+    if (out.q && (out.mean || out.sigma))
+    {
+        rc = stage_reserve(ctx, 12, sizeof(float) * 2 * slab * out.q);
+        if (rc)
+            return rc;
+        predDev = static_cast<float *>(ctx->stage[12]);
+    }
     ScoreOut dev;
     dev.bmu = static_cast<unsigned *>(ctx->stage[1]);
     dev.dist = static_cast<float *>(ctx->stage[2]);
@@ -1411,11 +1494,25 @@ static int score_exact_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_
     for (size_t r0 = 0; r0 < n; r0 += slab)
     {
         const size_t rows = std::min(slab, n - r0);
-        VSOM_CUDA(ctx, cudaMemcpyAsync(xDev, xHost + r0 * ctx->Din, sizeof(float) * rows * ctx->Din, cudaMemcpyHostToDevice, ctx->stream));
-        rc = launch_find_bmu_list(ctx, xDev, rows, nullptr, nullptr, minHits, dev, ctx->stream, nullptr, scan_map(ctx));
+        VSOM_CUDA(ctx, cudaMemcpyAsync(xDev, xHost + r0 * xD, sizeof(float) * rows * xD, cudaMemcpyHostToDevice, ctx->stream));
+        const float *xs = xDev;
+        if (map.cols)
+        {
+            rc = launch_gather_columns(ctx, xDev, rows, xD, map.cols, static_cast<int>(D), static_cast<int>(D), cDev, ctx->stream);
+            if (rc)
+                return rc;
+            xs = cDev;
+        }
+        rc = launch_find_bmu_list(ctx, xs, rows, nullptr, nullptr, minHits, dev, ctx->stream, nullptr, map);
         if (rc)
             return rc;
-        rc = slab_to_host(ctx, xDev, rows, dev, out.at(r0), ctx->stream);
+        ScoreOut host = out.at(r0);
+        if (predDev)
+        {
+            host.meanDev = predDev;
+            host.sigmaDev = predDev + slab * out.q;
+        }
+        rc = slab_to_host(ctx, xs, rows, dev, host, ctx->stream, ctx->stream);
         if (rc)
             return rc;
         VSOM_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); // the staging buffers are reused by the next slab
@@ -1425,11 +1522,14 @@ static int score_exact_host(vsom_ctx *ctx, const float *xHost, size_t n, uint64_
 
 // Batches of at least kTcMinRows rows on a shape K2 covers take the tensor-core candidate search + exact rescore (same results,
 // bit for bit); everything else the exact scan.  K2 covers the Standard / Median Comparer (the contraction form of |m - x|^2) up to
-// Dm = 2048; rows longer than TC_MAXK stream their A k-blocks.
+// 2048 model columns; rows longer than TC_MAXK stream their A k-blocks.
 static const size_t kTcMinRows = 1024;
 
-int score_rows(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, uint64_t minHits, bool allowTc, const ScoreOut &out, uint64_t *fallbackRows)
+int score_rows(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, uint64_t minHits, bool allowTc, const ScoreOut &out, uint64_t *fallbackRows,
+               const ScanMap &map)
 {
+    // floats between the caller's rows
+    const size_t xD = static_cast<size_t>(hostRows && map.cols ? map.srcDin : map.Din);
     if (fallbackRows)
         *fallbackRows = 0;
     if (hostRows && n == 0)
@@ -1437,7 +1537,7 @@ int score_rows(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, uint64_t 
     int tier = 0;
     size_t done = 0;
     unsigned long long fallback = 0;
-    if (allowTc && ctx->transform != VSOM_CLR && ctx->Dm <= 2048 && n >= kTcMinRows)
+    if (allowTc && map.transform != VSOM_CLR && map.Dr <= 2048 && n >= kTcMinRows)
     {
         // test knobs; smaller device slabs measured slower (per-slab ramp and tail of the persistent kernel)
         const char *slabEnv = getenv(hostRows ? "VSOM_TC_HOST_SLAB_LOG2" : "VSOM_TC_SLAB_LOG2");
@@ -1448,8 +1548,8 @@ int score_rows(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, uint64_t 
             [&](size_t r0, size_t rows, int t, unsigned long long &fb) {
                 const int split = t == 2 ? 1 : 0;
                 const size_t slab = t == 2 ? slab2 : slab1;
-                return hostRows ? tc_run_host(ctx, x + r0 * ctx->Din, rows, minHits, split, slab, out.at(r0), fb)
-                                : tc_run_device(ctx, x + r0 * ctx->Din, rows, minHits, split, slab, out.at(r0), fb);
+                return hostRows ? tc_run_host(ctx, map, x + r0 * xD, rows, minHits, split, slab, out.at(r0), fb)
+                                : tc_run_device(ctx, map, x + r0 * xD, rows, minHits, split, slab, out.at(r0), fb);
             },
             tier, done, fallback);
         if (rc)
@@ -1458,12 +1558,20 @@ int score_rows(vsom_ctx *ctx, const float *x, bool hostRows, size_t n, uint64_t 
     ctx->lastScoreTier = tier;
     if (done < n) // every row, or the rows the probes sent to the exact scan (tier 3)
     {
-        const float *xr = x + done * ctx->Din;
-        const int rc = hostRows ? score_exact_host(ctx, xr, n - done, minHits, out.at(done))
-                                : launch_find_bmu_list(ctx, xr, n - done, nullptr, nullptr, minHits, out.at(done), ctx->stream, nullptr, scan_map(ctx));
+        const float *xr = x + done * xD;
+        const int rc = hostRows ? score_exact_host(ctx, map, xr, n - done, minHits, out.at(done))
+                                : launch_find_bmu_list(ctx, xr, n - done, nullptr, nullptr, minHits, out.at(done), ctx->stream, nullptr, map);
         if (rc)
             return rc;
         fallback += n - done;
+    }
+    if (!hostRows && out.q && (out.mean || out.sigma))
+    {
+        // device rows: the predicted columns behind the final BMUs, which the context's stream owns again (tc_finish joined the
+        // re-scoring stream)
+        const int rc = launch_predict_fill(ctx, out.bmu, n, out, false, ctx->stream);
+        if (rc)
+            return rc;
     }
     if (fallbackRows)
         *fallbackRows = fallback;

@@ -473,6 +473,31 @@ void Som::mapDataSet(const DataSet &dataset, std::vector<size_t> &bmuOut, std::v
     bmuOut.assign(bmu.begin(), bmu.end());
 }
 
+// Prediction from a column subset (an addition, not in the reference): vsom_predict_columns over the loaded chunk.
+void Som::predictColumns(const DataSet &dataset, const std::vector<bool> &matchColumns, std::vector<size_t> &bmuOut, std::vector<float> &distOut,
+                         std::vector<float> &meanOut, std::vector<float> &sigmaOut, size_t minBmuHits) const
+{
+    if (transform.deviceKind() == Transformation::DeviceKind::LinearRegression)
+        throw std::invalid_argument("Som::predictColumns: a CLR map's model vector holds regression coefficients, not data columns");
+    if (matchColumns.size() != depth)
+        throw std::invalid_argument("Som::predictColumns: the mask's length differs from getDepth()");
+    std::vector<uint8_t> match(depth);
+    size_t matched = 0;
+    for (size_t j = 0; j < depth; ++j)
+        matched += match[j] = matchColumns[j] ? 1 : 0;
+    if (matched == 0)
+        throw std::invalid_argument("Som::predictColumns: the mask has no matched column");
+    vsom_ctx *ctx = context();
+    const size_t rows = dataset.size(), q = depth - matched;
+    std::vector<uint32_t> bmu(rows);
+    distOut.resize(rows);
+    meanOut.resize(rows * q);
+    sigmaOut.resize(rows * q);
+    if (vsom_predict_columns(ctx, dataset.contiguousRows(), rows, match.data(), minBmuHits, bmu.data(), distOut.data(), meanOut.data(), sigmaOut.data()) != VSOM_OK)
+        fail(ctx, "Som::predictColumns");
+    bmuOut.assign(bmu.begin(), bmu.end());
+}
+
 void Som::mapDataSetTopTwo(const DataSet &dataset, std::vector<size_t> &bmuOut, std::vector<float> &distOut, std::vector<size_t> &bmu2Out,
                            std::vector<float> &dist2Out, size_t minBmuHits) const
 {
